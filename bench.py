@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host cores
     python bench.py --config {standing4096,walking65536,legacy16384,mixed1M} [--data replay]
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as .npy
 
 One "step" = one TSID tick (computeProblemData + solve + decode, ref:main.py:119-127) of every env of the
 batch.  The headline workload (default) is BASELINE.json configs[2]: robot/v1 LIPM walking, 65536 envs per GPU
@@ -57,6 +58,8 @@ CONFIGS = {
 }
 GAIT = {"v1": (0.3, 0.2, 0.2, 0.5), "v0": (0.1, 0.1275, 0.05, 0.7)}  # ref:ctrl/conf.py:24-28, ref:legacy/op3_conf.py:9-12
 CHUNK = 131072  # envs per handle call (workspace 30 KB per env)
+DUMP_FIELDS = ("tau", "ddq", "f", "status", "iters", "active_set")  # what TsidEngine.compute hands the bench's tick
+DUMP_BYTES = 60 << 20  # array bytes of --dump-outputs over all ranks; with the .npy headers the files stay under 64 MB
 
 
 # ----------------------------------------------------------------------------------------------
@@ -248,16 +251,48 @@ class Shard:
     def set_inputs(self, qd, vd, md, rd):
         self.qd, self.vd, self.md, self.rd = qd, vd, md, rd
 
-    def tick(self):
-        """One tick of every env of the shard (a handle call per chunk of <= CHUNK envs); returns (status, iters)."""
+    def tick(self, keep=False):
+        """One tick of every env of the shard (a handle call per chunk of <= CHUNK envs); returns (status, iters).
+        self.outs: the TickOutput of every chunk.  With one chunk that is the engine's buffers (valid until the next
+        tick); with several each call overwrites the previous chunk's buffers, so keep=True copies them (inside the
+        tick) and otherwise self.outs is None."""
         if len(self.chunks) == 1:
             o = self.eng.compute(self.qd, self.vd, self.md, self.rd, want_active=True)
+            self.outs = [o]
             return o.status, o.iters
-        outs = []
+        outs, self.outs = [], [] if keep else None
         for lo, hi in self.chunks:
             o = self.eng.compute(self.qd[lo:hi], self.vd[lo:hi], self.md[lo:hi], {k: r[lo:hi] for k, r in self.rd.items()})
             outs.append((o.status.clone(), o.iters.clone()))
+            if keep:
+                from tsid_control_b200.engine import TickOutput
+
+                self.outs.append(TickOutput(**{k: getattr(o, k).clone() for k in DUMP_FIELDS}))
         return self.torch.cat([a for a, _ in outs]), self.torch.cat([b for _, b in outs])
+
+
+def dump_outputs(out_dir: str, shards, prefix: str, limit: int) -> None:
+    """The outputs of the shards' last tick as out_dir/<prefix><kind>_<field>.npy, float64: tau, ddq, f, status, iters,
+    active_set as [N, 6] (each of its three 64-bit words as low and high 32 bits, exact in float64) and env, the env index
+    within the shard of every row.  Above `limit` bytes every shard keeps the same share of its envs, drawn with a fixed
+    seed: with the same arguments the rows are the same envs on the same inputs from run to run."""
+    import torch
+
+    bytes_per_env = [8 * (s.eng.na + s.eng.nv + 24 + 2 + 6 + 1) for s in shards]
+    total = sum(s.n * b for s, b in zip(shards, bytes_per_env))
+    os.makedirs(out_dir, exist_ok=True)
+    for s in shards:
+        env = np.arange(s.n)
+        if total > limit:
+            env = np.sort(np.random.default_rng(0).choice(s.n, s.n * limit // total, replace=False))
+        idx = torch.as_tensor(env, device=s.dev)
+        out = {f: torch.cat([getattr(o, f) for o in s.outs], dim=1 if f == "active_set" else 0) for f in DUMP_FIELDS}
+        out = {f: (t[:, idx].T if f == "active_set" else t[idx]).cpu().numpy() for f, t in out.items()}
+        words = out["active_set"].view(np.uint64)
+        out["active_set"] = np.stack([words & 0xFFFFFFFF, words >> 32], axis=-1).reshape(len(env), 6)
+        out["env"] = env
+        for f, a in out.items():
+            np.save(os.path.join(out_dir, f"{prefix}{s.kind}_{f}.npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def main() -> None:
@@ -276,11 +311,20 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true",
                     help="profiling runs only: skip the end-to-end and latency legs (the line then has no e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the outputs of the last one (tau, ddq, f, status, iters, active_set) "
+                         "as DIR/<kind>_<name>.npy, float64, at most 64 MB in all (above that a fixed, seeded sample of the "
+                         "envs); configs of more than 131072 envs per model copy each chunk's outputs inside that step")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
         return
 
+    sys.dont_write_bytecode = True  # the tree may be read-only: the modules imported below leave no __pycache__ in it
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -354,14 +398,14 @@ def main() -> None:
 
     step_no = [0]
 
-    def step():
+    def step(keep=False):
         if replay is not None:
             shards[0].set_inputs(*replay[step_no[0] % len(replay)])
             step_no[0] += 1
         off = 0
         res = []
         for s in shards:
-            st, it = s.tick()
+            st, it = s.tick(keep)
             res.append((st, it))
             if world > 1:
                 diag_st[off:off + s.n] = st
@@ -385,17 +429,19 @@ def main() -> None:
     launches0 = sum(s.eng.launch_count() for s in shards)
     evs = []
     iters_seen, mask_seen = [], []
-    for _ in range(args.steps):
+    for i in range(args.steps):
         flush.zero_()  # evict the inputs from L2 (outside the timed events)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        res = step()
+        res = step(keep=bool(args.dump_outputs) and i == args.steps - 1)
         e1.record()
         evs.append((e0, e1))
         if replay is not None:  # the iteration histogram differs from step to step: keep them all (outside the events)
             iters_seen.append(res[0][1].cpu().numpy().copy())
             mask_seen.append(shards[0].md.cpu().numpy().copy())
     torch.cuda.synchronize()
+    if args.dump_outputs:  # before any other tick reuses the output buffers
+        dump_outputs(args.dump_outputs, shards, f"rank{rank}_" if world > 1 else "", DUMP_BYTES // world)
     if world > 1:
         dist.barrier()
     launches = sum(s.eng.launch_count() for s in shards) - launches0
