@@ -225,8 +225,40 @@ int tsidb_compute_host_devrefs(tsidb_handle* h, int n_envs, const double* q, con
  * RobotWrapper::computeAllTerms / the solver's H, g build produce inside ref:main.py:119,121.  Host pointers;
  * synchronous.  Valid when the last tick ran without a contact mask or with at most TSIDB_SMALL_N envs (no class sort:
  * slot == env) on a handle created with TSIDB_SMALL_LOCAL_N=0 (the images of the smallest ticks otherwise stay in shared
- * memory); n_contacts = contacts of that env in that tick. */
+ * memory); n_contacts = contacts of that env in that tick.  A tsidb_problem_data call also fills these images (slot ==
+ * env, every env of that call): after it this function reads that call's terms. */
 int tsidb_debug_terms(tsidb_handle* h, int env, int n_contacts, double* M, double* nle, double* JF, double* H, double* g);
+
+/* ---- the assembled QP without the solve ---------------------------------------------------------------------------
+ * formulation.computeProblemData (ref:main.py:119) for n_envs robots: exactly the problem SolverHQuadProgFast hands to
+ * eiquadprog for each env,
+ *     min 1/2 x^T H x + g^T x   s.t.   CE x + ce0 = 0,   CI x + ci0 >= 0,
+ * in compact variables x = [dv; f of the feet in contact, LF first] (n = nv + 12 nc; the force-block order of the tick).
+ *   equality rows:   base dynamics (6; ce0 = h_u), then the contact-motion rows of the feet in contact, LF first;
+ *   inequality rows: the blocks [LF force (in contact), RF force (in contact), actuation (use_torque_bounds), joint bounds
+ *                    (use_joint_bounds)], each stacked [lower rows (A, -lb); upper rows (-A, ub)] as SolverHQuadProgFast
+ *                    stacks a two-sided constraint.
+ * Every array is per env, row-major, DEVICE memory, zero outside the env's (n, neq, nin); any pointer may be NULL (that
+ * part is not written).  H, CE and CI must be 16-byte aligned.  The maxima come from tsidb_problem_sizes:
+ * n_max = nv + 24, neq_max = 18, nin_max = 2 (34 + na use_torque_bounds + nv use_joint_bounds) (robot/v1: 50 / 18 / 160). */
+typedef struct tsidb_problem_out {
+  double* H;      /* [N][n_max][n_max]   full symmetric Hessian, regulariser included */
+  double* g;      /* [N][n_max]                                                         */
+  double* CE;     /* [N][neq_max][n_max]                                                */
+  double* ce0;    /* [N][neq_max]                                                       */
+  double* CI;     /* [N][nin_max][n_max]  one-sided rows                                */
+  double* ci0;    /* [N][nin_max]                                                       */
+  int32_t* sizes; /* [N][3]  n, neq, nin of this env                                    */
+} tsidb_problem_out;
+
+int tsidb_problem_sizes(const tsidb_handle* h, int* n_max, int* neq_max, int* nin_max);
+/* q, v, contact_mask and refs as in tsidb_compute (`layout` applies to them only; the outputs are always row-major per
+ * env); a NULL mask means double support, NULL refs the handle's defaults.  Asynchronous on cuda_stream.  The call keeps
+ * no state that a later tick reads (it leaves the scheduling hint's forecast alone), but it uses the handle's image
+ * workspaces, so it is ordered with the other calls on the handle like any of them, and tsidb_debug_terms reads its
+ * images afterwards. */
+int tsidb_problem_data(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
+                       const uint8_t* contact_mask, const tsidb_refs* refs, const tsidb_problem_out* out, void* cuda_stream);
 
 /* controller.integrate_dv(q, v, dv, dt) (ref:ctrl/WalkController.py:291-295,
  * ref:legacy/biped.py:236-240): v_mean = v + dt/2*dv; v += dt*dv;

@@ -100,6 +100,10 @@ class TsidbAuxOut(C.Structure):
     ]
 
 
+class TsidbProblemOut(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("H", "g", "CE", "ce0", "CI", "ci0", "sizes")]
+
+
 def _fill(arr, values) -> None:
     v = np.asarray(values, dtype=np.float64).ravel()
     for i, x in enumerate(v):
@@ -257,6 +261,10 @@ def load_library() -> C.CDLL:
     lib.tsidb_diagnostics.restype = ip
     lib.tsidb_debug_terms.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp]
     lib.tsidb_debug_terms.restype = ip
+    lib.tsidb_problem_sizes.argtypes = [vp, C.POINTER(ip), C.POINTER(ip), C.POINTER(ip)]
+    lib.tsidb_problem_sizes.restype = ip
+    lib.tsidb_problem_data.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), C.POINTER(TsidbProblemOut), vp]
+    lib.tsidb_problem_data.restype = ip
     _LIB = lib
     return lib
 
@@ -273,4 +281,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_fp64_peak", "tsidb_launch_count", "tsidb_set_timing", "tsidb_set_sched_hint", "tsidb_last_tick_ms",
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
+    "tsidb_problem_sizes", "tsidb_problem_data",
 ]

@@ -178,7 +178,7 @@ static int upload_const(tsidb_handle* h) {
 
 /* everything of tsidb_create that can fail after the handle exists; on any failure the caller destroys the handle
  * (tsidb_destroy tolerates members that were never created), which also returns the constant-memory slot */
-static int create_impl(tsidb_handle* h, const cudaDeviceProp& prop, int max_envs, int device) {
+static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDeviceProp& prop, int max_envs, int device) {
   h->sm_count = prop.multiProcessorCount;
   const size_t smem = ((size_t)TSIDB_WARPS_PER_BLOCK * SM_PER_ENV + MDL_SIZE) * sizeof(double);
   /* Every CTA of the elimination, basis and active-set kernels is one warp; WARPS of them are to be resident per SM
@@ -220,6 +220,8 @@ static int create_impl(tsidb_handle* h, const cudaDeviceProp& prop, int max_envs
   TSIDB_E_ATTR(26, 2, TSIDB_E_WARPS); TSIDB_E_ATTR(26, 1, TSIDB_E_WARPS_LIGHT); TSIDB_E_ATTR(26, 0, TSIDB_E_WARPS_LIGHT);
   TSIDB_E_ATTR(24, 2, TSIDB_E_WARPS); TSIDB_E_ATTR(24, 1, TSIDB_E_WARPS_LIGHT); TSIDB_E_ATTR(24, 0, TSIDB_E_WARPS_LIGHT);
 #undef TSIDB_E_ATTR
+  TSIDB_ATTR(tsidb_problem_kernel<26>, TSIDB_P_SMEM(26), TSIDB_P_CTAS_PER_SM, "QP export kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_problem_kernel<24>, TSIDB_P_SMEM(24), TSIDB_P_CTAS_PER_SM, "QP export kernel", cudaSharedmemCarveoutMaxShared);
 #undef TSIDB_ATTR
   CK(cudaMalloc(&h->counter, TSIDB_NCOUNTER * TSIDB_MAX_CHUNKS * sizeof(int32_t)));
   CK(cudaMalloc(&h->pred, (size_t)max_envs * sizeof(int32_t)));
@@ -232,6 +234,11 @@ static int create_impl(tsidb_handle* h, const cudaDeviceProp& prop, int max_envs
   CK(cudaMalloc(&h->cls_pos, (size_t)max_envs * sizeof(int32_t)));
   CK(cudaMalloc(&h->tables, TBL_SIZE * sizeof(double)));
   if (upload_const(h) != 0) return -2;
+  {
+    double pt[PT_SIZE];
+    tsidb_fill_problem_table(conf, &h->dc, pt);
+    CK(cudaMemcpy(h->tables + TBL_oPROB, pt, sizeof pt, cudaMemcpyHostToDevice));
+  }
   /* host-call staging: inputs q(nq) v(nv) refs(9+24+24+12+12+na); outputs tau(na) ddq(nv) f(24) */
   const int na = h->dc.na, nv = h->dc.nv, nq = h->dc.nq;
   const size_t in_per = nq + nv + 9 + 24 + 24 + 12 + 12 + na, out_per = na + nv + 24;
@@ -295,7 +302,7 @@ extern "C" int tsidb_create(const tsidb_model* model, const tsidb_conf* conf, in
       if (!g_slot_used[device][s]) { g_slot_used[device][s] = true; h->slot = s; break; }
   }
   if (h->slot < 0) { g_err = "tsidb_create: all constant-memory slots of this device are in use"; delete h; return -1; }
-  const int rc = create_impl(h, prop, max_envs, device);
+  const int rc = create_impl(h, conf, prop, max_envs, device);
   if (rc != 0) {
     const std::string keep = g_err; /* tsidb_destroy must not hide the cause */
     tsidb_destroy(h);               /* frees whatever was allocated so far and returns the slot */
@@ -362,6 +369,19 @@ extern "C" int tsidb_set_default_refs(tsidb_handle* h, const double* com9, const
   return upload_const(h);
 }
 
+/* the dynamics kernel over a.n_envs envs on a persistent grid (kernel D of the tick; also the first stage of the QP export) */
+static int launch_dynamics(tsidb_handle* h, const TickArgs& a, cudaStream_t st) {
+  const int warps = TSIDB_WARPS_PER_BLOCK;
+  int blocks = (a.n_envs + warps - 1) / warps;
+  if (blocks > TSIDB_D_CTAS_PER_SM * h->sm_count) blocks = TSIDB_D_CTAS_PER_SM * h->sm_count; /* persistent */
+  const size_t smem = ((size_t)warps * SM_PER_ENV + MDL_SIZE) * sizeof(double);
+  if (h->dc.nv == 26) tsidb_dynamics_kernel<26><<<blocks, 32 * warps, smem, st>>>(a);
+  else tsidb_dynamics_kernel<24><<<blocks, 32 * warps, smem, st>>>(a);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
 /* One tick over a.n_envs envs on stream st.  `base` / `chunk` select a window of the workspaces and a work
  * counter of its own, so that chunks of one host call can be in flight on different streams. */
 static int launch_tick(tsidb_handle* h, TickArgs& a, cudaStream_t st, int base = 0, int chunk = 0) {
@@ -411,14 +431,7 @@ static int launch_tick(tsidb_handle* h, TickArgs& a, cudaStream_t st, int base =
   if (timed) CK(cudaEventRecord(h->ev[1], st));
   {
     NvtxRange r("tsidb:dynamics");
-    const int warps = TSIDB_WARPS_PER_BLOCK;
-    int blocks = (n + warps - 1) / warps;
-    if (blocks > TSIDB_D_CTAS_PER_SM * h->sm_count) blocks = TSIDB_D_CTAS_PER_SM * h->sm_count; /* persistent */
-    const size_t smem = ((size_t)warps * SM_PER_ENV + MDL_SIZE) * sizeof(double);
-    if (h->dc.nv == 26) tsidb_dynamics_kernel<26><<<blocks, 32 * warps, smem, st>>>(a);
-    else tsidb_dynamics_kernel<24><<<blocks, 32 * warps, smem, st>>>(a);
-    CK(cudaGetLastError());
-    h->launches += 1;
+    if (const int rc = launch_dynamics(h, a, st)) return rc;
   }
   if (timed) CK(cudaEventRecord(h->ev[2], st));
   if (!a.kin_only) {
@@ -710,6 +723,56 @@ extern "C" int tsidb_debug_terms(tsidb_handle* h, int env, int n_contacts, doubl
   for (int r = 0; r < 12; r++)
     for (int j = 0; j < nv; j++) JF[r * nv + j] = ea[SE_oJF + r * TSIDB_NVX + j];
   (void)na;
+  return 0;
+}
+
+static void problem_maxima(const tsidb_handle* h, int* n_max, int* neq_max, int* nin_max) {
+  *n_max = h->dc.nv + 24;
+  *neq_max = 18;
+  *nin_max = 2 * (34 + (h->dc.use_tb ? h->dc.na : 0) + (h->dc.use_jb ? h->dc.nv : 0));
+}
+
+extern "C" int tsidb_problem_sizes(const tsidb_handle* h, int* n_max, int* neq_max, int* nin_max) {
+  if (!h || !n_max || !neq_max || !nin_max) { g_err = "tsidb_problem_sizes: null argument"; return -1; }
+  problem_maxima(h, n_max, neq_max, nin_max);
+  return 0;
+}
+
+/* computeProblemData without the solve: the dynamics kernel (no class sort, slot == env, never the single-launch path,
+ * whose images stay in shared memory) leaves every env's images in the handle's workspaces, then the export kernel writes
+ * the compact problem of every env.  pred, the work counters and the timing events are not touched. */
+extern "C" int tsidb_problem_data(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
+                                  const uint8_t* contact_mask, const tsidb_refs* refs, const tsidb_problem_out* out,
+                                  void* cuda_stream) {
+  if (!h || !q || !v || !out) { g_err = "tsidb_problem_data: null argument"; return -1; }
+  if (n_envs <= 0 || n_envs > h->max_envs) { g_err = "tsidb_problem_data: n_envs must be in [1, max_envs]"; return -1; }
+  if (layout != 0 && layout != 1) { g_err = "tsidb_problem_data: layout must be 0 ([N][dof]) or 1 ([dof][N])"; return -1; }
+  for (const double* p : {out->H, out->CE, out->CI})
+    if (((uintptr_t)p & 15) != 0) { g_err = "tsidb_problem_data: H, CE and CI must be 16-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  TickArgs a;
+  memset(&a, 0, sizeof a);
+  a.n_envs = n_envs; a.layout = layout;
+  a.q = q; a.v = v; a.mask = contact_mask;
+  if (refs) {
+    a.r_com = refs->com; a.r_foot[0] = refs->foot_lf; a.r_foot[1] = refs->foot_rf;
+    a.r_contact[0] = refs->contact_lf; a.r_contact[1] = refs->contact_rf; a.r_posture = refs->posture;
+  }
+  a.slot = h->slot;
+  a.tables = h->tables;
+  a.ws = h->ws;
+  a.ws3 = h->ws3;
+  a.perm = nullptr;
+  if (const int rc = launch_dynamics(h, a, st)) return rc;
+  ProblemOut o;
+  o.H = out->H; o.g = out->g; o.CE = out->CE; o.ce0 = out->ce0; o.CI = out->CI; o.ci0 = out->ci0; o.sizes = out->sizes;
+  long blocks = (n_envs + TSIDB_P_CTA_WARPS - 1) / TSIDB_P_CTA_WARPS;
+  if (blocks > (long)TSIDB_P_CTAS_PER_SM * h->sm_count) blocks = (long)TSIDB_P_CTAS_PER_SM * h->sm_count; /* persistent */
+  if (h->dc.nv == 26) tsidb_problem_kernel<26><<<(int)blocks, 32 * TSIDB_P_CTA_WARPS, TSIDB_P_SMEM(26), st>>>(a, o);
+  else tsidb_problem_kernel<24><<<(int)blocks, 32 * TSIDB_P_CTA_WARPS, TSIDB_P_SMEM(24), st>>>(a, o);
+  CK(cudaGetLastError());
+  h->launches += 1;
   return 0;
 }
 

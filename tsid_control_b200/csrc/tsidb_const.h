@@ -108,6 +108,23 @@ struct DevConst {
 #define SE_oSc (SE_oBm + 12)        /* contact mask, pad                         2 */
 #define SE_IMAGE (SE_oSc + 2)       /* doubles handed over per env            1248 */
 
+/* constants of the QP export (tsidb_problem_data), a section of the handle's global table (TBL_oPROB) filled on the
+ * host by tsidb_fill_problem_table: every env shares them and the export reads them with lane-dependent indices */
+#define PT_oHF 0                    /* force block of the Hessian w_freg (W T)^T (W T) + hreg I   12 x 12 */
+#define PT_oB (PT_oHF + 144)        /* Contact6d inequality rows (pyramid 16, normal 1)           17 x 12 */
+#define PT_oT (PT_oB + 204)         /* force generator T                                           6 x 12 */
+#define PT_oTMIN (PT_oT + 72)       /* tau_min, tau_max, v_min, v_max                          4 x 24    */
+#define PT_oTMAX (PT_oTMIN + 24)
+#define PT_oVMIN (PT_oTMAX + 24)
+#define PT_oVMAX (PT_oVMIN + 24)
+#define PT_SIZE (PT_oVMAX + 24)     /*                                                          516       */
+
+/* output arrays of the QP export (tsidb_problem_out of include/tsidb.h); a null pointer: that part is not written */
+struct ProblemOut {
+  double *H, *g, *CE, *ce0, *CI, *ci0;
+  int32_t* sizes;
+};
+
 struct TickArgs {
   int32_t n_envs, layout, pad_;
   const double* q;

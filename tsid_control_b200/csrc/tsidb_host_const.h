@@ -11,6 +11,19 @@
 #include "../../include/tsidb.h"
 #include "tsidb_const.h"
 
+/* force block of the Hessian, identical for every env and foot: w_freg (W T)^T (W T) + hreg I */
+static inline void tsidb_force_hessian(const tsidb_conf* c, const double (*T)[12], double (*Hf)[12]) {
+  for (int i = 0; i < 12; i++)
+    for (int j = 0; j < 12; j++) {
+      double s = 0.0;
+      for (int r = 0; r < 6; r++) {
+        const double wr = c->force_reg_weights[r];
+        s += (wr * T[r][i]) * (wr * T[r][j]);
+      }
+      Hf[i][j] = c->w_force_reg * s + (i == j ? c->hessian_reg : 0.0);
+    }
+}
+
 static inline bool tsidb_fill_devconst(const tsidb_model* m, const tsidb_conf* c, DevConst* D, std::string* err) {
   memset(D, 0, sizeof *D);
   const int nb = m->nb;
@@ -106,15 +119,7 @@ static inline bool tsidb_fill_devconst(const tsidb_model* m, const tsidb_conf* c
 
   /* force block of the Hessian and its factor (identical for all envs and feet) */
   double Hf[12][12];
-  for (int i = 0; i < 12; i++)
-    for (int j = 0; j < 12; j++) {
-      double s = 0.0;
-      for (int r = 0; r < 6; r++) {
-        const double wr = c->force_reg_weights[r];
-        s += (wr * D->T[r][i]) * (wr * D->T[r][j]);
-      }
-      Hf[i][j] = c->w_force_reg * s + (i == j ? c->hessian_reg : 0.0);
-    }
+  tsidb_force_hessian(c, D->T, Hf);
   D->Hf_trace = 0.0;
   for (int i = 0; i < 12; i++) D->Hf_trace += Hf[i][i];
   for (int j = 0; j < 12; j++) {
@@ -143,6 +148,23 @@ static inline bool tsidb_fill_devconst(const tsidb_model* m, const tsidb_conf* c
     D->ref_contact[f][3] = D->ref_contact[f][7] = D->ref_contact[f][11] = 1.0;
   }
   return true;
+}
+
+/* the QP export's section of the global table (PT_* layout, tsidb_const.h), from a filled DevConst */
+static inline void tsidb_fill_problem_table(const tsidb_conf* c, const DevConst* D, double* t) {
+  memset(t, 0, PT_SIZE * sizeof(double));
+  tsidb_force_hessian(c, D->T, reinterpret_cast<double(*)[12]>(t + PT_oHF));
+  /* [UPSTREAM Contact6d::updateForceInequalityConstraints]: four pyramid rows per corner, then the total normal force */
+  for (int i = 0; i < 4; i++)
+    for (int k = 0; k < 3; k++) {
+      for (int r = 0; r < 4; r++) t[PT_oB + (4 * i + r) * 12 + 3 * i + k] = D->fric[r][k];
+      t[PT_oB + 16 * 12 + 3 * i + k] = D->nrm[k];
+    }
+  memcpy(t + PT_oT, D->T, 72 * sizeof(double));
+  memcpy(t + PT_oTMIN, D->tau_min, 23 * sizeof(double));
+  memcpy(t + PT_oTMAX, D->tau_max, 23 * sizeof(double));
+  memcpy(t + PT_oVMIN, D->v_min, 23 * sizeof(double));
+  memcpy(t + PT_oVMAX, D->v_max, 23 * sizeof(double));
 }
 
 #endif

@@ -26,6 +26,8 @@
  *        decode     dv, f, tau = h_a + M_a dv - J_a^T f.   [ref:main.py:126-127]
  *   E and A are instantiated and launched per contact class (nc = 2, 1, 0): every size is a compile-time
  *   constant; the host runs the three class chains E -> A on forked streams (tsidb.cu, launch_tick).
+ *   kernel P  tsidb_problem_kernel  not part of the tick: after kernel D (slot == env) it writes each env's assembled QP
+ *                   (H, g, CE, ce0, CI, ci0) to the caller's arrays instead of solving it (tsidb_problem_data).
  *
  * The file also compiles for the host under tests/emu (lock-step warp emulator that poisons shared memory with
  * NaN) so that the kernel logic can be exercised without a GPU; TSIDB_EMU selects that build.
@@ -201,7 +203,8 @@ TSIDB_DEV void stage_model(const DevConst& C, double* mdl, int tid, int nthreads
 #define TBL_oMDL 0
 #define TBL_oLF ((MDL_SIZE + 1) & ~1)
 #define TBL_oLANE (TBL_oLF + 144)   /* LaneConst of the 32 lanes, value j of lane l at [j][l]: 19 x 32 */
-#define TBL_SIZE (TBL_oLANE + 19 * 32)
+#define TBL_oPROB (TBL_oLANE + 19 * 32)   /* constants of the QP export (PT_*, tsidb_const.h), filled on the host */
+#define TBL_SIZE (TBL_oPROB + PT_SIZE)
 TSIDB_DEV void load_table(double* dst, const double* src, int count /* even */, int tid, int nthreads) {
   const double2* s2 = reinterpret_cast<const double2*>(src);
   double2* d2 = reinterpret_cast<double2*>(dst);
@@ -2254,6 +2257,181 @@ TSIDB_DEV void activeset_env(const DevConst& C, LaneConst& K, double* sm, const 
   __syncwarp();
 }
 
+/* ================================================================= QP export of one env (tsidb_problem_data) */
+/* The problem SolverHQuadProgFast hands to eiquadprog for this env, in the compact variables x = [dv; f of the feet in
+ * contact, LF first], written row-major and zero padded to the handle's maxima (include/tsidb.h).  Everything comes from
+ * the images the dynamics kernel left for this env (slot == env) and from the handle's constants; nothing is solved.
+ * Lanes run over the column pairs of a row and every row leaves as one 16-byte store per lane. */
+template <int NV>
+struct PB {
+  enum : int {
+    oE = 0,                                  /* assembly image                          SE_IMAGE */
+    oMa = SE_IMAGE,                          /* M_a (rows 6.. of M)                  na x SA_LDM */
+    oNle = oMa + (NV - 6) * SA_LDM,          /* nle_a                                          na */
+    oVj = oNle + even_up(NV - 6),            /* joint velocities                               na */
+    oJc = oVj + even_up(NV - 6),             /* Jc = T^T JF of the feet in contact, transposed: [j][12 s + k], nv x 24 */
+    per_env = oJc + NV * 24
+  };
+};
+TSIDB_DEV void st_pair(double* p, double x, double y) { *reinterpret_cast<double2*>(p) = make_double2(x, y); }
+
+/* CI row ri of an env -> (block 0 force / 2 actuation / 3 joint bounds / -1 padding, side, row i, force slot) */
+TSIDB_DEV int ci_block(const DevConst& C, int ri, int nc, int na, int nv, int& side, int& i, int& slot) {
+  int r = ri;
+  for (int s = 0; s < nc; s++) {
+    if (r < 34) { slot = s; side = r >= 17; i = r - 17 * side; return 0; }
+    r -= 34;
+  }
+  if (C.use_tb) {
+    if (r < 2 * na) { side = r >= na; i = r - na * side; return 2; }
+    r -= 2 * na;
+  }
+  if (C.use_jb && r < 2 * nv) { side = r >= nv; i = r - nv * side; return 3; }
+  return -1;
+}
+
+template <int NV>
+TSIDB_DEV void problem_env(const DevConst& C, const double* pt, double* sm, const TickArgs& a, const ProblemOut& o, int env,
+                           int lane) {
+  typedef PB<NV> P;
+  constexpr int nv = NV, na = NV - 6, NX = NV + 24, NEQX = 18;
+  const double BIG = 1e10; /* [UPSTREAM TaskJointBounds] unbounded base rows; Contact6d's open pyramid side */
+  const int nin_x = 2 * (34 + (C.use_tb ? na : 0) + (C.use_jb ? nv : 0));
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  {
+    const double2* s = reinterpret_cast<const double2*>(a.ws3 + (size_t)env * SE_IMAGE);
+    double2* d = reinterpret_cast<double2*>(sm + P::oE);
+    for (int k = lane; k < SE_IMAGE / 2; k += 32) d[k] = s[k];
+  }
+  const int mask = a.mask ? (a.mask[env] & 3) : 3;
+  const int nc = (mask & 1) + ((mask >> 1) & 1);
+  const int n = nv + 12 * nc, neq = 6 + 6 * nc;
+  const int nin = 2 * (17 * nc + (C.use_tb ? na : 0) + (C.use_jb ? nv : 0));
+  const int f0 = (mask & 1) ? 0 : 1; /* foot of force slot 0; slot 1 is RF */
+  {
+    const ALayout L = a_layout(nv, nc);
+    const double* img = a.ws + (size_t)env * SA_IMAGE;
+    const double2* s = reinterpret_cast<const double2*>(img + L.oMa);
+    double2* d = reinterpret_cast<double2*>(sm + P::oMa);
+    for (int k = lane; k < na * SA_LDM / 2; k += 32) d[k] = s[k];
+    if (lane < na) { sm[P::oNle + lane] = img[L.oNle + lane]; sm[P::oVj + lane] = img[L.oVj + lane]; }
+  }
+  __syncwarp();
+  const double* E = sm + P::oE;
+  const double* Ma = sm + P::oMa;
+  double* Jc = sm + P::oJc;
+  if (lane < nv) {
+    for (int s = 0; s < nc; s++) {
+      const int f = s == 0 ? f0 : 1;
+      double jf[6];
+#pragma unroll
+      for (int m = 0; m < 6; m++) jf[m] = E[SE_oJF + (f * 6 + m) * TSIDB_NVX + lane];
+#pragma unroll
+      for (int k = 0; k < 12; k++) {
+        double acc = 0.0;
+#pragma unroll
+        for (int m = 0; m < 6; m++) acc += pt[PT_oT + m * 12 + k] * jf[m];
+        Jc[lane * 24 + 12 * s + k] = acc;
+      }
+    }
+  }
+  __syncwarp();
+  const bool cols = lane < NX / 2; /* this lane's columns 2 lane, 2 lane + 1 */
+  if (o.H && cols) {
+    double* out = o.H + (size_t)env * NX * NX + 2 * lane;
+    for (int i = 0; i < NX; i++) {
+      double x[2];
+#pragma unroll
+      for (int u = 0; u < 2; u++) {
+        const int j = 2 * lane + u;
+        double val = 0.0;
+        if (i < n && j < n) {
+          if (i < nv && j < nv) val = E[SE_oH + (i >= j ? i * SM_LDM + j : j * SM_LDM + i)]; /* lower triangle */
+          else if (i >= nv && j >= nv && (i - nv) / 12 == (j - nv) / 12) val = pt[PT_oHF + ((i - nv) % 12) * 12 + (j - nv) % 12];
+        }
+        x[u] = val;
+      }
+      st_pair(out + i * NX, x[0], x[1]);
+    }
+  }
+  if (o.g)
+    for (int k = lane; k < NX; k += 32) o.g[(size_t)env * NX + k] = k < nv ? E[SE_oG + k] : 0.0;
+  if (o.CE && cols) {
+    double* out = o.CE + (size_t)env * NEQX * NX + 2 * lane;
+    for (int r = 0; r < NEQX; r++) {
+      double x[2];
+#pragma unroll
+      for (int u = 0; u < 2; u++) {
+        const int j = 2 * lane + u;
+        double val = 0.0;
+        if (r < 6) { /* base dynamics: [M_u | -Jc^T] x + h_u = 0 */
+          if (j < nv) val = E[SE_oMu + r * SM_LDM + j];
+          else if (j < n) val = -Jc[r * 24 + j - nv];
+        } else if (r < neq && j < nv) { /* contact motion: JF x - a_des = 0 */
+          const int f = (r < 12) ? f0 : 1;
+          val = E[SE_oJF + (f * 6 + (r - 6) % 6) * TSIDB_NVX + j];
+        }
+        x[u] = val;
+      }
+      st_pair(out + r * NX, x[0], x[1]);
+    }
+  }
+  if (o.ce0 && lane < NEQX) {
+    double val = 0.0;
+    if (lane < 6) val = E[SE_oNle + lane];
+    else if (lane < neq) val = -E[SE_oBm + ((lane < 12) ? f0 : 1) * 6 + (lane - 6) % 6];
+    o.ce0[(size_t)env * NEQX + lane] = val;
+  }
+  if (o.CI && cols) {
+    double* out = o.CI + (size_t)env * nin_x * NX + 2 * lane;
+    for (int ri = 0; ri < nin_x; ri++) {
+      int side = 0, i = 0, slot = 0;
+      const int blk = ci_block(C, ri, nc, na, nv, side, i, slot);
+      double x[2];
+#pragma unroll
+      for (int u = 0; u < 2; u++) {
+        const int j = 2 * lane + u;
+        double val = 0.0;
+        if (blk == 0) {
+          const int k = j - nv - 12 * slot;
+          if (k >= 0 && k < 12) val = pt[PT_oB + i * 12 + k];
+        } else if (blk == 2) { /* [M_a | -Jc_a^T] x + h_a in [tau_min, tau_max] */
+          if (j < nv) val = Ma[i * SA_LDM + j];
+          else if (j < n) val = -Jc[(6 + i) * 24 + j - nv];
+        } else if (blk == 3) {
+          val = (j == i) ? 1.0 : 0.0;
+        }
+        x[u] = side ? -val : val; /* [lower rows: A x - lb >= 0; upper rows: -A x + ub >= 0] */
+      }
+      st_pair(out + ri * NX, x[0], x[1]);
+    }
+  }
+  if (o.ci0) {
+    for (int ri = lane; ri < nin_x; ri += 32) {
+      int side = 0, i = 0, slot = 0;
+      const int blk = ci_block(C, ri, nc, na, nv, side, i, slot);
+      double lb = 0.0, ub = 0.0;
+      if (blk == 0) {
+        lb = (i < 16) ? -BIG : C.fmin;
+        ub = (i < 16) ? 0.0 : C.fmax;
+      } else if (blk == 2) {
+        lb = pt[PT_oTMIN + i] - sm[P::oNle + i];
+        ub = pt[PT_oTMAX + i] - sm[P::oNle + i];
+      } else if (blk == 3) {
+        lb = -BIG; ub = BIG;
+        if (i >= 6) {
+          const double vj = sm[P::oVj + i - 6];
+          const double hi = (pt[PT_oVMAX + i - 6] - vj) / C.jb_dt, lo = (pt[PT_oVMIN + i - 6] - vj) / C.jb_dt;
+          ub = hi < BIG ? hi : BIG;
+          lb = lo > -BIG ? lo : -BIG;
+        }
+      }
+      o.ci0[(size_t)env * nin_x + ri] = (blk < 0) ? 0.0 : (side ? ub : -lb);
+    }
+  }
+  if (o.sizes && lane < 3) o.sizes[(size_t)env * 3 + lane] = (lane == 0) ? n : ((lane == 1) ? neq : nin);
+}
+
 #ifndef TSIDB_EMU
 /* class sort: slots ordered double support, single support, flight, so that the warps of a CTA round in
  * kernel F have equal trip counts and kernel A starts with the longest jobs. */
@@ -2441,6 +2619,25 @@ tsidb_activeset_kernel(const TickArgs a) {
     k = kn;
     env = envn;
   }
+}
+
+/* QP export (tsidb_problem_data), after the dynamics kernel ran with slot == env: one warp per env on a persistent grid.
+ * It is bound by its HBM writes (~93 KB per double-support robot/v1 env), so it does nothing but form and store rows. */
+#define TSIDB_P_CTA_WARPS 4
+#define TSIDB_P_CTAS_PER_SM 2
+#define TSIDB_P_SMEM(NV) (((size_t)PT_SIZE + (size_t)TSIDB_P_CTA_WARPS * PB<NV>::per_env) * sizeof(double))
+template <int NV>
+__global__ void __launch_bounds__(32 * TSIDB_P_CTA_WARPS, TSIDB_P_CTAS_PER_SM)
+tsidb_problem_kernel(const TickArgs a, const ProblemOut o) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  double* pt = smem;
+  double* sm = smem + PT_SIZE + wid * PB<NV>::per_env;
+  load_table(pt, a.tables + TBL_oPROB, PT_SIZE, threadIdx.x, blockDim.x);
+  __syncthreads();
+  const DevConst& C = g_const[a.slot];
+  for (int env = blockIdx.x * TSIDB_P_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_P_CTA_WARPS)
+    problem_env<NV>(C, pt, sm, a, o, env, lane);
 }
 
 /* ---- Small batches: the whole tick of one env in ONE launch ----

@@ -388,6 +388,45 @@ class TsidEngine:
                                          res["support"].data_ptr(), self._stream()), "tsidb_diagnostics")
         return res
 
+    PROBLEM_PARTS = ("H", "g", "CE", "ce0", "CI", "ci0")
+
+    def problem_sizes(self) -> Tuple[int, int, int]:
+        """(n_max, neq_max, nin_max): the padding of :meth:`problem_data`'s arrays (tsidb_problem_sizes)."""
+        n, neq, nin = C.c_int(), C.c_int(), C.c_int()
+        check(self.lib.tsidb_problem_sizes(self.h, C.byref(n), C.byref(neq), C.byref(nin)), "tsidb_problem_sizes")
+        return n.value, neq.value, nin.value
+
+    def problem_data(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                     refs: Optional[Dict[str, torch.Tensor]] = None, parts=PROBLEM_PARTS) -> Dict[str, torch.Tensor]:
+        """computeProblemData without the solve (tsidb_problem_data): for every env the QP SolverHQuadProgFast hands to
+        eiquadprog, min 1/2 x'Hx + g'x s.t. CE x + ce0 = 0, CI x + ci0 >= 0, in x = [dv; f of the feet in contact, LF
+        first].  Returns new CUDA tensors H [N,n,n], g [N,n], CE [N,18,n], ce0 [N,18], CI [N,nin,n], ci0 [N,nin] (the
+        requested `parts`, padded with zeros to problem_sizes()) and sizes [N,3] int32 = (n, neq, nin) of each env.
+        Inputs as in :meth:`compute`; a later tick's results do not depend on this call."""
+        n = q.shape[0]
+        self._chk(q, n, self.nq, "q")
+        self._chk(v, n, self.nv, "v")
+        if contact_mask is not None:
+            if contact_mask.dtype is not torch.uint8 or not contact_mask.is_cuda or contact_mask.get_device() != self._dev_index \
+                    or contact_mask.shape != (n,):
+                raise TypeError("contact_mask: expected a uint8 [N] tensor on the engine's device")
+        unknown = set(parts) - set(self.PROBLEM_PARTS)
+        if unknown:
+            raise ValueError(f"parts: unknown {sorted(unknown)}; choose from {self.PROBLEM_PARTS}")
+        r = TsidbRefs()
+        for k, nd in self._ref_dims:
+            t = refs.get(k) if refs else None
+            setattr(r, k, None if t is None else self._chk(t, n, nd, k).data_ptr())
+        nx, neq, nin = self.problem_sizes()
+        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin)}
+        out = {k: torch.empty(shapes[k], dtype=torch.float64, device=self.device) for k in parts}
+        out["sizes"] = torch.empty((n, 3), dtype=torch.int32, device=self.device)
+        po = _capi.TsidbProblemOut(**{k: t.data_ptr() for k, t in out.items()})
+        check(self.lib.tsidb_problem_data(self.h, n, 0, q.data_ptr(), v.data_ptr(),
+                                          contact_mask.data_ptr() if contact_mask is not None else None, C.byref(r),
+                                          C.byref(po), self._stream()), "tsidb_problem_data")
+        return out
+
     def ci_row(self, block: int, side: int, i: int) -> int:
         return int(self.lib.tsidb_ci_row(self.h, block, side, i))
 

@@ -107,8 +107,25 @@ class Contact(Task):
 
 
 class HQPData:
-    def __init__(self, t, q, v, sizes):
+    """What formulation.computeProblemData returns: the state, the sizes and, read on first access, the assembled QP of
+    the single-robot view in the reference's variable and row order (SolverHQuadProgFast's input):
+    min 1/2 x'Hx + g'x  s.t.  CE x + ce0 = 0,  CI x + ci0 >= 0, x = [dv; f of the contacts in insertion order].
+    The matrices are formed on the device at the first access of any of them (TsidEngine.problem_data), with the
+    contacts of the computeProblemData call and the task references current at that access."""
+
+    PARTS = ("H", "g", "CE", "ce0", "CI", "ci0")
+
+    def __init__(self, t, q, v, sizes, formulation=None, contact_order=(), ci_order=()):
         self.t, self.q, self.v, self.sizes = t, q, v, sizes
+        self._formulation, self._contact_order, self._ci_order = formulation, list(contact_order), list(ci_order)
+        self._problem = None
+
+    def __getattr__(self, name):
+        if name in HQPData.PARTS and self.__dict__.get("_formulation") is not None:
+            if self._problem is None:
+                self._problem = self._formulation._problem(self)
+            return self._problem[name]
+        raise AttributeError(name)
 
     def print_all(self) -> None:
         n, neq, nin = self.sizes
@@ -198,8 +215,36 @@ class FormulationMirror:
         com, lf, rf = c.engine.kinematics(qd, vd)
         self._data.com = com[0].cpu().numpy()
         self._data.foot = [lf[0].cpu().numpy(), rf[0].cpu().numpy()]
-        self._pending = HQPData(t, qd, vd, (self.nVar, self.nEq, self.nIn))
+        self._pending = HQPData(t, qd, vd, (self.nVar, self.nEq, self.nIn), self, c._contact_order, c._ci_order)
         return self._pending
+
+    def _problem(self, hqp: HQPData) -> Dict[str, np.ndarray]:
+        """The exported QP of env 0 (compact order: contacts LF first, CI blocks [LF, RF, actuation, joint bounds]),
+        permuted into the order of hqp's contacts and level-0 blocks."""
+        c = self._c
+        e = c.engine
+        mask = sum(1 << f for f in hqp._contact_order)
+        refs = {k: t[0:1].contiguous() for k, t in c.refs.items()}
+        out = e.problem_data(hqp.q, hqp.v, torch.tensor([mask], dtype=torch.uint8, device=e.device), refs)
+        P = {k: out[k][0].cpu().numpy() for k in HQPData.PARTS}
+        nv, feet = e.nv, sorted(hqp._contact_order)
+        var = list(range(nv))
+        eq = list(range(6))
+        for f in hqp._contact_order:
+            k = feet.index(f)
+            var += range(nv + 12 * k, nv + 12 * k + 12)
+            eq += range(6 + 6 * k, 12 + 6 * k)
+        rows = {0: 17, 1: 17, 2: e.na, 3: e.nv}
+        off, start = 0, {}
+        for blk in feet + [b for b in (2, 3) if b in hqp._ci_order]:
+            start[blk] = off
+            off += 2 * rows[blk]
+        ci: List[int] = []
+        for blk in hqp._ci_order:
+            ci += range(start[blk], start[blk] + 2 * rows[blk])
+        ix = np.ix_
+        return {"H": P["H"][ix(var, var)], "g": P["g"][var], "CE": P["CE"][ix(eq, var)], "ce0": P["ce0"][eq],
+                "CI": P["CI"][ix(ci, var)], "ci0": P["ci0"][ci]}
 
     def data(self) -> Data:
         return self._data
