@@ -249,6 +249,10 @@ typedef struct tsidb_problem_out {
   double* CI;     /* [N][nin_max][n_max]  one-sided rows                                */
   double* ci0;    /* [N][nin_max]                                                       */
   int32_t* sizes; /* [N][3]  n, neq, nin of this env                                    */
+  /* The struct grew at its end with the actuation map, tau = TA x + ta0 (getActuatorForces: TA = [M_a | -J_c,a^T],
+   * ta0 = h_a); a caller that zero-initialises the struct keeps the six parts above and nothing more. */
+  double* TA;     /* [N][na][n_max]      16-byte aligned like H, CE and CI                */
+  double* ta0;    /* [N][na]                                                            */
 } tsidb_problem_out;
 
 int tsidb_problem_sizes(const tsidb_handle* h, int* n_max, int* neq_max, int* nin_max);
@@ -259,6 +263,35 @@ int tsidb_problem_sizes(const tsidb_handle* h, int* n_max, int* neq_max, int* ni
  * images afterwards. */
 int tsidb_problem_data(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
                        const uint8_t* contact_mask, const tsidb_refs* refs, const tsidb_problem_out* out, void* cuda_stream);
+
+/* ---- solving a caller-supplied QP ---------------------------------------------------------------------------------
+ * tsidb_qp_solve runs eiquadprog-fast (the solver SolverHQuadProgFast calls, with the handle's conf.max_iter) on n_envs
+ * problems in the layout tsidb_problem_data writes, possibly modified or enlarged by the caller: qp->H, g, CE, ce0, CI,
+ * ci0 and sizes are read (DEVICE memory, per env row-major with the strides n_max, neq_max, nin_max, which may exceed
+ * tsidb_problem_sizes).  Nothing outside an env's own (n, neq, nin) = qp->sizes[e] is read, so padding may hold anything.
+ * Required: H, g, sizes, out->x, out->status; CE and ce0 when neq_max > 0; CI and ci0 when nin_max > 0; TA and ta0 when
+ * out->tau is given.  n_max <= TSIDB_QP_MAX_N, neq_max <= n_max, nin_max <= TSIDB_QP_MAX_NIN.  Any other output pointer
+ * may be NULL.  An env whose sizes violate 1 <= n <= n_max, 0 <= neq <= min(n, neq_max), 0 <= nin <= nin_max gets
+ * TSIDB_STATUS_ERROR and zero outputs; the rest of the batch is solved.  Statuses as the tick maps eiquadprog's result
+ * (H not positive definite or an unbounded step: INFEASIBLE; max_iter: MAX_ITER_REACHED; a redundant equality row:
+ * ERROR); x, the working set and the multipliers are written for OPTIMAL and MAX_ITER_REACHED, zeros (active: -1)
+ * otherwise.  At the optimum H x + g = CI^T lambda + CE^T lambda_eq over the working set.
+ * The call uses none of the handle's workspaces or forecast (only its launch counter), so it may be enqueued on any
+ * stream, also while a tick of the same handle runs on another one.  Asynchronous on cuda_stream, no host round trip. */
+#define TSIDB_QP_MAX_N 64
+#define TSIDB_QP_MAX_NIN 512
+typedef struct tsidb_qp_out {
+  double* x;          /* [N][n_max]    primal solution, in the caller's variable order                              */
+  int32_t* status;    /* [N]           TSIDB_STATUS_*                                                               */
+  int32_t* iters;     /* [N]           eiquadprog iteration count                                                   */
+  int32_t* active;    /* [N][n_max]    CI rows of the final working set in working-set order, -1 padded             */
+  double* lambda;     /* [N][n_max]    their multipliers, same order                                                */
+  double* lambda_eq;  /* [N][neq_max]  multipliers of the equality rows                                             */
+  double* tau;        /* [N][na]       TA x + ta0                                                                   */
+} tsidb_qp_out;
+
+int tsidb_qp_solve(tsidb_handle* h, int n_envs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* qp,
+                   const tsidb_qp_out* out, void* cuda_stream);
 
 /* controller.integrate_dv(q, v, dv, dt) (ref:ctrl/WalkController.py:291-295,
  * ref:legacy/biped.py:236-240): v_mean = v + dt/2*dv; v += dt*dv;

@@ -101,7 +101,12 @@ class TsidbAuxOut(C.Structure):
 
 
 class TsidbProblemOut(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("H", "g", "CE", "ce0", "CI", "ci0", "sizes")]
+    # TA, ta0 were appended to the C struct; ctypes leaves unnamed fields NULL, so older callers are unchanged
+    _fields_ = [(k, C.c_void_p) for k in ("H", "g", "CE", "ce0", "CI", "ci0", "sizes", "TA", "ta0")]
+
+
+class TsidbQpOut(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("x", "status", "iters", "active", "lambda", "lambda_eq", "tau")]
 
 
 def _fill(arr, values) -> None:
@@ -265,6 +270,8 @@ def load_library() -> C.CDLL:
     lib.tsidb_problem_sizes.restype = ip
     lib.tsidb_problem_data.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), C.POINTER(TsidbProblemOut), vp]
     lib.tsidb_problem_data.restype = ip
+    lib.tsidb_qp_solve.argtypes = [vp, ip, ip, ip, ip, C.POINTER(TsidbProblemOut), C.POINTER(TsidbQpOut), vp]
+    lib.tsidb_qp_solve.restype = ip
     _LIB = lib
     return lib
 
@@ -281,5 +288,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_fp64_peak", "tsidb_launch_count", "tsidb_set_timing", "tsidb_set_sched_hint", "tsidb_last_tick_ms",
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
-    "tsidb_problem_sizes", "tsidb_problem_data",
+    "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve",
 ]

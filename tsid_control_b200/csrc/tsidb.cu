@@ -222,6 +222,8 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
 #undef TSIDB_E_ATTR
   TSIDB_ATTR(tsidb_problem_kernel<26>, TSIDB_P_SMEM(26), TSIDB_P_CTAS_PER_SM, "QP export kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_problem_kernel<24>, TSIDB_P_SMEM(24), TSIDB_P_CTAS_PER_SM, "QP export kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_qp_kernel, qp_layout(TSIDB_QP_MAX_N, TSIDB_QP_MAX_NIN).per_env * sizeof(double), 1, "generic QP kernel",
+             cudaSharedmemCarveoutMaxShared);
 #undef TSIDB_ATTR
   CK(cudaMalloc(&h->counter, TSIDB_NCOUNTER * TSIDB_MAX_CHUNKS * sizeof(int32_t)));
   CK(cudaMalloc(&h->pred, (size_t)max_envs * sizeof(int32_t)));
@@ -749,6 +751,7 @@ extern "C" int tsidb_problem_data(tsidb_handle* h, int n_envs, int layout, const
   if (layout != 0 && layout != 1) { g_err = "tsidb_problem_data: layout must be 0 ([N][dof]) or 1 ([dof][N])"; return -1; }
   for (const double* p : {out->H, out->CE, out->CI})
     if (((uintptr_t)p & 15) != 0) { g_err = "tsidb_problem_data: H, CE and CI must be 16-byte aligned"; return -1; }
+  if (((uintptr_t)out->TA & 15) != 0) { g_err = "tsidb_problem_data: TA must be 16-byte aligned"; return -1; }
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   TickArgs a;
@@ -767,10 +770,55 @@ extern "C" int tsidb_problem_data(tsidb_handle* h, int n_envs, int layout, const
   if (const int rc = launch_dynamics(h, a, st)) return rc;
   ProblemOut o;
   o.H = out->H; o.g = out->g; o.CE = out->CE; o.ce0 = out->ce0; o.CI = out->CI; o.ci0 = out->ci0; o.sizes = out->sizes;
+  o.TA = out->TA; o.ta0 = out->ta0;
   long blocks = (n_envs + TSIDB_P_CTA_WARPS - 1) / TSIDB_P_CTA_WARPS;
   if (blocks > (long)TSIDB_P_CTAS_PER_SM * h->sm_count) blocks = (long)TSIDB_P_CTAS_PER_SM * h->sm_count; /* persistent */
   if (h->dc.nv == 26) tsidb_problem_kernel<26><<<(int)blocks, 32 * TSIDB_P_CTA_WARPS, TSIDB_P_SMEM(26), st>>>(a, o);
   else tsidb_problem_kernel<24><<<(int)blocks, 32 * TSIDB_P_CTA_WARPS, TSIDB_P_SMEM(24), st>>>(a, o);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
+/* eiquadprog-fast on caller-supplied problems: one launch of the generic QP kernel, no workspace of the handle */
+extern "C" int tsidb_qp_solve(tsidb_handle* h, int n_envs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* qp,
+                              const tsidb_qp_out* out, void* cuda_stream) {
+  if (!h || !qp || !out) { g_err = "tsidb_qp_solve: null argument"; return -1; }
+  if (n_envs <= 0) { g_err = "tsidb_qp_solve: n_envs must be positive"; return -1; }
+  if (n_max < 1 || n_max > TSIDB_QP_MAX_N || neq_max < 0 || neq_max > n_max || nin_max < 0 || nin_max > TSIDB_QP_MAX_NIN) {
+    g_err = "tsidb_qp_solve: strides must satisfy 1 <= n_max <= TSIDB_QP_MAX_N (64), 0 <= neq_max <= n_max, "
+            "0 <= nin_max <= TSIDB_QP_MAX_NIN (512)";
+    return -1;
+  }
+  if (!qp->H || !qp->g || !qp->sizes || !out->x || !out->status) {
+    g_err = "tsidb_qp_solve: H, g, sizes, x and status are required";
+    return -1;
+  }
+  if ((neq_max > 0 && (!qp->CE || !qp->ce0)) || (nin_max > 0 && (!qp->CI || !qp->ci0))) {
+    g_err = "tsidb_qp_solve: CE and ce0 are required when neq_max > 0, CI and ci0 when nin_max > 0";
+    return -1;
+  }
+  if (out->tau && (!qp->TA || !qp->ta0)) { g_err = "tsidb_qp_solve: tau needs TA and ta0"; return -1; }
+  for (const void* p : {(const void*)qp->H, (const void*)qp->g, (const void*)qp->CE, (const void*)qp->ce0, (const void*)qp->CI,
+                        (const void*)qp->ci0, (const void*)qp->TA, (const void*)qp->ta0, (const void*)out->x,
+                        (const void*)out->lambda, (const void*)out->lambda_eq, (const void*)out->tau})
+    if (((uintptr_t)p & 7) != 0) { g_err = "tsidb_qp_solve: fp64 arrays must be 8-byte aligned"; return -1; }
+  for (const void* p : {(const void*)qp->sizes, (const void*)out->status, (const void*)out->iters, (const void*)out->active})
+    if (((uintptr_t)p & 3) != 0) { g_err = "tsidb_qp_solve: int32 arrays must be 4-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  QpArgs q;
+  q.n_envs = n_envs; q.n_max = n_max; q.neq_max = neq_max; q.nin_max = nin_max; q.na = h->dc.na; q.max_iter = h->dc.max_iter;
+  q.H = qp->H; q.g = qp->g; q.CE = qp->CE; q.ce0 = qp->ce0; q.CI = qp->CI; q.ci0 = qp->ci0; q.TA = qp->TA; q.ta0 = qp->ta0;
+  q.sizes = qp->sizes;
+  q.x = out->x; q.status = out->status; q.iters = out->iters; q.active = out->active;
+  q.lambda = out->lambda; q.lambda_eq = out->lambda_eq; q.tau = out->tau;
+  const size_t smem = qp_layout(n_max, nin_max).per_env * sizeof(double);
+  int per_sm = 0;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tsidb_qp_kernel, 32, smem));
+  if (per_sm < 1) { g_err = "tsidb_qp_solve: the kernel does not fit an SM"; return -2; }
+  long blocks = (long)per_sm * h->sm_count; /* persistent */
+  if (blocks > n_envs) blocks = n_envs;
+  tsidb_qp_kernel<<<(int)blocks, 32, smem, (cudaStream_t)cuda_stream>>>(q);
   CK(cudaGetLastError());
   h->launches += 1;
   return 0;

@@ -123,6 +123,18 @@ struct DevConst {
 struct ProblemOut {
   double *H, *g, *CE, *ce0, *CI, *ci0;
   int32_t* sizes;
+  double *TA, *ta0; /* actuation map tau = TA x + ta0 */
+};
+
+/* arguments of the generic QP solve (tsidb_qp_solve): caller-supplied problems in the layout of tsidb_problem_out, the
+ * caller's strides, and the outputs of tsidb_qp_out (include/tsidb.h) */
+struct QpArgs {
+  int32_t n_envs, n_max, neq_max, nin_max, na, max_iter;
+  const double *H, *g, *CE, *ce0, *CI, *ci0, *TA, *ta0;
+  const int32_t* sizes;
+  double* x;
+  int32_t *status, *iters, *active;
+  double *lambda, *lambda_eq, *tau;
 };
 
 struct TickArgs {

@@ -2429,7 +2429,470 @@ TSIDB_DEV void problem_env(const DevConst& C, const double* pt, double* sm, cons
       o.ci0[(size_t)env * nin_x + ri] = (blk < 0) ? 0.0 : (side ? ub : -lb);
     }
   }
+  if (o.TA && cols) { /* getActuatorForces: tau = [M_a | -Jc_a^T] x + h_a */
+    double* out = o.TA + (size_t)env * na * NX + 2 * lane;
+    for (int r = 0; r < na; r++) {
+      double x[2];
+#pragma unroll
+      for (int u = 0; u < 2; u++) {
+        const int j = 2 * lane + u;
+        x[u] = (j < nv) ? Ma[r * SA_LDM + j] : ((j < n) ? -Jc[(6 + r) * 24 + j - nv] : 0.0);
+      }
+      st_pair(out + r * NX, x[0], x[1]);
+    }
+  }
+  if (o.ta0)
+    for (int r = lane; r < na; r += 32) o.ta0[(size_t)env * na + r] = sm[P::oNle + r];
   if (o.sizes && lane < 3) o.sizes[(size_t)env * 3 + lane] = (lane == 0) ? n : ((lane == 1) ? neq : nin);
+}
+
+/* ================================================================= generic QP solve of one env (tsidb_qp_solve) */
+/* eiquadprog-fast solve_quadprog on a caller-supplied problem, min 1/2 x'Hx + g'x s.t. CE x + ce0 = 0, CI x + ci0 >= 0,
+ * step for step as the oracle's eq_solve states it: LLT of H, J = L^-T, x0 = -H^-1 g, the equalities added one by one,
+ * then the dual active-set passes (most violated row first, lowest index on ties; psi stopping test; Givens add/delete).
+ * J, R and the per-row state live in shared memory; lanes run over rows or columns of J and R (row k / column c: lanes
+ * k % 32, two per lane at n = 64), every scalar that steers the iteration is computed identically by all lanes, so the
+ * control flow is warp-uniform.  Sums over k keep the oracle's order where a lane owns the whole sum (d = J'np,
+ * z = J2 d2, the violation scan); the triangular solves run column-oriented and the dot products as warp sums. */
+#define QP_SLOTS (TSIDB_QP_MAX_N / 32)
+struct QpLayout {
+  int ld;                                            /* row stride of J and R: odd, so column walks are conflict-free */
+  int oJ, oR, ox, oxo, od, oz, or_, onp, ou, ouo, os; /* doubles */
+  int oA, oAo, oiai, oix;                            /* int32, from sm + oI */
+  int oI, per_env;
+};
+TSIDB_HD inline QpLayout qp_layout(int n_max, int nin_max) {
+  QpLayout L;
+  L.ld = n_max | 1;
+  L.oJ = 0;
+  L.oR = L.oJ + n_max * L.ld;
+  L.ox = L.oR + n_max * L.ld;
+  L.oxo = L.ox + n_max;
+  L.od = L.oxo + n_max;
+  L.oz = L.od + n_max;
+  L.or_ = L.oz + n_max;
+  L.onp = L.or_ + n_max;
+  L.ou = L.onp + n_max;
+  L.ouo = L.ou + n_max + 1;
+  L.os = L.ouo + n_max + 1;
+  L.oI = L.os + nin_max;
+  L.oA = 0;
+  L.oAo = n_max + 1;
+  L.oiai = 2 * (n_max + 1);
+  L.oix = L.oiai + nin_max;
+  L.per_env = L.oI + (L.oix + nin_max + 1) / 2;
+  L.per_env += L.per_env & 1; /* every env's area starts 16-byte aligned */
+  return L;
+}
+
+TSIDB_DEV double eq_distance(double a, double b) {
+  const double a1 = fabs(a), b1 = fabs(b);
+  if (a1 > b1) { const double t = b1 / a1; return a1 * sqrt(1.0 + t * t); }
+  if (b1 > a1) { const double t = a1 / b1; return b1 * sqrt(1.0 + t * t); }
+  return a1 * sqrt(2.0);
+}
+
+/* (value, index) argmin over the warp: the smallest value, the lowest index among equal values; idx < 0 = no candidate.
+ * The butterfly leaves the same pair in every lane. */
+TSIDB_DEV void warp_argmin(double& val, int& idx) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ov = __shfl_xor_sync(FULL, val, o);
+    const int oi = __shfl_xor_sync(FULL, idx, o);
+    if (oi >= 0 && (idx < 0 || ov < val || (ov == val && oi < idx))) { val = ov; idx = oi; }
+  }
+}
+
+struct QpEnv {
+  int n, nm, ld;
+  double *J, *R, *x, *xo, *d, *z, *r, *np, *u, *uo, *s;
+  int *A, *Ao, *iai, *iax;
+};
+
+/* d = J' np (lane per column, k ascending) */
+TSIDB_DEV void qp_compute_d(const QpEnv& E, int lane) {
+  for (int c = lane; c < E.n; c += 32) {
+    double s = 0.0;
+    for (int k = 0; k < E.n; k++) s += E.J[k * E.ld + c] * E.np[k];
+    E.d[c] = s;
+  }
+}
+/* z = J[:, iq:] d[iq:] (lane per row, k ascending; zero when iq >= n) */
+TSIDB_DEV void qp_update_z(const QpEnv& E, int iq, int lane) {
+  for (int i = lane; i < E.n; i += 32) {
+    double s = 0.0;
+    for (int k = iq; k < E.n; k++) s += E.J[i * E.ld + k] * E.d[k];
+    E.z[i] = s;
+  }
+}
+/* R[:iq, :iq] r = d[:iq], column-oriented back substitution */
+TSIDB_DEV void qp_update_r(const QpEnv& E, int iq, int lane) {
+  double acc[QP_SLOTS];
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++) acc[t] = (lane + 32 * t < iq) ? E.d[lane + 32 * t] : 0.0;
+  for (int i = iq - 1; i >= 0; i--) {
+    const double ri = __shfl_sync(FULL, (i >> 5) ? acc[QP_SLOTS - 1] : acc[0], i & 31) / E.R[i * E.ld + i];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int m = lane + 32 * t;
+      if (m < i) acc[t] -= E.R[m * E.ld + i] * ri;
+      else if (m == i) acc[t] = ri;
+    }
+  }
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++)
+    if (lane + 32 * t < iq) E.r[lane + 32 * t] = acc[t];
+  __syncwarp();
+}
+/* add_constraint: Givens rotations that zero d[iq+1..n-1] into J, then the new column of R; false when the new column is
+ * (numerically) dependent.  d is read by every lane and carried in registers; lane 0 writes it back. */
+TSIDB_DEV bool qp_add_constraint(const QpEnv& E, int& iq, double& R_norm, int lane) {
+  const int n = E.n, ld = E.ld;
+  if (n - 1 >= iq + 1) {
+    double cur = E.d[n - 1];
+    for (int j = n - 1; j >= iq + 1; j--) {
+      double cc = E.d[j - 1], ss = cur;
+      const double h = eq_distance(cc, ss);
+      if (h == 0.0) { cur = cc; continue; }
+      ss = ss / h;
+      cc = cc / h;
+      if (cc < 0) { cc = -cc; ss = -ss; cur = -h; }
+      else cur = h;
+      const double xny = ss / (1.0 + cc);
+      for (int k = lane; k < n; k += 32) {
+        const double t1 = E.J[k * ld + j - 1], t2 = E.J[k * ld + j];
+        const double a = t1 * cc + t2 * ss;
+        E.J[k * ld + j - 1] = a;
+        E.J[k * ld + j] = xny * (t1 + a) - t2;
+      }
+    }
+    __syncwarp();
+    if (lane == 0) {
+      E.d[iq] = cur;
+      for (int j = iq + 1; j < n; j++) E.d[j] = 0.0;
+    }
+    __syncwarp();
+  }
+  iq++;
+  for (int i = lane; i < iq; i += 32) E.R[i * ld + iq - 1] = E.d[i];
+  __syncwarp();
+  const double dl = fabs(E.d[iq - 1]);
+  if (dl <= TS_EPS * R_norm) return false;
+  if (dl > R_norm) R_norm = dl;
+  return true;
+}
+/* delete_constraint: drop inequality row l from the working set, restore R to triangular with Givens rotations */
+TSIDB_DEV void qp_delete_constraint(const QpEnv& E, int neq, int& iq, int l, int lane) {
+  const int n = E.n, ld = E.ld;
+  int qq = 0;
+  for (int i = neq; i < iq; i++)
+    if (E.A[i] == l) { qq = i; break; }
+  for (int k = lane; k < n; k += 32)
+    for (int i = qq; i < iq - 1; i++) E.R[k * ld + i] = E.R[k * ld + i + 1];
+  __syncwarp();
+  if (lane == 0) {
+    for (int i = qq; i < iq - 1; i++) { E.A[i] = E.A[i + 1]; E.u[i] = E.u[i + 1]; }
+    E.A[iq - 1] = E.A[iq];
+    E.u[iq - 1] = E.u[iq];
+    E.A[iq] = 0;
+    E.u[iq] = 0.0;
+  }
+  for (int j = lane; j < iq; j += 32) E.R[j * ld + iq - 1] = 0.0;
+  __syncwarp();
+  iq--;
+  if (iq == 0) return;
+  for (int j = qq; j < iq; j++) {
+    double cc = E.R[j * ld + j], ss = E.R[(j + 1) * ld + j];
+    const double h = eq_distance(cc, ss);
+    if (h == 0.0) continue;
+    cc = cc / h;
+    ss = ss / h;
+    __syncwarp(); /* every lane has read the pivot pair */
+    if (lane == 0) E.R[(j + 1) * ld + j] = 0.0;
+    if (cc < 0) {
+      if (lane == 0) E.R[j * ld + j] = -h;
+      cc = -cc;
+      ss = -ss;
+    } else if (lane == 0) E.R[j * ld + j] = h;
+    const double xny = ss / (1.0 + cc);
+    for (int k = j + 1 + lane; k < iq; k += 32) {
+      const double t1 = E.R[j * ld + k], t2 = E.R[(j + 1) * ld + k];
+      const double a = t1 * cc + t2 * ss;
+      E.R[j * ld + k] = a;
+      E.R[(j + 1) * ld + k] = xny * (t1 + a) - t2;
+    }
+    for (int k = lane; k < n; k += 32) {
+      const double t1 = E.J[k * ld + j], t2 = E.J[k * ld + j + 1];
+      const double a = t1 * cc + t2 * ss;
+      E.J[k * ld + j] = a;
+      E.J[k * ld + j + 1] = xny * (a + t1) - t2;
+    }
+    __syncwarp();
+  }
+}
+
+/* eiquadprog-fast result codes (the oracle's eq_solve) */
+enum { QP_OPTIMAL = 0, QP_INFEASIBLE = 1, QP_UNBOUNDED = 2, QP_MAX_ITER = 3, QP_REDUNDANT_EQ = 4 };
+
+/* one env; sm holds qp_layout(q.n_max, q.nin_max).per_env doubles of this warp */
+TSIDB_DEV void qp_env(const QpArgs& q, double* sm, int env, int lane) {
+  const QpLayout Ly = qp_layout(q.n_max, q.nin_max);
+  const int nm = q.n_max, ld = Ly.ld;
+  int* smi = reinterpret_cast<int*>(sm + Ly.oI);
+  QpEnv E;
+  E.nm = nm; E.ld = ld;
+  E.J = sm + Ly.oJ; E.R = sm + Ly.oR; E.x = sm + Ly.ox; E.xo = sm + Ly.oxo; E.d = sm + Ly.od; E.z = sm + Ly.oz;
+  E.r = sm + Ly.or_; E.np = sm + Ly.onp; E.u = sm + Ly.ou; E.uo = sm + Ly.ouo; E.s = sm + Ly.os;
+  E.A = smi + Ly.oA; E.Ao = smi + Ly.oAo; E.iai = smi + Ly.oiai; E.iax = smi + Ly.oix;
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  const int n = q.sizes[(size_t)env * 3], neq = q.sizes[(size_t)env * 3 + 1], nin = q.sizes[(size_t)env * 3 + 2];
+  E.n = n;
+  int res = QP_REDUNDANT_EQ, iter = 0, iq = 0;
+  const bool valid = n >= 1 && n <= nm && neq >= 0 && neq <= n && neq <= q.neq_max && nin >= 0 && nin <= q.nin_max;
+  if (valid) {
+    const double* H = q.H + (size_t)env * nm * nm;
+    const double* g = q.g + (size_t)env * nm;
+    const double* CE = q.CE + (size_t)env * q.neq_max * nm;
+    const double* ce0 = q.ce0 + (size_t)env * q.neq_max;
+    const double* CI = q.CI + (size_t)env * q.nin_max * nm;
+    const double* ci0 = q.ci0 + (size_t)env * q.nin_max;
+    double* J = E.J;
+    double* R = E.R;
+    double* L = E.R; /* the factor lives where R goes; R is cleared once J and x0 are formed */
+    double c1 = 0.0, c2 = 0.0, R_norm = 1.0;
+    int ip = 0, l = 0;
+    double ss = 0.0;
+    for (int i = 0; i < n; i++) c1 += H[(size_t)i * nm + i];
+    /* Eigen::LLT (lower): column j of L by the lanes that own rows i >= j */
+    for (int j = 0; j < n; j++) {
+      double acc[QP_SLOTS];
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) {
+        const int i = lane + 32 * t;
+        acc[t] = 0.0;
+        if (i >= j && i < n) {
+          double a = H[(size_t)i * nm + j];
+          for (int k = 0; k < j; k++) a -= L[i * ld + k] * L[j * ld + k];
+          acc[t] = a;
+        }
+      }
+      const double sdiag = __shfl_sync(FULL, (j >> 5) ? acc[QP_SLOTS - 1] : acc[0], j & 31);
+      if (!(sdiag > 0)) { res = QP_UNBOUNDED; goto done; }
+      const double ljj = sqrt(sdiag);
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) {
+        const int i = lane + 32 * t;
+        if (i == j) L[i * ld + j] = ljj;
+        else if (i > j && i < n) L[i * ld + j] = acc[t] / ljj;
+      }
+      __syncwarp();
+    }
+    /* J = L^-T: L' J = I column by column, a lane per column */
+    for (int c = lane; c < n; c += 32)
+      for (int i = n - 1; i >= 0; i--) {
+        double a = (i == c) ? 1.0 : 0.0;
+        for (int k = i + 1; k < n; k++) a -= L[k * ld + i] * J[k * ld + c];
+        J[i * ld + c] = a / L[i * ld + i];
+      }
+    __syncwarp();
+    for (int i = 0; i < n; i++) c2 += J[i * ld + i];
+    /* x = -H^-1 g: L y = g, then L' x = y, column-oriented */
+    {
+      double acc[QP_SLOTS];
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) acc[t] = (lane + 32 * t < n) ? g[lane + 32 * t] : 0.0;
+      for (int i = 0; i < n; i++) {
+        const double yi = __shfl_sync(FULL, (i >> 5) ? acc[QP_SLOTS - 1] : acc[0], i & 31) / L[i * ld + i];
+#pragma unroll
+        for (int t = 0; t < QP_SLOTS; t++) {
+          const int m = lane + 32 * t;
+          if (m > i && m < n) acc[t] -= L[m * ld + i] * yi;
+          else if (m == i) acc[t] = yi;
+        }
+      }
+      for (int i = n - 1; i >= 0; i--) {
+        const double xi = __shfl_sync(FULL, (i >> 5) ? acc[QP_SLOTS - 1] : acc[0], i & 31) / L[i * ld + i];
+#pragma unroll
+        for (int t = 0; t < QP_SLOTS; t++) {
+          const int m = lane + 32 * t;
+          if (m < i) acc[t] -= L[i * ld + m] * xi;
+          else if (m == i) acc[t] = xi;
+        }
+      }
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++)
+        if (lane + 32 * t < n) E.x[lane + 32 * t] = -acc[t];
+    }
+    __syncwarp();
+    for (int k = lane; k < n * ld; k += 32) R[k] = 0.0;
+    for (int k = lane; k < n; k += 32) E.d[k] = 0.0;
+    __syncwarp();
+    /* equality constraints, in row order */
+    for (int i = 0; i < neq; i++) {
+      for (int k = lane; k < n; k += 32) E.np[k] = CE[(size_t)i * nm + k];
+      __syncwarp();
+      qp_compute_d(E, lane);
+      __syncwarp();
+      qp_update_z(E, iq, lane);
+      qp_update_r(E, iq, lane);
+      double zz = 0.0, znp = 0.0, npx = 0.0;
+      for (int k = lane; k < n; k += 32) { zz += E.z[k] * E.z[k]; znp += E.z[k] * E.np[k]; npx += E.np[k] * E.x[k]; }
+      zz = warp_sum(zz); znp = warp_sum(znp); npx = warp_sum(npx);
+      double t2 = 0.0;
+      if (fabs(zz) > TS_EPS) t2 = (-npx - ce0[i]) / znp;
+      for (int k = lane; k < n; k += 32) E.x[k] += t2 * E.z[k];
+      for (int k = lane; k < iq; k += 32) E.u[k] -= t2 * E.r[k];
+      if (lane == 0) { E.u[iq] = t2; E.A[i] = -i - 1; }
+      __syncwarp();
+      if (!qp_add_constraint(E, iq, R_norm, lane)) { res = QP_REDUNDANT_EQ; goto done; }
+    }
+    for (int i = lane; i < nin; i += 32) E.iai[i] = i;
+    __syncwarp();
+
+  l1:
+    iter++;
+    if (iter >= q.max_iter) { res = QP_MAX_ITER; goto done; }
+    for (int i = neq + lane; i < iq; i += 32) E.iai[E.A[i]] = -1;
+    ss = 0.0;
+    ip = 0;
+    {
+      /* violation scan: a lane per row, streaming the row from global memory with the oracle's k order */
+      double psi = 0.0;
+      for (int i = lane; i < nin; i += 32) {
+        const double* row = CI + (size_t)i * nm;
+        double a = 0.0;
+        for (int k = 0; k < n; k++) a += row[k] * E.x[k];
+        const double si = a + ci0[i];
+        E.s[i] = si;
+        E.iax[i] = 1;
+        psi += si < 0 ? si : 0.0;
+      }
+      psi = warp_sum(psi);
+      __syncwarp();
+      if (fabs(psi) <= nin * TS_EPS * c1 * c2 * 100.0) { res = QP_OPTIMAL; goto done; }
+    }
+    for (int i = lane; i < iq; i += 32) { E.uo[i] = E.u[i]; E.Ao[i] = E.A[i]; }
+    for (int k = lane; k < n; k += 32) E.xo[k] = E.x[k];
+    __syncwarp();
+
+  l2:
+    {
+      double best = ss;
+      int bi = -1;
+      for (int i = lane; i < nin; i += 32)
+        if (E.s[i] < best && E.iai[i] != -1 && E.iax[i]) { best = E.s[i]; bi = i; }
+      warp_argmin(best, bi);
+      if (bi >= 0) { ss = best; ip = bi; }
+    }
+    if (ss >= 0) { res = QP_OPTIMAL; goto done; }
+    for (int k = lane; k < n; k += 32) E.np[k] = CI[(size_t)ip * nm + k];
+    if (lane == 0) { E.u[iq] = 0.0; E.A[iq] = ip; }
+    __syncwarp();
+
+  l2a:
+    {
+      qp_compute_d(E, lane);
+      __syncwarp();
+      if (iq >= n) {
+        for (int k = lane; k < n; k += 32) E.z[k] = 0.0;
+      } else {
+        qp_update_z(E, iq, lane);
+      }
+      qp_update_r(E, iq, lane);
+      /* partial step length t1: the smallest u/r over the inequalities of the working set with r > 0, first on ties */
+      double t1 = TS_INF;
+      {
+        int bk = -1;
+        for (int k = neq + lane; k < iq; k += 32) {
+          double tmp;
+          if (E.r[k] > 0 && ((tmp = E.u[k] / E.r[k]) < t1)) { t1 = tmp; bk = k; }
+        }
+        warp_argmin(t1, bk);
+        l = bk >= 0 ? E.A[bk] : 0;
+      }
+      double zz = 0.0, znp = 0.0;
+      for (int k = lane; k < n; k += 32) { zz += E.z[k] * E.z[k]; znp += E.z[k] * E.np[k]; }
+      zz = warp_sum(zz); znp = warp_sum(znp);
+      const double t2 = (fabs(zz) > TS_EPS) ? -E.s[ip] / znp : TS_INF;
+      const double t = t1 < t2 ? t1 : t2;
+      if (t >= TS_INF) { res = QP_UNBOUNDED; goto done; }
+      if (t2 >= TS_INF) {
+        for (int k = lane; k < iq; k += 32) E.u[k] -= t * E.r[k];
+        __syncwarp();
+        if (lane == 0) { E.u[iq] += t; E.iai[l] = l; }
+        __syncwarp();
+        qp_delete_constraint(E, neq, iq, l, lane);
+        goto l2a;
+      }
+      for (int k = lane; k < n; k += 32) E.x[k] += t * E.z[k];
+      for (int k = lane; k < iq; k += 32) E.u[k] -= t * E.r[k];
+      __syncwarp();
+      if (lane == 0) E.u[iq] += t;
+      __syncwarp();
+      if (t == t2) {
+        if (!qp_add_constraint(E, iq, R_norm, lane)) {
+          if (lane == 0) E.iax[ip] = 0;
+          __syncwarp();
+          qp_delete_constraint(E, neq, iq, ip, lane);
+          for (int i = lane; i < nin; i += 32) E.iai[i] = i;
+          __syncwarp();
+          if (lane == 0)
+            for (int i = 0; i < iq; i++) {
+              E.A[i] = E.Ao[i];
+              if (E.A[i] >= 0) E.iai[E.A[i]] = -1;
+              E.u[i] = E.uo[i];
+            }
+          for (int k = lane; k < n; k += 32) E.x[k] = E.xo[k];
+          __syncwarp();
+          goto l2;
+        }
+        if (lane == 0) E.iai[ip] = -1;
+        __syncwarp();
+        goto l1;
+      }
+      if (lane == 0) E.iai[l] = l;
+      __syncwarp();
+      qp_delete_constraint(E, neq, iq, l, lane);
+      {
+        double a = 0.0;
+        for (int k = lane; k < n; k += 32) a += CI[(size_t)ip * nm + k] * E.x[k];
+        a = warp_sum(a);
+        if (lane == 0) E.s[ip] = a + ci0[ip];
+        __syncwarp();
+      }
+      goto l2a;
+    }
+  }
+done:
+  __syncwarp();
+  /* SolverHQuadProgFast's status mapping; the solution and the working set are reported for OPTIMAL and MAX_ITER */
+  const int status = !valid ? ST_ERROR
+                     : (res == QP_OPTIMAL ? ST_OPTIMAL
+                        : (res == QP_MAX_ITER ? ST_MAX_ITER
+                           : ((res == QP_UNBOUNDED || res == QP_INFEASIBLE) ? ST_INFEASIBLE : ST_ERROR)));
+  const bool out = status == ST_OPTIMAL || status == ST_MAX_ITER;
+  const int nw = out ? iq : 0, ne = out ? neq : 0, nx = out ? n : 0;
+  if (lane == 0) {
+    q.status[env] = status;
+    if (q.iters) q.iters[env] = valid ? iter : 0;
+  }
+  for (int k = lane; k < nm; k += 32) {
+    q.x[(size_t)env * nm + k] = k < nx ? E.x[k] : 0.0;
+    if (q.active) q.active[(size_t)env * nm + k] = k < nw - ne ? E.A[ne + k] : -1;
+    if (q.lambda) q.lambda[(size_t)env * nm + k] = k < nw - ne ? E.u[ne + k] : 0.0;
+  }
+  if (q.lambda_eq)
+    for (int k = lane; k < q.neq_max; k += 32) q.lambda_eq[(size_t)env * q.neq_max + k] = k < ne ? E.u[k] : 0.0;
+  if (q.tau)
+    for (int r = lane; r < q.na; r += 32) {
+      double a = 0.0;
+      if (out) {
+        const double* row = q.TA + ((size_t)env * q.na + r) * nm;
+        for (int k = 0; k < n; k++) a += row[k] * E.x[k];
+        a += q.ta0[(size_t)env * q.na + r];
+      }
+      q.tau[(size_t)env * q.na + r] = a;
+    }
 }
 
 #ifndef TSIDB_EMU
@@ -2638,6 +3101,15 @@ tsidb_problem_kernel(const TickArgs a, const ProblemOut o) {
   const DevConst& C = g_const[a.slot];
   for (int env = blockIdx.x * TSIDB_P_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_P_CTA_WARPS)
     problem_env<NV>(C, pt, sm, a, o, env, lane);
+}
+
+/* Generic QP solve (tsidb_qp_solve): one one-warp CTA per env on a persistent grid.  The dynamic shared memory is
+ * qp_layout(n_max, nin_max).per_env doubles, so the resident CTAs per SM follow from the call's strides. */
+#define TSIDB_Q_MIN_CTAS 16 /* register cap: 128 per thread */
+__global__ void __launch_bounds__(32, TSIDB_Q_MIN_CTAS) tsidb_qp_kernel(const QpArgs q) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31;
+  for (int env = blockIdx.x; env < q.n_envs; env += gridDim.x) qp_env(q, smem, env, lane);
 }
 
 /* ---- Small batches: the whole tick of one env in ONE launch ----

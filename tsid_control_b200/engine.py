@@ -389,6 +389,7 @@ class TsidEngine:
         return res
 
     PROBLEM_PARTS = ("H", "g", "CE", "ce0", "CI", "ci0")
+    ACTUATION_PARTS = ("TA", "ta0")
 
     def problem_sizes(self) -> Tuple[int, int, int]:
         """(n_max, neq_max, nin_max): the padding of :meth:`problem_data`'s arrays (tsidb_problem_sizes)."""
@@ -402,6 +403,7 @@ class TsidEngine:
         eiquadprog, min 1/2 x'Hx + g'x s.t. CE x + ce0 = 0, CI x + ci0 >= 0, in x = [dv; f of the feet in contact, LF
         first].  Returns new CUDA tensors H [N,n,n], g [N,n], CE [N,18,n], ce0 [N,18], CI [N,nin,n], ci0 [N,nin] (the
         requested `parts`, padded with zeros to problem_sizes()) and sizes [N,3] int32 = (n, neq, nin) of each env.
+        `parts` may also name the actuation map TA [N,na,n], ta0 [N,na]: tau = TA x + ta0 (getActuatorForces).
         Inputs as in :meth:`compute`; a later tick's results do not depend on this call."""
         n = q.shape[0]
         self._chk(q, n, self.nq, "q")
@@ -410,21 +412,61 @@ class TsidEngine:
             if contact_mask.dtype is not torch.uint8 or not contact_mask.is_cuda or contact_mask.get_device() != self._dev_index \
                     or contact_mask.shape != (n,):
                 raise TypeError("contact_mask: expected a uint8 [N] tensor on the engine's device")
-        unknown = set(parts) - set(self.PROBLEM_PARTS)
+        unknown = set(parts) - set(self.PROBLEM_PARTS + self.ACTUATION_PARTS)
         if unknown:
-            raise ValueError(f"parts: unknown {sorted(unknown)}; choose from {self.PROBLEM_PARTS}")
+            raise ValueError(f"parts: unknown {sorted(unknown)}; choose from {self.PROBLEM_PARTS + self.ACTUATION_PARTS}")
         r = TsidbRefs()
         for k, nd in self._ref_dims:
             t = refs.get(k) if refs else None
             setattr(r, k, None if t is None else self._chk(t, n, nd, k).data_ptr())
         nx, neq, nin = self.problem_sizes()
-        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin)}
+        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin),
+                  "TA": (n, self.na, nx), "ta0": (n, self.na)}
         out = {k: torch.empty(shapes[k], dtype=torch.float64, device=self.device) for k in parts}
         out["sizes"] = torch.empty((n, 3), dtype=torch.int32, device=self.device)
         po = _capi.TsidbProblemOut(**{k: t.data_ptr() for k, t in out.items()})
         check(self.lib.tsidb_problem_data(self.h, n, 0, q.data_ptr(), v.data_ptr(),
                                           contact_mask.data_ptr() if contact_mask is not None else None, C.byref(r),
                                           C.byref(po), self._stream()), "tsidb_problem_data")
+        return out
+
+    def qp_solve(self, problem: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+        """eiquadprog-fast with this controller's max_iter on every env of `problem` (tsidb_qp_solve): a dict in the
+        layout :meth:`problem_data` returns, possibly modified or enlarged.  H [N,n_max,n_max], g [N,n_max] and sizes
+        [N,3] int32 are required; CE [N,neq_max,n_max] with ce0 [N,neq_max], CI [N,nin_max,n_max] with ci0 [N,nin_max]
+        and TA [N,na,n_max] with ta0 [N,na] are optional (absent = no such rows / no tau).  The strides come from the
+        shapes.  Returns new CUDA tensors x [N,n_max], status, iters [N] int32, active [N,n_max] int32 (CI rows of the
+        working set in working-set order, -1 padded), lambda [N,n_max] (their multipliers), lambda_eq [N,neq_max] and,
+        with TA and ta0, tau [N,na]."""
+        for k in ("H", "g", "sizes"):
+            if k not in problem:
+                raise ValueError(f"qp_solve: {k} is required")
+        for a, b in (("CE", "ce0"), ("CI", "ci0"), ("TA", "ta0")):
+            if (a in problem) != (b in problem):
+                raise ValueError(f"qp_solve: {a} and {b} go together")
+        unknown = set(problem) - set(self.PROBLEM_PARTS + self.ACTUATION_PARTS + ("sizes",))
+        if unknown:
+            raise ValueError(f"qp_solve: unknown parts {sorted(unknown)}")
+        n, nx = problem["g"].shape if problem["g"].dim() == 2 else (-1, -1)
+        neq = problem["ce0"].shape[-1] if "ce0" in problem else 0
+        nin = problem["ci0"].shape[-1] if "ci0" in problem else 0
+        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin),
+                  "TA": (n, self.na, nx), "ta0": (n, self.na), "sizes": (n, 3)}
+        for k, t in problem.items():
+            dt = torch.int32 if k == "sizes" else torch.float64
+            if not isinstance(t, torch.Tensor) or t.dtype is not dt or not t.is_cuda or t.get_device() != self._dev_index \
+                    or not t.is_contiguous() or tuple(t.shape) != shapes[k]:
+                raise TypeError(f"qp_solve: {k}: expected a contiguous {dt} tensor of shape {shapes[k]} on the engine's device")
+        f64 = dict(dtype=torch.float64, device=self.device)
+        i32 = dict(dtype=torch.int32, device=self.device)
+        out = {"x": torch.empty((n, nx), **f64), "status": torch.empty(n, **i32), "iters": torch.empty(n, **i32),
+               "active": torch.empty((n, nx), **i32), "lambda": torch.empty((n, nx), **f64),
+               "lambda_eq": torch.empty((n, neq), **f64)}
+        if "TA" in problem:
+            out["tau"] = torch.empty((n, self.na), **f64)
+        po = _capi.TsidbProblemOut(**{k: t.data_ptr() for k, t in problem.items()})
+        qo = _capi.TsidbQpOut(**{k: t.data_ptr() for k, t in out.items()})
+        check(self.lib.tsidb_qp_solve(self.h, n, nx, neq, nin, C.byref(po), C.byref(qo), self._stream()), "tsidb_qp_solve")
         return out
 
     def ci_row(self, block: int, side: int, i: int) -> int:
