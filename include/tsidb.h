@@ -293,6 +293,29 @@ typedef struct tsidb_qp_out {
 int tsidb_qp_solve(tsidb_handle* h, int n_envs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* qp,
                    const tsidb_qp_out* out, void* cuda_stream);
 
+/* ---- differentiating the QP solve ---------------------------------------------------------------------------------
+ * tsidb_qp_grad is the adjoint (reverse-mode derivative) of tsidb_qp_solve: given the problem qp that was solved (same
+ * strides and required arrays as the solve; TA also when grad_in->tau is given), the solve's result sol (x, status,
+ * active, lambda and, when neq_max > 0, lambda_eq are read) and the gradients of a loss with respect to the solve's
+ * outputs, grad_in (x, lambda, lambda_eq, tau: dL/d of each, same layout; a NULL part counts as zero; status, iters and
+ * active must be NULL), it writes dL/d of the problem's parts into grad_out (H, g, CE, ce0, CI, ci0, TA, ta0: NULL = not
+ * written; sizes must be NULL), every byte of each requested part with zeros in the padding.  All DEVICE memory.
+ * The derivative is the one of the KKT system of the final working set W (rows CE and CI_W, multipliers lambda_eq and
+ * lambda): at a degenerate point (a row of W with a zero multiplier, or an inactive row with zero slack) it is the
+ * one-sided derivative that keeps W.  With G = [CE; CI_W], nu = [lambda_eq; lambda_W] and (p, q) the solution of
+ * H p + G' q = dL/dx + TA' dL/dtau, G p = -[dL/dlambda_eq; dL/dlambda_W]:  dg = -p, dG = nu p' - q x', d[ce0; ci0_W] = -q,
+ * dTA = dL/dtau x', dta0 = dL/dtau; rows of CI outside W get zero.  The solve reads only the lower triangle of H, so
+ * dL/dH is lower triangular: dH = tril(P + P', -1) + diag(P) with P = -p x'; a caller with a symmetric H by
+ * construction gets the same total as with the symmetric convention.
+ * An env is differentiated (status[e] = TSIDB_STATUS_OPTIMAL) when sol->status[e] is OPTIMAL, its sizes fit the strides,
+ * its working set is valid (entries in [0, nin), no duplicate, -1 padding after the last entry, neq + |W| <= n), H is
+ * positive definite and the rows of W are independent; otherwise status[e] = TSIDB_STATUS_ERROR and its gradients are
+ * zero.  Nothing outside an env's (n, neq, nin) and working set is read.  No workspace of the handle is used, so the call
+ * may run on any stream.  Asynchronous on cuda_stream, no host round trip. */
+int tsidb_qp_grad(tsidb_handle* h, int n_envs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* qp,
+                  const tsidb_qp_out* sol, const tsidb_qp_out* grad_in, const tsidb_problem_out* grad_out, int32_t* status,
+                  void* cuda_stream);
+
 /* controller.integrate_dv(q, v, dv, dt) (ref:ctrl/WalkController.py:291-295,
  * ref:legacy/biped.py:236-240): v_mean = v + dt/2*dv; v += dt*dv;
  * q = pin.integrate(q, dt*v_mean).  In place on device arrays.                   */

@@ -272,6 +272,9 @@ def load_library() -> C.CDLL:
     lib.tsidb_problem_data.restype = ip
     lib.tsidb_qp_solve.argtypes = [vp, ip, ip, ip, ip, C.POINTER(TsidbProblemOut), C.POINTER(TsidbQpOut), vp]
     lib.tsidb_qp_solve.restype = ip
+    lib.tsidb_qp_grad.argtypes = [vp, ip, ip, ip, ip, C.POINTER(TsidbProblemOut), C.POINTER(TsidbQpOut), C.POINTER(TsidbQpOut),
+                                  C.POINTER(TsidbProblemOut), vp, vp]
+    lib.tsidb_qp_grad.restype = ip
     _LIB = lib
     return lib
 
@@ -288,5 +291,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_fp64_peak", "tsidb_launch_count", "tsidb_set_timing", "tsidb_set_sched_hint", "tsidb_last_tick_ms",
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
-    "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve",
+    "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve", "tsidb_qp_grad",
 ]

@@ -224,6 +224,8 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
   TSIDB_ATTR(tsidb_problem_kernel<24>, TSIDB_P_SMEM(24), TSIDB_P_CTAS_PER_SM, "QP export kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_qp_kernel, qp_layout(TSIDB_QP_MAX_N, TSIDB_QP_MAX_NIN).per_env * sizeof(double), 1, "generic QP kernel",
              cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_qp_grad_kernel, qg_layout(TSIDB_QP_MAX_N, TSIDB_QP_MAX_NIN).per_env * sizeof(double), 1,
+             "QP gradient kernel", cudaSharedmemCarveoutMaxShared);
 #undef TSIDB_ATTR
   CK(cudaMalloc(&h->counter, TSIDB_NCOUNTER * TSIDB_MAX_CHUNKS * sizeof(int32_t)));
   CK(cudaMalloc(&h->pred, (size_t)max_envs * sizeof(int32_t)));
@@ -819,6 +821,60 @@ extern "C" int tsidb_qp_solve(tsidb_handle* h, int n_envs, int n_max, int neq_ma
   long blocks = (long)per_sm * h->sm_count; /* persistent */
   if (blocks > n_envs) blocks = n_envs;
   tsidb_qp_kernel<<<(int)blocks, 32, smem, (cudaStream_t)cuda_stream>>>(q);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
+/* adjoint of tsidb_qp_solve: one launch of the QP gradient kernel, no workspace of the handle */
+extern "C" int tsidb_qp_grad(tsidb_handle* h, int n_envs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* qp,
+                             const tsidb_qp_out* sol, const tsidb_qp_out* grad_in, const tsidb_problem_out* grad_out,
+                             int32_t* status, void* cuda_stream) {
+  if (!h || !qp || !sol || !grad_in || !grad_out) { g_err = "tsidb_qp_grad: null argument"; return -1; }
+  if (n_envs <= 0) { g_err = "tsidb_qp_grad: n_envs must be positive"; return -1; }
+  if (n_max < 1 || n_max > TSIDB_QP_MAX_N || neq_max < 0 || neq_max > n_max || nin_max < 0 || nin_max > TSIDB_QP_MAX_NIN) {
+    g_err = "tsidb_qp_grad: strides must satisfy 1 <= n_max <= TSIDB_QP_MAX_N (64), 0 <= neq_max <= n_max, "
+            "0 <= nin_max <= TSIDB_QP_MAX_NIN (512)";
+    return -1;
+  }
+  if (!qp->H || !qp->g || !qp->sizes || !sol->x || !sol->status || !sol->active || !sol->lambda || !status) {
+    g_err = "tsidb_qp_grad: H, g, sizes, the solution's x, status, active and lambda, and status are required";
+    return -1;
+  }
+  if ((neq_max > 0 && (!qp->CE || !qp->ce0 || !sol->lambda_eq)) || (nin_max > 0 && (!qp->CI || !qp->ci0))) {
+    g_err = "tsidb_qp_grad: CE, ce0 and lambda_eq are required when neq_max > 0, CI and ci0 when nin_max > 0";
+    return -1;
+  }
+  if (grad_in->tau && !qp->TA) { g_err = "tsidb_qp_grad: a tau gradient needs TA"; return -1; }
+  if (grad_in->status || grad_in->iters || grad_in->active || grad_out->sizes) {
+    g_err = "tsidb_qp_grad: grad_in's status, iters, active and grad_out's sizes must be NULL";
+    return -1;
+  }
+  for (const void* p : {(const void*)qp->H, (const void*)qp->g, (const void*)qp->CE, (const void*)qp->ce0, (const void*)qp->CI,
+                        (const void*)qp->ci0, (const void*)qp->TA, (const void*)qp->ta0, (const void*)sol->x,
+                        (const void*)sol->lambda, (const void*)sol->lambda_eq, (const void*)grad_in->x,
+                        (const void*)grad_in->lambda, (const void*)grad_in->lambda_eq, (const void*)grad_in->tau,
+                        (const void*)grad_out->H, (const void*)grad_out->g, (const void*)grad_out->CE, (const void*)grad_out->ce0,
+                        (const void*)grad_out->CI, (const void*)grad_out->ci0, (const void*)grad_out->TA, (const void*)grad_out->ta0})
+    if (((uintptr_t)p & 7) != 0) { g_err = "tsidb_qp_grad: fp64 arrays must be 8-byte aligned"; return -1; }
+  for (const void* p : {(const void*)qp->sizes, (const void*)sol->status, (const void*)sol->active, (const void*)status})
+    if (((uintptr_t)p & 3) != 0) { g_err = "tsidb_qp_grad: int32 arrays must be 4-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  QpGradArgs a;
+  a.n_envs = n_envs; a.n_max = n_max; a.neq_max = neq_max; a.nin_max = nin_max; a.na = h->dc.na;
+  a.H = qp->H; a.CE = qp->CE; a.CI = qp->CI; a.TA = qp->TA; a.sizes = qp->sizes;
+  a.x = sol->x; a.lambda = sol->lambda; a.lambda_eq = sol->lambda_eq; a.sol_status = sol->status; a.active = sol->active;
+  a.gx = grad_in->x; a.glambda = grad_in->lambda; a.glambda_eq = grad_in->lambda_eq; a.gtau = grad_in->tau;
+  a.dH = grad_out->H; a.dg = grad_out->g; a.dCE = grad_out->CE; a.dce0 = grad_out->ce0; a.dCI = grad_out->CI;
+  a.dci0 = grad_out->ci0; a.dTA = grad_out->TA; a.dta0 = grad_out->ta0;
+  a.status = status;
+  const size_t smem = qg_layout(n_max, nin_max).per_env * sizeof(double);
+  int per_sm = 0;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tsidb_qp_grad_kernel, 32, smem));
+  if (per_sm < 1) { g_err = "tsidb_qp_grad: the kernel does not fit an SM"; return -2; }
+  long blocks = (long)per_sm * h->sm_count; /* persistent */
+  if (blocks > n_envs) blocks = n_envs;
+  tsidb_qp_grad_kernel<<<(int)blocks, 32, smem, (cudaStream_t)cuda_stream>>>(a);
   CK(cudaGetLastError());
   h->launches += 1;
   return 0;

@@ -137,6 +137,19 @@ struct QpArgs {
   double *lambda, *lambda_eq, *tau;
 };
 
+/* arguments of the adjoint of the QP solve (tsidb_qp_grad): the solved problem and its solution (read), the incoming
+ * gradients (NULL = zero) and the requested gradients of the problem's parts (NULL = not written), same layouts */
+struct QpGradArgs {
+  int32_t n_envs, n_max, neq_max, nin_max, na;
+  const double *H, *CE, *CI, *TA;
+  const int32_t* sizes;
+  const double *x, *lambda, *lambda_eq;
+  const int32_t *sol_status, *active;
+  const double *gx, *glambda, *glambda_eq, *gtau;
+  double *dH, *dg, *dCE, *dce0, *dCI, *dci0, *dTA, *dta0;
+  int32_t* status;
+};
+
 struct TickArgs {
   int32_t n_envs, layout, pad_;
   const double* q;

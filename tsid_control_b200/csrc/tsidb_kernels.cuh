@@ -2634,6 +2634,35 @@ TSIDB_DEV void qp_delete_constraint(const QpEnv& E, int neq, int& iq, int l, int
 /* eiquadprog-fast result codes (the oracle's eq_solve) */
 enum { QP_OPTIMAL = 0, QP_INFEASIBLE = 1, QP_UNBOUNDED = 2, QP_MAX_ITER = 3, QP_REDUNDANT_EQ = 4 };
 
+/* Eigen::LLT (lower) of the n x n matrix H (row stride nm; the strict upper triangle is never read) into L (row stride
+ * ld): column j by the lanes that own rows i >= j.  False when H is not positive definite. */
+TSIDB_DEV bool qp_llt(const double* H, int nm, double* L, int ld, int n, int lane) {
+  for (int j = 0; j < n; j++) {
+    double acc[QP_SLOTS];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int i = lane + 32 * t;
+      acc[t] = 0.0;
+      if (i >= j && i < n) {
+        double a = H[(size_t)i * nm + j];
+        for (int k = 0; k < j; k++) a -= L[i * ld + k] * L[j * ld + k];
+        acc[t] = a;
+      }
+    }
+    const double sdiag = __shfl_sync(FULL, (j >> 5) ? acc[QP_SLOTS - 1] : acc[0], j & 31);
+    if (!(sdiag > 0)) return false;
+    const double ljj = sqrt(sdiag);
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int i = lane + 32 * t;
+      if (i == j) L[i * ld + j] = ljj;
+      else if (i > j && i < n) L[i * ld + j] = acc[t] / ljj;
+    }
+    __syncwarp();
+  }
+  return true;
+}
+
 /* one env; sm holds qp_layout(q.n_max, q.nin_max).per_env doubles of this warp */
 TSIDB_DEV void qp_env(const QpArgs& q, double* sm, int env, int lane) {
   const QpLayout Ly = qp_layout(q.n_max, q.nin_max);
@@ -2663,30 +2692,7 @@ TSIDB_DEV void qp_env(const QpArgs& q, double* sm, int env, int lane) {
     int ip = 0, l = 0;
     double ss = 0.0;
     for (int i = 0; i < n; i++) c1 += H[(size_t)i * nm + i];
-    /* Eigen::LLT (lower): column j of L by the lanes that own rows i >= j */
-    for (int j = 0; j < n; j++) {
-      double acc[QP_SLOTS];
-#pragma unroll
-      for (int t = 0; t < QP_SLOTS; t++) {
-        const int i = lane + 32 * t;
-        acc[t] = 0.0;
-        if (i >= j && i < n) {
-          double a = H[(size_t)i * nm + j];
-          for (int k = 0; k < j; k++) a -= L[i * ld + k] * L[j * ld + k];
-          acc[t] = a;
-        }
-      }
-      const double sdiag = __shfl_sync(FULL, (j >> 5) ? acc[QP_SLOTS - 1] : acc[0], j & 31);
-      if (!(sdiag > 0)) { res = QP_UNBOUNDED; goto done; }
-      const double ljj = sqrt(sdiag);
-#pragma unroll
-      for (int t = 0; t < QP_SLOTS; t++) {
-        const int i = lane + 32 * t;
-        if (i == j) L[i * ld + j] = ljj;
-        else if (i > j && i < n) L[i * ld + j] = acc[t] / ljj;
-      }
-      __syncwarp();
-    }
+    if (!qp_llt(H, nm, L, ld, n, lane)) { res = QP_UNBOUNDED; goto done; }
     /* J = L^-T: L' J = I column by column, a lane per column */
     for (int c = lane; c < n; c += 32)
       for (int i = n - 1; i >= 0; i--) {
@@ -2893,6 +2899,266 @@ done:
       }
       q.tau[(size_t)env * q.na + r] = a;
     }
+}
+
+/* ================================================================= adjoint of the QP solve of one env (tsidb_qp_grad) */
+/* At an OPTIMAL solution with working set W, x and nu = [lambda_eq; lambda_W] solve the KKT system of the rows
+ * G = [CE; CI_W], b = [ce0; ci0_W]:  H x + g = G' nu,  G x + b = 0.  Its adjoint for incoming xb (+ TA' taub) and nub is
+ *   H p + G' q = xb,  G p = -nub,
+ * from which gb = -p, Gb = nu p' - q x', bb = -q, TAb = taub x', ta0b = taub and, since the solve reads only the lower
+ * triangle of H, Hb = tril(P + P', -1) + diag(P) with P = -p x'.  The system is solved through the factors of the
+ * forward: H = L L', M = L^-1 G' = [Q1 Q2] [R; 0] (Householder), y = L^-1 xb:
+ *   p~ = Q2 Q2' y - Q1 R^-T nub,  q = R^-1 (Q1' y + R^-T nub),  p = L^-T p~
+ * (no normal equations G H^-1 G', which would square the conditioning of the contact rows). */
+struct QgLayout {
+  int ld;                     /* row stride of L and M: odd, so column walks are conflict-free */
+  int oL, oM, ox, op, oq, onu, obeta, ordiag; /* doubles */
+  int oW, opos;               /* int32, from sm + oI */
+  int oI, per_env;
+};
+TSIDB_HD inline QgLayout qg_layout(int n_max, int nin_max) {
+  QgLayout L;
+  L.ld = n_max | 1;
+  L.oL = 0;
+  L.oM = L.oL + n_max * L.ld;
+  L.ox = L.oM + n_max * L.ld;
+  L.op = L.ox + n_max;
+  L.oq = L.op + n_max;
+  L.onu = L.oq + n_max;
+  L.obeta = L.onu + n_max;
+  L.ordiag = L.obeta + n_max;
+  L.oI = L.ordiag + n_max;
+  L.oW = 0;
+  L.opos = n_max;
+  L.per_env = L.oI + (n_max + nin_max + 1) / 2;
+  L.per_env += L.per_env & 1;
+  return L;
+}
+
+/* out[r * nm + c] = f(r, c) for the rows x nm block: the warp stores 32 consecutive doubles at a time */
+template <class F>
+TSIDB_DEV void qg_store(double* out, int rows, int nm, int lane, F f) {
+  if (rows <= 0 || nm <= 0) return;
+  int r = 0, c = lane;
+  while (c >= nm) { c -= nm; r++; }
+  const long total = (long)rows * nm;
+  for (long k = lane; k < total; k += 32) {
+    out[k] = f(r, c);
+    c += 32;
+    while (c >= nm) { c -= nm; r++; }
+  }
+}
+
+/* y = Q' y (fwd) or Q y for the Householder reflectors in the columns 0..m-1 of M; y in the lane-owned registers */
+TSIDB_DEV void qg_reflect(const double* M, int ld, const double* beta, int n, int m, bool fwd, double (&y)[QP_SLOTS], int lane) {
+  for (int s = 0; s < m; s++) {
+    const int k = fwd ? s : m - 1 - s;
+    double d = 0.0;
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int i = lane + 32 * t;
+      if (i >= k && i < n) d += M[i * ld + k] * y[t];
+    }
+    d = warp_sum(d) * beta[k];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int i = lane + 32 * t;
+      if (i >= k && i < n) y[t] -= d * M[i * ld + k];
+    }
+  }
+}
+
+TSIDB_DEV double qg_lane(const double (&v)[QP_SLOTS], int i) { return __shfl_sync(FULL, (i >> 5) ? v[QP_SLOTS - 1] : v[0], i & 31); }
+
+/* one env; sm holds qg_layout(a.n_max, a.nin_max).per_env doubles of this warp */
+TSIDB_DEV void qp_grad_env(const QpGradArgs& a, double* sm, int env, int lane) {
+  const QgLayout Ly = qg_layout(a.n_max, a.nin_max);
+  const int nm = a.n_max, ld = Ly.ld, na = a.na;
+  double *L = sm + Ly.oL, *M = sm + Ly.oM, *x = sm + Ly.ox, *p = sm + Ly.op, *q = sm + Ly.oq, *nu = sm + Ly.onu;
+  double *beta = sm + Ly.obeta, *rdiag = sm + Ly.ordiag;
+  int* W = reinterpret_cast<int*>(sm + Ly.oI) + Ly.oW;
+  int* pos = reinterpret_cast<int*>(sm + Ly.oI) + Ly.opos;
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  const int n = a.sizes[(size_t)env * 3], neq = a.sizes[(size_t)env * 3 + 1], nin = a.sizes[(size_t)env * 3 + 2];
+  bool ok = a.sol_status[env] == ST_OPTIMAL && n >= 1 && n <= nm && neq >= 0 && neq <= n && neq <= a.neq_max && nin >= 0 &&
+            nin <= a.nin_max;
+  int m = 0;
+  if (ok) {
+    /* the working set: -1 padded entries of [0, nin), no duplicates, neq + |W| <= n */
+    int act[QP_SLOTS];
+    bool bad = false;
+    for (int r = lane; r < nin; r += 32) pos[r] = -1;
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int k = lane + 32 * t;
+      act[t] = k < n ? a.active[(size_t)env * nm + k] : -1;
+      bad |= act[t] < -1 || act[t] >= nin;
+    }
+    unsigned long long used = 0;
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) used |= (unsigned long long)__ballot_sync(FULL, act[t] >= 0) << (32 * t);
+    int w = 0;
+    while (w < 64 && ((used >> w) & 1ull)) w++;
+    bad |= (used & (used + 1)) != 0 || neq + w > n; /* the entries >= 0 are a prefix */
+    __syncwarp();
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++)
+      if (!bad && act[t] >= 0) {
+        pos[act[t]] = lane + 32 * t;
+        W[lane + 32 * t] = act[t];
+      }
+    __syncwarp();
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) bad |= !bad && act[t] >= 0 && pos[act[t]] != lane + 32 * t; /* duplicate row */
+    ok = __ballot_sync(FULL, bad) == 0;
+    m = neq + w;
+  }
+  const double* H = a.H + (size_t)env * nm * nm;
+  if (ok) ok = qp_llt(H, nm, L, ld, n, lane);
+  double y[QP_SLOTS], v[QP_SLOTS];
+  if (ok) {
+    const double* CE = a.CE + (size_t)env * a.neq_max * nm;
+    const double* CI = a.CI + (size_t)env * a.nin_max * nm;
+    /* M = G' (row j of G into column j), x, nu, y = xb + TA' taub */
+    for (int j = 0; j < m; j++) {
+      const double* row = j < neq ? CE + (size_t)j * nm : CI + (size_t)W[j - neq] * nm;
+      for (int i = lane; i < n; i += 32) M[i * ld + j] = row[i];
+    }
+    for (int i = lane; i < n; i += 32) x[i] = a.x[(size_t)env * nm + i];
+    for (int j = lane; j < m; j += 32) nu[j] = j < neq ? a.lambda_eq[(size_t)env * a.neq_max + j] : a.lambda[(size_t)env * nm + j - neq];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int i = lane + 32 * t;
+      double s = 0.0;
+      if (i < n) {
+        if (a.gx) s = a.gx[(size_t)env * nm + i];
+        if (a.gtau)
+          for (int r = 0; r < na; r++) s += a.TA[((size_t)env * na + r) * nm + i] * a.gtau[(size_t)env * na + r];
+      }
+      y[t] = s;
+      const int j = i;
+      v[t] = 0.0;
+      if (j < neq && a.glambda_eq) v[t] = a.glambda_eq[(size_t)env * a.neq_max + j];
+      else if (j >= neq && j < m && a.glambda) v[t] = a.glambda[(size_t)env * nm + j - neq];
+    }
+    __syncwarp();
+    /* M = L^-1 G': forward substitution, a lane per column */
+    for (int j = lane; j < m; j += 32)
+      for (int i = 0; i < n; i++) {
+        double s = M[i * ld + j];
+        for (int k = 0; k < i; k++) s -= L[i * ld + k] * M[k * ld + j];
+        M[i * ld + j] = s / L[i * ld + i];
+      }
+    /* y = L^-1 y, column-oriented */
+    for (int i = 0; i < n; i++) {
+      const double yi = qg_lane(y, i) / L[i * ld + i];
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) {
+        const int k = lane + 32 * t;
+        if (k > i && k < n) y[t] -= L[k * ld + i] * yi;
+        else if (k == i) y[t] = yi;
+      }
+    }
+    __syncwarp();
+    /* Householder QR of M: reflector k in column k (rows k..n-1), R above the diagonal, its diagonal in rdiag.  A
+     * diagonal at or below eps times the largest so far is a dependent row (the solve's own test in add_constraint). */
+    double R_norm = 1.0;
+    for (int k = 0; k < m; k++) {
+      double s2 = 0.0;
+      for (int i = k + lane; i < n; i += 32) s2 += M[i * ld + k] * M[i * ld + k];
+      s2 = warp_sum(s2);
+      const double x0 = M[k * ld + k], nrm = sqrt(s2);
+      const double alpha = x0 > 0 ? -nrm : nrm;
+      if (!(nrm > TS_EPS * R_norm)) { ok = false; break; }
+      if (nrm > R_norm) R_norm = nrm;
+      const double bk = 1.0 / (nrm * (nrm + fabs(x0))); /* 2 / v'v */
+      __syncwarp();
+      if (lane == 0) { M[k * ld + k] = x0 - alpha; beta[k] = bk; rdiag[k] = alpha; }
+      __syncwarp();
+      for (int j = k + 1 + lane; j < m; j += 32) {
+        double d = 0.0;
+        for (int i = k; i < n; i++) d += M[i * ld + k] * M[i * ld + j];
+        d *= bk;
+        for (int i = k; i < n; i++) M[i * ld + j] -= d * M[i * ld + k];
+      }
+      __syncwarp();
+    }
+  }
+  if (ok) {
+    qg_reflect(M, ld, beta, n, m, true, y, lane); /* y = Q' L^-1 xb = [z1; z2] */
+    /* v = R^-T nub, column-oriented forward substitution */
+    for (int i = 0; i < m; i++) {
+      const double vi = qg_lane(v, i) / rdiag[i];
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) {
+        const int j = lane + 32 * t;
+        if (j > i && j < m) v[t] -= M[i * ld + j] * vi;
+        else if (j == i) v[t] = vi;
+      }
+    }
+    /* q = R^-1 (z1 + v), back substitution; then y = [-v; z2] */
+    double u[QP_SLOTS];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int j = lane + 32 * t;
+      u[t] = j < m ? y[t] + v[t] : 0.0;
+      if (j < m) y[t] = -v[t];
+    }
+    for (int i = m - 1; i >= 0; i--) {
+      const double qi = qg_lane(u, i) / rdiag[i];
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) {
+        const int j = lane + 32 * t;
+        if (j < i) u[t] -= M[j * ld + i] * qi;
+        else if (j == i) u[t] = qi;
+      }
+    }
+    qg_reflect(M, ld, beta, n, m, false, y, lane); /* p~ */
+    /* p = L^-T p~, column-oriented back substitution */
+    for (int i = n - 1; i >= 0; i--) {
+      const double pi = qg_lane(y, i) / L[i * ld + i];
+#pragma unroll
+      for (int t = 0; t < QP_SLOTS; t++) {
+        const int k = lane + 32 * t;
+        if (k < i) y[t] -= L[i * ld + k] * pi;
+        else if (k == i) y[t] = pi;
+      }
+    }
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int k = lane + 32 * t;
+      if (k < n) p[k] = y[t];
+      if (k < m) q[k] = u[t];
+    }
+  }
+  __syncwarp();
+  /* every byte of every requested part; zeros outside the env's sizes and for an env that was not differentiated */
+  if (lane == 0) a.status[env] = ok ? ST_OPTIMAL : ST_ERROR;
+  const int nx = ok ? n : 0, ne = ok ? neq : 0, ni = ok ? nin : 0;
+  if (a.dH)
+    qg_store(a.dH + (size_t)env * nm * nm, nm, nm, lane, [&](int i, int j) {
+      return (i < nx && j <= i) ? (j < i ? -(p[i] * x[j] + p[j] * x[i]) : -(p[i] * x[i])) : 0.0;
+    });
+  if (a.dg) qg_store(a.dg + (size_t)env * nm, 1, nm, lane, [&](int, int j) { return j < nx ? -p[j] : 0.0; });
+  if (a.dCE)
+    qg_store(a.dCE + (size_t)env * a.neq_max * nm, a.neq_max, nm, lane, [&](int r, int j) {
+      return (r < ne && j < nx) ? nu[r] * p[j] - q[r] * x[j] : 0.0;
+    });
+  if (a.dce0) qg_store(a.dce0 + (size_t)env * a.neq_max, 1, a.neq_max, lane, [&](int, int r) { return r < ne ? -q[r] : 0.0; });
+  if (a.dCI)
+    qg_store(a.dCI + (size_t)env * a.nin_max * nm, a.nin_max, nm, lane, [&](int r, int j) {
+      const int k = r < ni ? pos[r] : -1;
+      return (k >= 0 && j < nx) ? nu[neq + k] * p[j] - q[neq + k] * x[j] : 0.0;
+    });
+  if (a.dci0)
+    qg_store(a.dci0 + (size_t)env * a.nin_max, 1, a.nin_max, lane, [&](int, int r) {
+      const int k = r < ni ? pos[r] : -1;
+      return k >= 0 ? -q[neq + k] : 0.0;
+    });
+  const double* gt = (ok && a.gtau) ? a.gtau + (size_t)env * na : nullptr;
+  if (a.dTA)
+    qg_store(a.dTA + (size_t)env * na * nm, na, nm, lane, [&](int r, int j) { return (gt && j < nx) ? gt[r] * x[j] : 0.0; });
+  if (a.dta0) qg_store(a.dta0 + (size_t)env * na, 1, na, lane, [&](int, int r) { return gt ? gt[r] : 0.0; });
 }
 
 #ifndef TSIDB_EMU
@@ -3110,6 +3376,15 @@ __global__ void __launch_bounds__(32, TSIDB_Q_MIN_CTAS) tsidb_qp_kernel(const Qp
   extern __shared__ double smem[];
   const int lane = threadIdx.x & 31;
   for (int env = blockIdx.x; env < q.n_envs; env += gridDim.x) qp_env(q, smem, env, lane);
+}
+
+/* Adjoint of the generic QP solve (tsidb_qp_grad): one one-warp CTA per env on a persistent grid, dynamic shared memory
+ * qg_layout(n_max, nin_max).per_env doubles (L and M, n_max x odd stride each, plus vectors). */
+#define TSIDB_QG_MIN_CTAS 16 /* register cap: 128 per thread */
+__global__ void __launch_bounds__(32, TSIDB_QG_MIN_CTAS) tsidb_qp_grad_kernel(const QpGradArgs a) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31;
+  for (int env = blockIdx.x; env < a.n_envs; env += gridDim.x) qp_grad_env(a, smem, env, lane);
 }
 
 /* ---- Small batches: the whole tick of one env in ONE launch ----

@@ -10,6 +10,7 @@ from typing import Dict, Optional, Tuple
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _capi
 from ._capi import TsidbAuxOut, TsidbGaitConf, TsidbRefs, check, conf_to_c, load_library, model_to_c
@@ -438,25 +439,7 @@ class TsidEngine:
         shapes.  Returns new CUDA tensors x [N,n_max], status, iters [N] int32, active [N,n_max] int32 (CI rows of the
         working set in working-set order, -1 padded), lambda [N,n_max] (their multipliers), lambda_eq [N,neq_max] and,
         with TA and ta0, tau [N,na]."""
-        for k in ("H", "g", "sizes"):
-            if k not in problem:
-                raise ValueError(f"qp_solve: {k} is required")
-        for a, b in (("CE", "ce0"), ("CI", "ci0"), ("TA", "ta0")):
-            if (a in problem) != (b in problem):
-                raise ValueError(f"qp_solve: {a} and {b} go together")
-        unknown = set(problem) - set(self.PROBLEM_PARTS + self.ACTUATION_PARTS + ("sizes",))
-        if unknown:
-            raise ValueError(f"qp_solve: unknown parts {sorted(unknown)}")
-        n, nx = problem["g"].shape if problem["g"].dim() == 2 else (-1, -1)
-        neq = problem["ce0"].shape[-1] if "ce0" in problem else 0
-        nin = problem["ci0"].shape[-1] if "ci0" in problem else 0
-        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin),
-                  "TA": (n, self.na, nx), "ta0": (n, self.na), "sizes": (n, 3)}
-        for k, t in problem.items():
-            dt = torch.int32 if k == "sizes" else torch.float64
-            if not isinstance(t, torch.Tensor) or t.dtype is not dt or not t.is_cuda or t.get_device() != self._dev_index \
-                    or not t.is_contiguous() or tuple(t.shape) != shapes[k]:
-                raise TypeError(f"qp_solve: {k}: expected a contiguous {dt} tensor of shape {shapes[k]} on the engine's device")
+        n, nx, neq, nin = self._qp_problem("qp_solve", problem)
         f64 = dict(dtype=torch.float64, device=self.device)
         i32 = dict(dtype=torch.int32, device=self.device)
         out = {"x": torch.empty((n, nx), **f64), "status": torch.empty(n, **i32), "iters": torch.empty(n, **i32),
@@ -468,6 +451,78 @@ class TsidEngine:
         qo = _capi.TsidbQpOut(**{k: t.data_ptr() for k, t in out.items()})
         check(self.lib.tsidb_qp_solve(self.h, n, nx, neq, nin, C.byref(po), C.byref(qo), self._stream()), "tsidb_qp_solve")
         return out
+
+    def _qp_problem(self, what: str, problem: Dict[str, torch.Tensor]) -> Tuple[int, int, int, int]:
+        """Checks a problem dict in the layout of :meth:`problem_data` -> (N, n_max, neq_max, nin_max) from its shapes."""
+        for k in ("H", "g", "sizes"):
+            if k not in problem:
+                raise ValueError(f"{what}: {k} is required")
+        for a, b in (("CE", "ce0"), ("CI", "ci0"), ("TA", "ta0")):
+            if (a in problem) != (b in problem):
+                raise ValueError(f"{what}: {a} and {b} go together")
+        unknown = set(problem) - set(self.PROBLEM_PARTS + self.ACTUATION_PARTS + ("sizes",))
+        if unknown:
+            raise ValueError(f"{what}: unknown parts {sorted(unknown)}")
+        n, nx = problem["g"].shape if problem["g"].dim() == 2 else (-1, -1)
+        neq = problem["ce0"].shape[-1] if "ce0" in problem else 0
+        nin = problem["ci0"].shape[-1] if "ci0" in problem else 0
+        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin),
+                  "TA": (n, self.na, nx), "ta0": (n, self.na), "sizes": (n, 3)}
+        self._qp_tensors(what, problem, shapes)
+        return n, nx, neq, nin
+
+    def _qp_tensors(self, what: str, tensors: Dict[str, torch.Tensor], shapes: Dict[str, tuple]) -> None:
+        for k, t in tensors.items():
+            dt = torch.int32 if k in ("sizes", "status", "iters", "active") else torch.float64
+            if not isinstance(t, torch.Tensor) or t.dtype is not dt or not t.is_cuda or t.get_device() != self._dev_index \
+                    or not t.is_contiguous() or tuple(t.shape) != shapes[k]:
+                raise TypeError(f"{what}: {k}: expected a contiguous {dt} tensor of shape {shapes[k]} on the engine's device")
+
+    def qp_grad(self, problem: Dict[str, torch.Tensor], sol: Dict[str, torch.Tensor], grads: Dict[str, torch.Tensor],
+                parts: Optional[Tuple[str, ...]] = None) -> Dict[str, torch.Tensor]:
+        """Adjoint of :meth:`qp_solve` (tsidb_qp_grad): the gradient of a loss with respect to the problem's parts from its
+        gradient with respect to the solve's outputs.  `problem` is what qp_solve was given and `sol` what it returned
+        (x, status, active, lambda, lambda_eq are read).  `grads` holds any of x [N,n_max], lambda [N,n_max],
+        lambda_eq [N,neq_max] and tau [N,na] (absent = zero; tau needs TA).  `parts` names the gradients to compute among
+        the float parts of `problem` (default: all of them).  Returns new CUDA tensors of those parts' shapes and status
+        [N] int32: 0 where the env was differentiated, 4 (zero gradients) where it was not (a solve status other than 0,
+        an invalid working set, H not positive definite or dependent working-set rows).  The gradient is the one of the
+        final working set's KKT system, and that of H is lower triangular (the solve reads only that triangle); see
+        INTEGRATION.md, "Differentiating a QP"."""
+        n, nx, neq, nin = self._qp_problem("qp_grad", problem)
+        floats = tuple(k for k in self.PROBLEM_PARTS + self.ACTUATION_PARTS if k in problem)
+        parts = floats if parts is None else tuple(parts)
+        if set(parts) - set(floats):
+            raise ValueError(f"qp_grad: parts {sorted(set(parts) - set(floats))} are not float parts of the problem")
+        need = ("x", "status", "active", "lambda", "lambda_eq")
+        if set(need) - set(sol):
+            raise ValueError(f"qp_grad: sol needs {need}")
+        if set(grads) - {"x", "lambda", "lambda_eq", "tau"}:
+            raise ValueError(f"qp_grad: unknown gradients {sorted(set(grads) - {'x', 'lambda', 'lambda_eq', 'tau'})}")
+        if "tau" in grads and "TA" not in problem:
+            raise ValueError("qp_grad: a tau gradient needs TA")
+        shapes = {"x": (n, nx), "status": (n,), "active": (n, nx), "lambda": (n, nx), "lambda_eq": (n, neq), "tau": (n, self.na)}
+        sol = {k: sol[k] for k in need}
+        self._qp_tensors("qp_grad", sol, shapes)
+        self._qp_tensors("qp_grad", grads, shapes)
+        out = {k: torch.empty_like(problem[k]) for k in parts}
+        out["status"] = torch.empty(n, dtype=torch.int32, device=self.device)
+        po = _capi.TsidbProblemOut(**{k: t.data_ptr() for k, t in problem.items()})
+        so = _capi.TsidbQpOut(**{k: t.data_ptr() for k, t in sol.items()})
+        gi = _capi.TsidbQpOut(**{k: t.data_ptr() for k, t in grads.items()})
+        go = _capi.TsidbProblemOut(**{k: out[k].data_ptr() for k in parts})
+        check(self.lib.tsidb_qp_grad(self.h, n, nx, neq, nin, C.byref(po), C.byref(so), C.byref(gi), C.byref(go),
+                                     out["status"].data_ptr(), self._stream()), "tsidb_qp_grad")
+        return out
+
+    def qp_layer(self, problem: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+        """:meth:`qp_solve` as a differentiable layer: the same result, with x, lambda, lambda_eq and tau carrying a
+        grad_fn for every float tensor of `problem` that requires grad; the backward pass is :meth:`qp_grad` (first
+        order only).  sizes gets no gradient, and an env that was not differentiated contributes zero."""
+        keys = tuple(k for k in self.PROBLEM_PARTS + self.ACTUATION_PARTS if k in problem)
+        outs = _QpLayer.apply(self, problem["sizes"], keys, *(problem[k] for k in keys))
+        names = ("x", "lambda", "lambda_eq", "status", "iters", "active") + (("tau",) if "TA" in problem else ())
+        return dict(zip(names, outs))
 
     def ci_row(self, block: int, side: int, i: int) -> int:
         return int(self.lib.tsidb_ci_row(self.h, block, side, i))
@@ -498,6 +553,33 @@ class TsidEngine:
         ms = (C.c_float * 5)()
         check(self.lib.tsidb_last_tick_ms(self.h, ms), "tsidb_last_tick_ms")
         return {k: float(ms[i]) for i, k in enumerate(self.KERNEL_NAMES)}
+
+
+class _QpLayer(torch.autograd.Function):
+    """forward: TsidEngine.qp_solve; backward: TsidEngine.qp_grad (the tensors of `keys` are the problem's float parts)."""
+
+    @staticmethod
+    def forward(ctx, engine, sizes, keys, *tensors):
+        problem = dict(zip(keys, tensors), sizes=sizes)
+        sol = engine.qp_solve(problem)
+        ctx.engine, ctx.keys = engine, keys
+        ctx.mark_non_differentiable(sol["status"], sol["iters"], sol["active"])
+        ctx.save_for_backward(sizes, *tensors, sol["x"], sol["status"], sol["active"], sol["lambda"], sol["lambda_eq"])
+        outs = (sol["x"], sol["lambda"], sol["lambda_eq"], sol["status"], sol["iters"], sol["active"])
+        return outs + ((sol["tau"],) if "tau" in sol else ())
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, *grad_outs):
+        saved = ctx.saved_tensors
+        nk = len(ctx.keys)
+        problem = dict(zip(ctx.keys, saved[1:1 + nk]), sizes=saved[0])
+        sol = dict(zip(("x", "status", "active", "lambda", "lambda_eq"), saved[1 + nk:]))
+        names = ("x", "lambda", "lambda_eq", None, None, None, "tau")
+        grads = {k: g.contiguous() for k, g in zip(names, grad_outs) if k is not None and g is not None}
+        parts = tuple(k for i, k in enumerate(ctx.keys) if ctx.needs_input_grad[3 + i])
+        out = ctx.engine.qp_grad(problem, sol, grads, parts)
+        return (None, None, None) + tuple(out.get(k) for k in ctx.keys)
 
 
 def fp64_peak_tflops(device: int = 0) -> float:
