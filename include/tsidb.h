@@ -316,6 +316,25 @@ int tsidb_qp_grad(tsidb_handle* h, int n_envs, int n_max, int neq_max, int nin_m
                   const tsidb_qp_out* sol, const tsidb_qp_out* grad_in, const tsidb_problem_out* grad_out, int32_t* status,
                   void* cuda_stream);
 
+/* ---- differentiating through the task references ------------------------------------------------------------------
+ * tsidb_refs_grad is the adjoint of the map references -> (g, ce0) of tsidb_problem_data: given dg = dL/dg [N][n_max] and
+ * dce0 = dL/dce0 [N][neq_max] (row-major DEVICE arrays with the caller's strides, n_max >= and neq_max >= the values of
+ * tsidb_problem_sizes, e.g. what tsidb_qp_grad returns; NULL counts as zero), it writes dL/d of each reference array the
+ * caller asks for in `out` (NULL = not written).  Only g and the contact-motion rows of ce0 depend on the references, and
+ * only columns 0..nv of dg and rows 6..6+6nc of dce0 are read, so padding and appended variables or rows may hold
+ * anything.  q, v, contact_mask, refs and `layout` as in tsidb_problem_data; `layout` also applies to the outputs.  The
+ * gradient is taken with respect to the raw doubles of each array (the 9 column-major entries of an SE3 reference's
+ * rotation, not a tangent vector), for a NULL reference array with respect to the default that was used; every requested
+ * byte is written, and the contact reference of a foot that is not in contact gets exact zeros.  The SE3 logarithm is
+ * differentiated branch by branch as the tick computes it (INTEGRATION.md, "Differentiating through the references").
+ * No workspace of the handle is used, so the call may run on any stream.  Asynchronous on cuda_stream. */
+typedef struct tsidb_refs_out { /* dL/d of each tsidb_refs array, same shapes; NULL = not written */
+  double *com, *foot_lf, *foot_rf, *contact_lf, *contact_rf, *posture;
+} tsidb_refs_out;
+int tsidb_refs_grad(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v, const uint8_t* contact_mask,
+                    const tsidb_refs* refs, int n_max, int neq_max, const double* dg, const double* dce0,
+                    const tsidb_refs_out* out, void* cuda_stream);
+
 /* controller.integrate_dv(q, v, dv, dt) (ref:ctrl/WalkController.py:291-295,
  * ref:legacy/biped.py:236-240): v_mean = v + dt/2*dv; v += dt*dv;
  * q = pin.integrate(q, dt*v_mean).  In place on device arrays.                   */

@@ -109,6 +109,10 @@ class TsidbQpOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("x", "status", "iters", "active", "lambda", "lambda_eq", "tau")]
 
 
+class TsidbRefsOut(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("com", "foot_lf", "foot_rf", "contact_lf", "contact_rf", "posture")]
+
+
 def _fill(arr, values) -> None:
     v = np.asarray(values, dtype=np.float64).ravel()
     for i, x in enumerate(v):
@@ -275,6 +279,8 @@ def load_library() -> C.CDLL:
     lib.tsidb_qp_grad.argtypes = [vp, ip, ip, ip, ip, C.POINTER(TsidbProblemOut), C.POINTER(TsidbQpOut), C.POINTER(TsidbQpOut),
                                   C.POINTER(TsidbProblemOut), vp, vp]
     lib.tsidb_qp_grad.restype = ip
+    lib.tsidb_refs_grad.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, vp, vp, C.POINTER(TsidbRefsOut), vp]
+    lib.tsidb_refs_grad.restype = ip
     _LIB = lib
     return lib
 
@@ -292,4 +298,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
     "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve", "tsidb_qp_grad",
+    "tsidb_refs_grad",
 ]

@@ -205,6 +205,8 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
   if (const char* e = getenv("TSIDB_D_CARVEOUT")) { const int v = atoi(e); if (v >= d_carve && v <= 100) d_carve = v; } /* tuning knob */
   TSIDB_ATTR(tsidb_dynamics_kernel<26>, smem, TSIDB_D_CTAS_PER_SM, "dynamics kernel", d_carve);
   TSIDB_ATTR(tsidb_dynamics_kernel<24>, smem, TSIDB_D_CTAS_PER_SM, "dynamics kernel", d_carve);
+  TSIDB_ATTR(tsidb_refs_grad_kernel<26>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_refs_grad_kernel<24>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<26, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_SMEM_DOUBLES(26) * sizeof(double)))));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<24, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_SMEM_DOUBLES(24) * sizeof(double)))));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<26, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_LOCAL_SMEM_DOUBLES(26) * sizeof(double)))));
@@ -875,6 +877,48 @@ extern "C" int tsidb_qp_grad(tsidb_handle* h, int n_envs, int n_max, int neq_max
   long blocks = (long)per_sm * h->sm_count; /* persistent */
   if (blocks > n_envs) blocks = n_envs;
   tsidb_qp_grad_kernel<<<(int)blocks, 32, smem, (cudaStream_t)cuda_stream>>>(a);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
+/* adjoint of the reference terms: one launch that recomputes K1 per env, no workspace of the handle */
+extern "C" int tsidb_refs_grad(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
+                               const uint8_t* contact_mask, const tsidb_refs* refs, int n_max, int neq_max, const double* dg,
+                               const double* dce0, const tsidb_refs_out* out, void* cuda_stream) {
+  if (!h || !q || !v || !out) { g_err = "tsidb_refs_grad: null argument"; return -1; }
+  if (n_envs <= 0 || n_envs > h->max_envs) { g_err = "tsidb_refs_grad: n_envs must be in [1, max_envs]"; return -1; }
+  if (layout != 0 && layout != 1) { g_err = "tsidb_refs_grad: layout must be 0 ([N][dof]) or 1 ([dof][N])"; return -1; }
+  int nx, neq, nin;
+  problem_maxima(h, &nx, &neq, &nin);
+  if (n_max < nx || neq_max < neq) {
+    g_err = "tsidb_refs_grad: n_max and neq_max must be at least tsidb_problem_sizes' n_max and neq_max";
+    return -1;
+  }
+  for (const void* p : {(const void*)q, (const void*)v, (const void*)dg, (const void*)dce0, (const void*)out->com,
+                        (const void*)out->foot_lf, (const void*)out->foot_rf, (const void*)out->contact_lf,
+                        (const void*)out->contact_rf, (const void*)out->posture})
+    if (((uintptr_t)p & 7) != 0) { g_err = "tsidb_refs_grad: fp64 arrays must be 8-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  TickArgs a;
+  memset(&a, 0, sizeof a);
+  a.n_envs = n_envs; a.layout = layout;
+  a.q = q; a.v = v; a.mask = contact_mask;
+  if (refs) {
+    a.r_com = refs->com; a.r_foot[0] = refs->foot_lf; a.r_foot[1] = refs->foot_rf;
+    a.r_contact[0] = refs->contact_lf; a.r_contact[1] = refs->contact_rf; a.r_posture = refs->posture;
+  }
+  a.slot = h->slot;
+  a.tables = h->tables;
+  RefsGradArgs r;
+  r.n_max = n_max; r.neq_max = neq_max; r.dg = dg; r.dce0 = dce0;
+  r.out[0] = out->com; r.out[1] = out->foot_lf; r.out[2] = out->foot_rf;
+  r.out[3] = out->contact_lf; r.out[4] = out->contact_rf; r.out[5] = out->posture;
+  int blocks = (n_envs + TSIDB_R_CTA_WARPS - 1) / TSIDB_R_CTA_WARPS;
+  if (blocks > h->sm_count) blocks = h->sm_count; /* persistent */
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  if (h->dc.nv == 26) tsidb_refs_grad_kernel<26><<<blocks, 32 * TSIDB_R_CTA_WARPS, TSIDB_R_SMEM, st>>>(a, r);
+  else tsidb_refs_grad_kernel<24><<<blocks, 32 * TSIDB_R_CTA_WARPS, TSIDB_R_SMEM, st>>>(a, r);
   CK(cudaGetLastError());
   h->launches += 1;
   return 0;

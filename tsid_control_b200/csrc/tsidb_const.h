@@ -150,6 +150,14 @@ struct QpGradArgs {
   int32_t* status;
 };
 
+/* arguments of the adjoint of the reference terms (tsidb_refs_grad): dL/dg [N][n_max] and dL/dce0 [N][neq_max] (NULL =
+ * zero) and dL/d of the tsidb_refs arrays com, foot_lf, foot_rf, contact_lf, contact_rf, posture (NULL = not written) */
+struct RefsGradArgs {
+  int32_t n_max, neq_max;
+  const double *dg, *dce0;
+  double* out[6];
+};
+
 struct TickArgs {
   int32_t n_envs, layout, pad_;
   const double* q;

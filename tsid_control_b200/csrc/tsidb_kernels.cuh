@@ -2446,6 +2446,221 @@ TSIDB_DEV void problem_env(const DevConst& C, const double* pt, double* sm, cons
   if (o.sizes && lane < 3) o.sizes[(size_t)env * 3 + lane] = (lane == 0) ? n : ((lane == 1) ? neq : nin);
 }
 
+/* ================================================================= adjoint of the reference terms (tsidb_refs_grad) */
+/* Reverse mode of log6_dev, branch for branch as log6_dev computes it: given (ol, oa) = dL/d(out lin, out ang), adds
+ * dL/dR (9, row-major, R taken as 9 free entries: the formulas are differentiated as written, not on SO(3)) to Rb and
+ * dL/dp to pb.  theta enters through the trace only, tr = R0 + R4 + R8:
+ *   small angle (theta < prec3): w = (R - R^T)^vee / 2 has no theta term; alpha and beta are series in s = theta^2, whose
+ *     derivative in the trace is -theta / sin(theta) = -(1 + s/6) to rounding; at the clamp tr >= 3 (theta = 0) that is the
+ *     interior limit -1.  Nothing is differentiated through acos or the clamp, so theta = 0 gives a finite gradient.
+ *   generic: dtheta/dtr = -1 / (2 sin theta); t = theta / (2 sin theta), alpha = theta sin / (2 (1 - cos)),
+ *     beta = (1 - alpha) / theta^2, differentiated in closed form.
+ *   near pi (theta >= pi - 1e-2): w_k = sign_k sqrt((R_kk + cphi) theta^2 / (1 + cphi)), cphi = -(tr - 1)/2; the signs are
+ *     piecewise constant, and a component whose sqrt argument is <= 0 (w_k = 0) contributes zero.  At tr <= -1
+ *     (theta = pi) dtheta/dtr is unbounded and the theta terms contribute zero. */
+TSIDB_DEV void log6_adj(const double* R, const double* p, const double* ol, const double* oa, double* Rb, double* pb) {
+  const double PI = 3.14159265358979323846;
+  const double prec3 = 1.220703125e-4;
+  const double tr = R[0] + R[4] + R[8];
+  double th;
+  if (tr >= 3.0) th = 0.0;
+  else if (tr <= -1.0) th = PI;
+  else th = acos((tr - 1.0) / 2.0);
+  const double ct = (tr >= 3.0) ? 1.0 : ((tr <= -1.0) ? -1.0 : (tr - 1.0) / 2.0);
+  const double st = sqrt(fmax((1.0 - ct) * (1.0 + ct), 0.0));
+  const double dth = st > 0.0 ? -0.5 / st : 0.0; /* dtheta/dtr */
+  const bool near_pi = th >= PI - 1e-2;
+  double w[3], v[3] = {R[7] - R[5], R[2] - R[6], R[3] - R[1]}, tk[3] = {0, 0, 0}, bpi = 0.0, cphi = 0.0, t = 0.5;
+  if (near_pi) {
+    cphi = -(tr - 1.0) / 2.0;
+    bpi = th * th / (1.0 + cphi);
+    tk[0] = (R[0] + cphi) * bpi; tk[1] = (R[4] + cphi) * bpi; tk[2] = (R[8] + cphi) * bpi;
+    w[0] = (R[7] > R[5] ? 1.0 : -1.0) * (tk[0] > 0 ? sqrt(tk[0]) : 0.0);
+    w[1] = (R[2] > R[6] ? 1.0 : -1.0) * (tk[1] > 0 ? sqrt(tk[1]) : 0.0);
+    w[2] = (R[3] > R[1] ? 1.0 : -1.0) * (tk[2] > 0 ? sqrt(tk[2]) : 0.0);
+  } else {
+    t = ((th > prec3) ? th / st : 1.0) / 2.0;
+    w[0] = t * v[0]; w[1] = t * v[1]; w[2] = t * v[2];
+  }
+  const double s = th * th;
+  double alpha, beta;
+  if (th < prec3) {
+    alpha = 1.0 - s / 12.0 - s * s / 720.0;
+    beta = 1.0 / 12.0 + s / 720.0;
+  } else {
+    alpha = th * st / (2.0 * (1.0 - ct));
+    beta = 1.0 / s - st / (2.0 * th * (1.0 - ct));
+  }
+  /* out_lin = alpha p - w x p / 2 + beta (w.p) w, out_ang = w */
+  const double wdp = dot3(w, p), wdo = dot3(w, ol);
+  double lxw[3], pxl[3], wb[3];
+  cross3(ol, w, lxw);
+  cross3(p, ol, pxl);
+#pragma unroll
+  for (int k = 0; k < 3; k++) {
+    pb[k] += alpha * ol[k] - 0.5 * lxw[k] + (beta * wdo) * w[k];
+    wb[k] = oa[k] - 0.5 * pxl[k] + beta * (wdo * p[k] + wdp * ol[k]);
+  }
+  const double ab = dot3(ol, p), bb = wdp * wdo; /* dL/dalpha, dL/dbeta */
+  double trb;
+  if (th < prec3) {
+    const double ds = (tr >= 3.0) ? -1.0 : -(1.0 + s / 6.0); /* ds/dtr */
+    trb = (ab * (-1.0 / 12.0 - s / 360.0) + bb / 720.0) * ds;
+  } else {
+    const double da = (st - th) / (2.0 * (1.0 - ct)); /* dalpha/dtheta */
+    const double db = -(da + 2.0 * th * beta) / s;     /* dbeta/dtheta */
+    trb = (ab * da + bb * db) * dth;
+  }
+  if (near_pi) {
+    double cb = 0.0, bpib = 0.0;
+    const double dd[3] = {R[0], R[4], R[8]};
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+      if (tk[k] > 0) {
+        const double tb = wb[k] * (w[k] > 0 ? 1.0 : -1.0) * 0.5 / sqrt(tk[k]);
+        Rb[4 * k] += tb * bpi;
+        cb += tb * bpi;
+        bpib += tb * (dd[k] + cphi);
+      }
+    }
+    cb -= bpib * s / ((1.0 + cphi) * (1.0 + cphi));
+    trb += -0.5 * cb + bpib * 2.0 * th / (1.0 + cphi) * dth;
+  } else {
+    const double vb[3] = {t * wb[0], t * wb[1], t * wb[2]};
+    Rb[7] += vb[0]; Rb[5] -= vb[0];
+    Rb[2] += vb[1]; Rb[6] -= vb[1];
+    Rb[3] += vb[2]; Rb[1] -= vb[2];
+    if (th > prec3) {
+      const double dt = (st - th * ct) / (2.0 * st * st); /* dt/dtheta */
+      trb += dot3(wb, v) * dt * dth;
+    }
+  }
+  Rb[0] += trb; Rb[4] += trb; Rb[8] += trb;
+}
+
+/* dL/d(references) of one env after K1 (frames, JF, Jcom in shared memory; references staged): the adjoint of the task
+ * right-hand sides (k2_assemble / se3_rhs) that g and the contact-motion rows of ce0 carry.
+ *   g_dv = -(w_foot JF^T b_foot + w_com Jcom^T b_com + w_post S^T b_post + w_am Ag^T b_am), ce0[6 + 6s + k] = -b_mot[f][k],
+ * so bb_foot = -w_foot JF gb, bb_com = -w_com Jcom gb, bb_post = -w_post gb[6:], bb_mot = -ce0b[contact rows]; the AM task
+ * has no reference.  lanes 0..3: the SE3 laws (contact LF, contact RF, foot LF, foot RF), 4..6: CoM, lanes < na: posture. */
+template <int NV>
+TSIDB_DEV void refs_adjoint_env(const DevConst& C, const double* mdl, double* sm, const TickArgs& a, const RefsGradArgs& r,
+                                int env, int lane, int mask) {
+  constexpr int nv = NV, na = NV - 6;
+  const int f0 = (mask & 1) ? 0 : 1; /* foot of contact slot 0; slot 1 is RF */
+  double* gb = sm + SM_oBv;       /* dL/dg_dv at [0, nv), bb_foot at [32, 44), bb_com at [44, 47) */
+  const double* fr = sm + SM_oFr;
+  const double* rf = sm + SM_oRef;
+  if (lane < nv) gb[lane] = r.dg ? r.dg[(size_t)env * r.n_max + lane] : 0.0;
+  __syncwarp();
+  double acc = 0.0;
+  if (lane < 12) {
+#pragma unroll 2
+    for (int j = 0; j < nv; j++) acc += sm[SM_oJF + lane * TSIDB_NVX + j] * gb[j];
+    acc *= -C.w_foot;
+  } else if (lane < 15) {
+#pragma unroll 2
+    for (int j = 0; j < nv; j++) acc += sm[SM_oJcom + (lane - 12) * TSIDB_NVX + j] * gb[j];
+    acc *= -C.w_com;
+  }
+  double postb = 0.0;
+  if (lane < na) postb = -C.w_post * gb[6 + lane];
+  __syncwarp();
+  if (lane < 15) gb[32 + lane] = acc;
+  __syncwarp();
+  if (lane < 4) {
+    const int f = lane & 1;
+    const bool is_contact = lane < 2;
+    double* out = is_contact ? r.out[3 + f] : r.out[1 + f];
+    const int nd = is_contact ? 12 : 24;
+    if (out) {
+      double bb[6];
+      const bool live = !is_contact || ((mask >> f) & 1);
+      if (is_contact) {
+        const int row = 6 + 6 * ((f == f0) ? 0 : 1);
+#pragma unroll
+        for (int k = 0; k < 6; k++) bb[k] = (live && r.dce0) ? -r.dce0[(size_t)env * r.neq_max + row + k] : 0.0;
+      } else {
+#pragma unroll
+        for (int k = 0; k < 6; k++) bb[k] = gb[32 + 6 * f + k];
+      }
+      const double* gains = C.kp_contact + (is_contact ? 0 : 12);
+      const double* ref = is_contact ? rf + RF_CONTACT + 12 * f : rf + RF_FOOT + 24 * f;
+      const double* pf = fr + FR_OMF + f * 12;
+      const double* Rf = pf + 3;
+      /* the 3 x 3 work of the lane lives in K1's scratch region (dead after K1), not in registers: E, dL/dE, ep, dL/dep */
+      double* E = sm + SM_oM + 32 * lane;
+      double* ep = E + 9;
+      double* Eb = E + 12;
+      double* epb = E + 21;
+      {
+        double Rr[9], dp[3];
+#pragma unroll
+        for (int c = 0; c < 3; c++)
+#pragma unroll
+          for (int q = 0; q < 3; q++) Rr[3 * q + c] = ref[3 + 3 * c + q];
+        dp[0] = ref[0] - pf[0]; dp[1] = ref[1] - pf[1]; dp[2] = ref[2] - pf[2];
+#pragma unroll
+        for (int i = 0; i < 3; i++)
+#pragma unroll
+          for (int j = 0; j < 3; j++) E[3 * i + j] = Rf[i] * Rr[j] + Rf[3 + i] * Rr[3 + j] + Rf[6 + i] * Rr[6 + j];
+        mtv3(Rf, dp, ep);
+      }
+#pragma unroll
+      for (int k = 0; k < 12; k++) Eb[k] = 0.0; /* Eb and epb */
+      {
+        double ol[3], oa[3];
+#pragma unroll
+        for (int k = 0; k < 3; k++) { ol[k] = gains[k] * bb[k]; oa[k] = gains[3 + k] * bb[3 + k]; }
+        log6_adj(E, ep, ol, oa, Eb, epb);
+      }
+      auto put = [&](int k, double val) { out[eidx(a, env, k, nd)] = live ? val : 0.0; }; /* not in contact: exact zeros */
+      double t3[3];
+      mv3(Rf, epb, t3); /* ep = Rf^T (p_ref - p_f) */
+      put(0, t3[0]); put(1, t3[1]); put(2, t3[2]);
+#pragma unroll
+      for (int c = 0; c < 3; c++) /* E = Rf^T R_ref: dL/dR_ref = Rf dL/dE, column c of it to ref[3 + 3c ..] */
+#pragma unroll
+        for (int q = 0; q < 3; q++) put(3 + 3 * c + q, Rf[3 * q] * Eb[c] + Rf[3 * q + 1] * Eb[3 + c] + Rf[3 * q + 2] * Eb[6 + c]);
+      if (!is_contact) { /* vl = Rf^T v_ref, al = Rf^T a_ref */
+        double kb[6];
+#pragma unroll
+        for (int k = 0; k < 6; k++) kb[k] = gains[6 + k] * bb[k];
+        mv3(Rf, kb, t3);     put(12, t3[0]); put(13, t3[1]); put(14, t3[2]);
+        mv3(Rf, kb + 3, t3); put(15, t3[0]); put(16, t3[1]); put(17, t3[2]);
+        mv3(Rf, bb, t3);     put(18, t3[0]); put(19, t3[1]); put(20, t3[2]);
+        mv3(Rf, bb + 3, t3); put(21, t3[0]); put(22, t3[1]); put(23, t3[2]);
+      }
+    }
+  } else if (lane < 7) {
+    const int q = lane - 4;
+    const double bb = gb[44 + q];
+    if (r.out[0]) {
+      r.out[0][eidx(a, env, q, 9)] = C.kp_com[q] * bb;
+      r.out[0][eidx(a, env, 3 + q, 9)] = C.kd_com[q] * bb;
+      r.out[0][eidx(a, env, 6 + q, 9)] = bb;
+    }
+  }
+  if (lane < na && r.out[5]) r.out[5][eidx(a, env, lane, na)] = mdl[MDL_oPOST + lane] * postb;
+}
+
+/* one env of tsidb_refs_grad: q, v and the references staged as the dynamics kernel stages them, K1, then the adjoint.
+ * Nothing is written to the handle's images. */
+template <int NV>
+TSIDB_DEV void refs_grad_env(const DevConst& C, const double* mdl, double* sm, const TickArgs& a, const RefsGradArgs& r,
+                             int env, int lane) {
+  constexpr int nv = NV, na = NV - 6, nq = NV + 1;
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  if (lane < nq) sm[SM_oQV + lane] = ldin(a.q, a, env, lane, nq);
+  if (lane < nv) sm[SM_oQV + 32 + lane] = ldin(a.v, a, env, lane, nv);
+  stage_refs(C, mdl, sm, a, env, lane, na);
+  __syncwarp();
+  k1_dynamics<NV>(C, mdl, sm, lane);
+  stage_refs_wait();
+  const int mask = a.mask ? (a.mask[env] & 3) : 3;
+  refs_adjoint_env<NV>(C, mdl, sm, a, r, env, lane, mask);
+}
+
 /* ================================================================= generic QP solve of one env (tsidb_qp_solve) */
 /* eiquadprog-fast solve_quadprog on a caller-supplied problem, min 1/2 x'Hx + g'x s.t. CE x + ce0 = 0, CI x + ci0 >= 0,
  * step for step as the oracle's eq_solve states it: LLT of H, J = L^-T, x0 = -H^-1 g, the equalities added one by one,
@@ -3385,6 +3600,26 @@ __global__ void __launch_bounds__(32, TSIDB_QG_MIN_CTAS) tsidb_qp_grad_kernel(co
   extern __shared__ double smem[];
   const int lane = threadIdx.x & 31;
   for (int env = blockIdx.x; env < a.n_envs; env += gridDim.x) qp_grad_env(a, smem, env, lane);
+}
+
+/* Adjoint of the reference terms (tsidb_refs_grad): the dynamics kernel's per-env shared memory and a CTA of warps sharing
+ * the staged model table, one warp per env on a persistent grid, no images and no class sort.  12 warps per CTA and one
+ * CTA per SM leave 168 registers per thread, which K1 followed by the adjoint needs to stay within the dynamics kernel's
+ * spills (at 16 warps and 128 registers it spilled 688 bytes). */
+#define TSIDB_R_CTA_WARPS 12
+#define TSIDB_R_SMEM (((size_t)TSIDB_R_CTA_WARPS * SM_PER_ENV + MDL_SIZE) * sizeof(double))
+template <int NV>
+__global__ void __launch_bounds__(32 * TSIDB_R_CTA_WARPS, 1)
+tsidb_refs_grad_kernel(const TickArgs a, const RefsGradArgs r) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  double* sm = smem + wid * SM_PER_ENV;
+  const DevConst& C = g_const[a.slot];
+  double* mdl = smem + TSIDB_R_CTA_WARPS * SM_PER_ENV;
+  load_table(mdl, a.tables + TBL_oMDL, MDL_SIZE, threadIdx.x, blockDim.x);
+  __syncthreads();
+  for (int env = blockIdx.x * TSIDB_R_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_R_CTA_WARPS)
+    refs_grad_env<NV>(C, mdl, sm, a, r, env, lane);
 }
 
 /* ---- Small batches: the whole tick of one env in ONE launch ----

@@ -524,6 +524,73 @@ class TsidEngine:
         names = ("x", "lambda", "lambda_eq", "status", "iters", "active") + (("tau",) if "TA" in problem else ())
         return dict(zip(names, outs))
 
+    def _state_args(self, what: str, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor],
+                    refs: Optional[Dict[str, torch.Tensor]]) -> TsidbRefs:
+        """Checks q, v, contact_mask and refs as :meth:`problem_data` does -> the refs struct (a missing name: the default)."""
+        n = q.shape[0]
+        self._chk(q, n, self.nq, "q")
+        self._chk(v, n, self.nv, "v")
+        if contact_mask is not None:
+            if contact_mask.dtype is not torch.uint8 or not contact_mask.is_cuda or contact_mask.get_device() != self._dev_index \
+                    or contact_mask.shape != (n,):
+                raise TypeError("contact_mask: expected a uint8 [N] tensor on the engine's device")
+        unknown = set(refs or ()) - set(REF_KEYS)
+        if unknown:
+            raise ValueError(f"{what}: unknown references {sorted(unknown)}; choose from {REF_KEYS}")
+        r = TsidbRefs()
+        for k, nd in self._ref_dims:
+            t = refs.get(k) if refs else None
+            setattr(r, k, None if t is None else self._chk(t, n, nd, k).data_ptr())
+        return r
+
+    def refs_grad(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                  refs: Optional[Dict[str, torch.Tensor]] = None, dg: Optional[torch.Tensor] = None,
+                  dce0: Optional[torch.Tensor] = None, parts: Optional[Tuple[str, ...]] = None) -> Dict[str, torch.Tensor]:
+        """Adjoint of the references' part of :meth:`problem_data` (tsidb_refs_grad): from dg = dL/dg [N,n_max] and
+        dce0 = dL/dce0 [N,neq_max] (None = zero; n_max, neq_max at least those of problem_sizes(), e.g. what
+        :meth:`qp_grad` returns), new CUDA tensors {name: [N,k]} = dL/d of the references named in `parts` (default: all of
+        REF_KEYS).  q, v, contact_mask and refs as in :meth:`problem_data`; a reference left out of `refs` is the handle's
+        default and its gradient is the one at that default.  SE3 references are differentiated in their raw 12 or 24
+        doubles (the rotation as its 9 column-major entries); the contact reference of a foot that is not in contact
+        gets zeros.  See INTEGRATION.md, "Differentiating through the references"."""
+        r = self._state_args("refs_grad", q, v, contact_mask, refs)
+        n = q.shape[0]
+        nx, neq, _ = self.problem_sizes()
+        parts = REF_KEYS if parts is None else tuple(parts)
+        if set(parts) - set(REF_KEYS):
+            raise ValueError(f"refs_grad: parts {sorted(set(parts) - set(REF_KEYS))} are not references; choose from {REF_KEYS}")
+        for name, t, lo in (("dg", dg, nx), ("dce0", dce0, neq)):
+            if t is None:
+                continue
+            if not isinstance(t, torch.Tensor) or t.dtype is not torch.float64 or not t.is_cuda or t.get_device() != self._dev_index \
+                    or not t.is_contiguous() or t.dim() != 2 or t.shape[0] != n or t.shape[1] < lo:
+                raise TypeError(f"refs_grad: {name}: expected a contiguous torch.float64 tensor of shape ({n}, >= {lo}) on the "
+                                f"engine's device")
+        dims = dict(self._ref_dims)
+        out = {k: torch.empty((n, dims[k]), dtype=torch.float64, device=self.device) for k in parts}
+        ro = _capi.TsidbRefsOut(**{k: t.data_ptr() for k, t in out.items()})
+        check(self.lib.tsidb_refs_grad(self.h, n, 0, q.data_ptr(), v.data_ptr(),
+                                       contact_mask.data_ptr() if contact_mask is not None else None, C.byref(r),
+                                       dg.shape[1] if dg is not None else nx, dce0.shape[1] if dce0 is not None else neq,
+                                       dg.data_ptr() if dg is not None else None, dce0.data_ptr() if dce0 is not None else None,
+                                       C.byref(ro), self._stream()), "tsidb_refs_grad")
+        return out
+
+    def tick_layer(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                   refs: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
+        """A tick as a differentiable function of its references: {tau [N,na], dv [N,nv], f [N,24], status, iters [N]
+        int32}, with tau, dv and f carrying a grad_fn for every tensor of `refs` that requires grad (first order only).
+        f holds the corner forces in the tick's fixed slots, LF 0..11 and RF 12..23, zero for a foot not in contact.
+        The forward pass is :meth:`problem_data` (with TA, ta0) followed by :meth:`qp_solve`, not the fast tick: the
+        backward pass (:meth:`qp_grad` for g and ce0, then :meth:`refs_grad`) must differentiate the working set its own
+        forward pass found, and the two solves can end in different working sets at degenerate contact-corner ties.  That
+        costs time: about 74 ms for the forward pass at 65536 walking envs against 3 ms for a tick.  An env whose solve or
+        adjoint status is not 0 contributes zero.  q, v and contact_mask get no gradient."""
+        self._state_args("tick_layer", q, v, contact_mask, refs)
+        keys = tuple(k for k in REF_KEYS if refs and refs.get(k) is not None)
+        outs = _TickLayer.apply(self, q, v, contact_mask, keys, *(refs[k] for k in keys))
+        return dict(zip(("tau", "dv", "f", "status", "iters"), outs))
+
     def ci_row(self, block: int, side: int, i: int) -> int:
         return int(self.lib.tsidb_ci_row(self.h, block, side, i))
 
@@ -580,6 +647,68 @@ class _QpLayer(torch.autograd.Function):
         parts = tuple(k for i, k in enumerate(ctx.keys) if ctx.needs_input_grad[3 + i])
         out = ctx.engine.qp_grad(problem, sol, grads, parts)
         return (None, None, None) + tuple(out.get(k) for k in ctx.keys)
+
+
+class _TickLayer(torch.autograd.Function):
+    """forward: TsidEngine.problem_data -> qp_solve; backward: qp_grad (g, ce0) -> refs_grad (the tensors of `keys` are
+    the caller's reference tensors)."""
+
+    SOL = ("x", "status", "active", "lambda", "lambda_eq")
+    PROB = TsidEngine.PROBLEM_PARTS + TsidEngine.ACTUATION_PARTS + ("sizes",)
+
+    @staticmethod
+    def _feet(mask: Optional[torch.Tensor], n: int, device) -> Tuple[torch.Tensor, torch.Tensor]:
+        """[N,1] bools: LF in contact, RF in contact (no mask: double support)."""
+        if mask is None:
+            t = torch.ones((n, 1), dtype=torch.bool, device=device)
+            return t, t
+        m = mask.to(torch.int32).unsqueeze(1)
+        return (m & 1) != 0, (m & 2) != 0
+
+    @staticmethod
+    def forward(ctx, engine, q, v, mask, keys, *tensors):
+        refs = dict(zip(keys, tensors))
+        prob = engine.problem_data(q, v, mask, refs, parts=engine.PROBLEM_PARTS + engine.ACTUATION_PARTS)
+        sol = engine.qp_solve(prob)
+        n, nv = q.shape[0], engine.nv
+        x = sol["x"]
+        lf, rf = _TickLayer._feet(mask, n, x.device)
+        zero = torch.zeros((), dtype=x.dtype, device=x.device)
+        s0, s1 = x[:, nv:nv + 12], x[:, nv + 12:nv + 24]  # force slot 0: LF if in contact, else RF; slot 1: RF
+        f = torch.cat([torch.where(lf, s0, zero), torch.where(rf, torch.where(lf, s1, s0), zero)], dim=1)
+        ctx.engine, ctx.keys = engine, keys
+        ctx.mark_non_differentiable(sol["status"], sol["iters"])
+        ctx.save_for_backward(q, v, mask, *(sol[k] for k in _TickLayer.SOL), *(prob[k] for k in _TickLayer.PROB), *tensors)
+        return sol["tau"], x[:, :nv].contiguous(), f, sol["status"], sol["iters"]
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gtau, gdv, gf, _gstatus, _giters):
+        e, ns, npb = ctx.engine, len(_TickLayer.SOL), len(_TickLayer.PROB)
+        q, v, mask, *rest = ctx.saved_tensors
+        sol, prob, tensors = dict(zip(_TickLayer.SOL, rest[:ns])), dict(zip(_TickLayer.PROB, rest[ns:ns + npb])), rest[ns + npb:]
+        parts = tuple(k for i, k in enumerate(ctx.keys) if ctx.needs_input_grad[5 + i])
+        if not parts:
+            return (None,) * (5 + len(ctx.keys))
+        n, nv = q.shape[0], e.nv
+        grads = {}
+        if gdv is not None or gf is not None:
+            gx = torch.zeros_like(sol["x"])
+            if gdv is not None:
+                gx[:, :nv] = gdv
+            if gf is not None:
+                lf, rf = _TickLayer._feet(mask, n, gx.device)
+                zero = torch.zeros((), dtype=gx.dtype, device=gx.device)
+                gx[:, nv:nv + 12] = torch.where(lf, gf[:, :12], torch.where(rf, gf[:, 12:], zero))
+                gx[:, nv + 12:nv + 24] = torch.where(lf & rf, gf[:, 12:], zero)
+            grads["x"] = gx
+        if gtau is not None:
+            grads["tau"] = gtau.contiguous()
+        if not grads:
+            return (None,) * (5 + len(ctx.keys))
+        qg = e.qp_grad(prob, sol, grads, ("g", "ce0"))
+        out = e.refs_grad(q, v, mask, dict(zip(ctx.keys, tensors)), qg["g"], qg["ce0"], parts)
+        return (None,) * 5 + tuple(out.get(k) for k in ctx.keys)
 
 
 def fp64_peak_tflops(device: int = 0) -> float:
