@@ -335,6 +335,22 @@ int tsidb_refs_grad(tsidb_handle* h, int n_envs, int layout, const double* q, co
                     const tsidb_refs* refs, int n_max, int neq_max, const double* dg, const double* dce0,
                     const tsidb_refs_out* out, void* cuda_stream);
 
+/* ---- differentiating with respect to the state ----------------------------------------------------------------------
+ * tsidb_state_grad is the adjoint of all of tsidb_problem_data (H, g, CE, ce0, CI, ci0, TA, ta0) with respect to q and
+ * v: given `grad` = dL/d of each part (DEVICE arrays in the layout tsidb_qp_grad writes, with the caller's strides n_max,
+ * neq_max, nin_max >= the values of tsidb_problem_sizes; grad NULL or a NULL part counts as zero), it writes dL/dq [N][nq]
+ * and dL/dv [N][nv] (NULL = not written, not both), in the call's `layout` like q and v.  q, v, contact_mask and refs as
+ * in tsidb_problem_data.  grad->H is the gradient with respect to every entry of the full H the export writes, so the
+ * lower-triangular gradient of tsidb_qp_grad composes unchanged.  Only the entries inside an env's own (n, neq, nin)
+ * that depend on the state are read (INTEGRATION.md, "Differentiating with respect to the state", lists them); padding,
+ * appended variables and rows and the constant blocks may hold anything.  The gradient is with respect to the raw doubles
+ * of q (the free-flyer quaternion's 4 components through the tick's unnormalised quat -> R formula).  A joint-bound entry
+ * of ci0 that the export clips to +-1e10 has zero derivative.  No workspace of the handle is used, so the call may run
+ * on any stream.  Asynchronous on cuda_stream. */
+int tsidb_state_grad(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v, const uint8_t* contact_mask,
+                     const tsidb_refs* refs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* grad, double* dq,
+                     double* dv, void* cuda_stream);
+
 /* controller.integrate_dv(q, v, dv, dt) (ref:ctrl/WalkController.py:291-295,
  * ref:legacy/biped.py:236-240): v_mean = v + dt/2*dv; v += dt*dv;
  * q = pin.integrate(q, dt*v_mean).  In place on device arrays.                   */

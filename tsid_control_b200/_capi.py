@@ -281,6 +281,9 @@ def load_library() -> C.CDLL:
     lib.tsidb_qp_grad.restype = ip
     lib.tsidb_refs_grad.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, vp, vp, C.POINTER(TsidbRefsOut), vp]
     lib.tsidb_refs_grad.restype = ip
+    lib.tsidb_state_grad.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, ip, C.POINTER(TsidbProblemOut), vp,
+                                     vp, vp]
+    lib.tsidb_state_grad.restype = ip
     _LIB = lib
     return lib
 
@@ -298,5 +301,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
     "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve", "tsidb_qp_grad",
-    "tsidb_refs_grad",
+    "tsidb_refs_grad", "tsidb_state_grad",
 ]

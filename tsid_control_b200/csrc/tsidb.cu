@@ -207,6 +207,8 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
   TSIDB_ATTR(tsidb_dynamics_kernel<24>, smem, TSIDB_D_CTAS_PER_SM, "dynamics kernel", d_carve);
   TSIDB_ATTR(tsidb_refs_grad_kernel<26>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_refs_grad_kernel<24>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_state_grad_kernel<26>, TSIDB_S_SMEM, 1, "state gradient kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_state_grad_kernel<24>, TSIDB_S_SMEM, 1, "state gradient kernel", cudaSharedmemCarveoutMaxShared);
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<26, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_SMEM_DOUBLES(26) * sizeof(double)))));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<24, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_SMEM_DOUBLES(24) * sizeof(double)))));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<26, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_LOCAL_SMEM_DOUBLES(26) * sizeof(double)))));
@@ -919,6 +921,54 @@ extern "C" int tsidb_refs_grad(tsidb_handle* h, int n_envs, int layout, const do
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (h->dc.nv == 26) tsidb_refs_grad_kernel<26><<<blocks, 32 * TSIDB_R_CTA_WARPS, TSIDB_R_SMEM, st>>>(a, r);
   else tsidb_refs_grad_kernel<24><<<blocks, 32 * TSIDB_R_CTA_WARPS, TSIDB_R_SMEM, st>>>(a, r);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
+/* adjoint of the export in q and v: one launch that recomputes K1 and K2 per env and runs K1 in tangent arithmetic along
+ * every raw input direction, no workspace of the handle */
+extern "C" int tsidb_state_grad(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
+                                const uint8_t* contact_mask, const tsidb_refs* refs, int n_max, int neq_max, int nin_max,
+                                const tsidb_problem_out* grad, double* dq, double* dv, void* cuda_stream) {
+  if (!h || !q || !v) { g_err = "tsidb_state_grad: null argument"; return -1; }
+  if (!dq && !dv) { g_err = "tsidb_state_grad: dq and dv are both NULL"; return -1; }
+  if (n_envs <= 0 || n_envs > h->max_envs) { g_err = "tsidb_state_grad: n_envs must be in [1, max_envs]"; return -1; }
+  if (layout != 0 && layout != 1) { g_err = "tsidb_state_grad: layout must be 0 ([N][dof]) or 1 ([dof][N])"; return -1; }
+  int nx, neq, nin;
+  problem_maxima(h, &nx, &neq, &nin);
+  if (n_max < nx || neq_max < neq || nin_max < nin) {
+    g_err = "tsidb_state_grad: n_max, neq_max and nin_max must be at least tsidb_problem_sizes' maxima";
+    return -1;
+  }
+  tsidb_problem_out none;
+  memset(&none, 0, sizeof none);
+  const tsidb_problem_out& gr = grad ? *grad : none;
+  for (const void* p : {(const void*)q, (const void*)v, (const void*)gr.H, (const void*)gr.g, (const void*)gr.CE,
+                        (const void*)gr.ce0, (const void*)gr.CI, (const void*)gr.ci0, (const void*)gr.TA, (const void*)gr.ta0,
+                        (const void*)dq, (const void*)dv})
+    if (((uintptr_t)p & 7) != 0) { g_err = "tsidb_state_grad: fp64 arrays must be 8-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  TickArgs a;
+  memset(&a, 0, sizeof a);
+  a.n_envs = n_envs; a.layout = layout;
+  a.q = q; a.v = v; a.mask = contact_mask;
+  if (refs) {
+    a.r_com = refs->com; a.r_foot[0] = refs->foot_lf; a.r_foot[1] = refs->foot_rf;
+    a.r_contact[0] = refs->contact_lf; a.r_contact[1] = refs->contact_rf; a.r_posture = refs->posture;
+  }
+  a.slot = h->slot;
+  a.tables = h->tables;
+  StateGradArgs r;
+  memset(&r, 0, sizeof r);
+  r.n_max = n_max; r.neq_max = neq_max; r.nin_max = nin_max;
+  r.H = gr.H; r.g = gr.g; r.CE = gr.CE; r.ce0 = gr.ce0; r.CI = gr.CI; r.ci0 = gr.ci0; r.TA = gr.TA; r.ta0 = gr.ta0;
+  r.dq = dq; r.dv = dv;
+  int blocks = (n_envs + TSIDB_S_CTA_WARPS - 1) / TSIDB_S_CTA_WARPS;
+  if (blocks > h->sm_count) blocks = h->sm_count; /* persistent */
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  if (h->dc.nv == 26) tsidb_state_grad_kernel<26><<<blocks, 32 * TSIDB_S_CTA_WARPS, TSIDB_S_SMEM, st>>>(a, r);
+  else tsidb_state_grad_kernel<24><<<blocks, 32 * TSIDB_S_CTA_WARPS, TSIDB_S_SMEM, st>>>(a, r);
   CK(cudaGetLastError());
   h->launches += 1;
   return 0;

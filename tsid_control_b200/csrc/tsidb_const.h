@@ -158,6 +158,14 @@ struct RefsGradArgs {
   double* out[6];
 };
 
+/* arguments of the adjoint of the export in q and v (tsidb_state_grad): dL/d of the parts of tsidb_problem_out with the
+ * caller's strides (NULL = zero) and dL/dq [N][nq], dL/dv [N][nv] in the call's layout (NULL = not written) */
+struct StateGradArgs {
+  int32_t n_max, neq_max, nin_max, pad_;
+  const double *H, *g, *CE, *ce0, *CI, *ci0, *TA, *ta0;
+  double *dq, *dv;
+};
+
 struct TickArgs {
   int32_t n_envs, layout, pad_;
   const double* q;

@@ -43,7 +43,10 @@
 #define TSIDB_DEV __device__ __forceinline__
 #define TSIDB_HD __host__ __device__
 #define TSIDB_DEVNI __device__ __noinline__
+#define TSIDB_DEVM __device__ __forceinline__ /* member functions */
 __constant__ DevConst g_const[TSIDB_MAX_SLOTS];
+#else
+#define TSIDB_DEVM inline
 #endif
 
 #define FULL 0xffffffffu
@@ -68,36 +71,69 @@ __constant__ DevConst g_const[TSIDB_MAX_SLOTS];
 #define ST_ERROR 4
 
 /* ---------------------------------------------------------------- small helpers */
+/* Tangent (forward-mode) scalar: a value and its derivative along one input direction.  K1 and the 3-vector helpers are
+ * templates on the scalar type; instantiated with double they are the code the tick runs, with Dual they carry one
+ * direction of d/dq, d/dv through the same arithmetic (tsidb_state_grad, stage 2). */
+struct Dual {
+  double v, d;
+  TSIDB_HD Dual(double x = 0.0, double t = 0.0) : v(x), d(t) {}
+};
+TSIDB_DEV Dual operator+(const Dual& a, const Dual& b) { return Dual(a.v + b.v, a.d + b.d); }
+TSIDB_DEV Dual operator+(const Dual& a, double b) { return Dual(a.v + b, a.d); }
+TSIDB_DEV Dual operator+(double a, const Dual& b) { return Dual(a + b.v, b.d); }
+TSIDB_DEV Dual operator-(const Dual& a, const Dual& b) { return Dual(a.v - b.v, a.d - b.d); }
+TSIDB_DEV Dual operator-(const Dual& a, double b) { return Dual(a.v - b, a.d); }
+TSIDB_DEV Dual operator-(double a, const Dual& b) { return Dual(a - b.v, -b.d); }
+TSIDB_DEV Dual operator-(const Dual& a) { return Dual(-a.v, -a.d); }
+TSIDB_DEV Dual operator*(const Dual& a, const Dual& b) { return Dual(a.v * b.v, a.d * b.v + a.v * b.d); }
+TSIDB_DEV Dual operator*(const Dual& a, double b) { return Dual(a.v * b, a.d * b); }
+TSIDB_DEV Dual operator*(double a, const Dual& b) { return Dual(a * b.v, a * b.d); }
+TSIDB_DEV Dual operator/(const Dual& a, const Dual& b) { const double r = a.v / b.v; return Dual(r, (a.d - r * b.d) / b.v); }
+TSIDB_DEV Dual operator/(double a, const Dual& b) { const double r = a / b.v; return Dual(r, -r * b.d / b.v); }
+TSIDB_DEV Dual& operator+=(Dual& a, const Dual& b) { a.v += b.v; a.d += b.d; return a; }
+TSIDB_DEV void sincos(const Dual& x, Dual* s, Dual* c) {
+  double sv, cv;
+  sincos(x.v, &sv, &cv);
+  *s = Dual(sv, cv * x.d);
+  *c = Dual(cv, -sv * x.d);
+}
+
 TSIDB_DEV double shfl(double x, int src) { return __shfl_sync(FULL, x, src); }
+TSIDB_DEV Dual shfl(const Dual& x, int src) { return Dual(__shfl_sync(FULL, x.v, src), __shfl_sync(FULL, x.d, src)); }
 TSIDB_DEV double warp_sum(double x) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(FULL, x, o);
   return x;
 }
-TSIDB_DEV void cross3(const double* a, const double* b, double* o) {
-  double x = a[1] * b[2] - a[2] * b[1], y = a[2] * b[0] - a[0] * b[2], z = a[0] * b[1] - a[1] * b[0];
+template <class A, class B, class O>
+TSIDB_DEV void cross3(const A* a, const B* b, O* o) {
+  O x = a[1] * b[2] - a[2] * b[1], y = a[2] * b[0] - a[0] * b[2], z = a[0] * b[1] - a[1] * b[0];
   o[0] = x; o[1] = y; o[2] = z;
 }
-TSIDB_DEV double dot3(const double* a, const double* b) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; }
+template <class A, class B>
+TSIDB_DEV auto dot3(const A* a, const B* b) -> decltype(a[0] * b[0]) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; }
 /* o = R v (R row-major) */
-TSIDB_DEV void mv3(const double* R, const double* v, double* o) {
-  double x = R[0] * v[0] + R[1] * v[1] + R[2] * v[2];
-  double y = R[3] * v[0] + R[4] * v[1] + R[5] * v[2];
-  double z = R[6] * v[0] + R[7] * v[1] + R[8] * v[2];
+template <class A, class B, class O>
+TSIDB_DEV void mv3(const A* R, const B* v, O* o) {
+  O x = R[0] * v[0] + R[1] * v[1] + R[2] * v[2];
+  O y = R[3] * v[0] + R[4] * v[1] + R[5] * v[2];
+  O z = R[6] * v[0] + R[7] * v[1] + R[8] * v[2];
   o[0] = x; o[1] = y; o[2] = z;
 }
 /* o = R^T v */
-TSIDB_DEV void mtv3(const double* R, const double* v, double* o) {
-  double x = R[0] * v[0] + R[3] * v[1] + R[6] * v[2];
-  double y = R[1] * v[0] + R[4] * v[1] + R[7] * v[2];
-  double z = R[2] * v[0] + R[5] * v[1] + R[8] * v[2];
+template <class A, class B, class O>
+TSIDB_DEV void mtv3(const A* R, const B* v, O* o) {
+  O x = R[0] * v[0] + R[3] * v[1] + R[6] * v[2];
+  O y = R[1] * v[0] + R[4] * v[1] + R[7] * v[2];
+  O z = R[2] * v[0] + R[5] * v[1] + R[8] * v[2];
   o[0] = x; o[1] = y; o[2] = z;
 }
-TSIDB_DEV void mm3(const double* A, const double* B, double* C) {
+template <class A, class B, class O>
+TSIDB_DEV void mm3(const A* A_, const B* B_, O* C) {
 #pragma unroll
   for (int i = 0; i < 3; i++)
 #pragma unroll
-    for (int j = 0; j < 3; j++) C[3 * i + j] = A[3 * i] * B[j] + A[3 * i + 1] * B[3 + j] + A[3 * i + 2] * B[6 + j];
+    for (int j = 0; j < 3; j++) C[3 * i + j] = A_[3 * i] * B_[j] + A_[3 * i + 1] * B_[3 + j] + A_[3 * i + 2] * B_[6 + j];
 }
 /* element (env, dof) of a per-env array with ndof entries per env:
  * layout 0: [N][ndof] row-major (PyTorch-natural), layout 1: SoA [ndof][N] */
@@ -218,37 +254,77 @@ TSIDB_DEV void load_table(double* dst, const double* src, int count /* even */, 
   }
 }
 
-template <int NV>
-TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int lane) {
+/* Where K1 keeps a lane's 28 inertial accumulators: registers in the double instantiation (the tick's); in the tangent
+ * passes, whose values and derivatives do not fit the register file next to the rest of K1, a per-lane row of shared
+ * memory past the env workspace (odd stride of 29 Duals: lanes hit different banks). */
+template <class T> struct K1Acc;
+template <> struct K1Acc<double> {
+  double r[28];
+  TSIDB_DEVM K1Acc(double*, int) {}
+  TSIDB_DEVM double& operator[](int k) { return r[k]; }
+};
+template <> struct K1Acc<Dual> {
+  Dual* p;
+  TSIDB_DEVM K1Acc(Dual* sm, int lane) : p(sm + SM_oRef + 29 * lane) {}
+  TSIDB_DEVM Dual& operator[](int k) { return p[k]; }
+};
+
+/* lane 0's placement (the base's R0, p0) on every lane: shuffled into registers in the double instantiation; in the
+ * tangent passes lane 0 leaves it in shared memory after the accumulator rows, where the other lanes read it */
+#define K1_DUAL_ROOT (SM_oRef + 29 * 32) /* tangent workspace (Duals): env workspace, 32 accumulator rows, R0 and p0 */
+#define K1_DUAL_SIZE (K1_DUAL_ROOT + 12)
+template <class T, int N> struct K1Root;
+template <int N> struct K1Root<double, N> {
+  double r[N];
+  TSIDB_DEVM K1Root(const double* src, double*, int) {
+#pragma unroll
+    for (int k = 0; k < N; k++) r[k] = shfl(src[k], 0);
+  }
+  TSIDB_DEVM const double* ptr() const { return r; }
+  TSIDB_DEVM double operator[](int k) const { return r[k]; }
+};
+template <int N> struct K1Root<Dual, N> {
+  const Dual* p;
+  TSIDB_DEVM K1Root(const Dual* src, Dual* dst, int lane) : p(dst) {
+    if (lane == 0)
+      for (int k = 0; k < N; k++) dst[k] = src[k];
+    __syncwarp();
+  }
+  TSIDB_DEVM const Dual* ptr() const { return p; }
+  TSIDB_DEVM Dual operator[](int k) const { return p[k]; }
+};
+
+template <int NV, class T>
+TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, T* sm, int lane) {
   constexpr int nb = NV - 5, nv = NV; /* bodies = floating base + NV - 6 revolute joints */
   const bool act = lane < nb;
   const int b = act ? lane : 0;
   const int par = act && lane > 0 ? (int)mdl[b * MDL_STRIDE + MDL_oPAR] : 0;
-  const double* qs = sm + SM_oQV;
-  const double* vs = sm + SM_oQV + 32;
+  const T* qs = sm + SM_oQV;
+  const T* vs = sm + SM_oQV + 32;
 
-  double R[9], p[3], Vl[3], Va[3], Al[3] = {0, 0, 0}, Aa[3] = {0, 0, 0};
-  double Rl[9], pl[3], qd = 0.0;
+  T R[9], p[3], Vl[3], Va[3], Al[3] = {0, 0, 0}, Aa[3] = {0, 0, 0};
+  T Rl[9], pl[3], qd = 0.0;
   if (lane == 0) {
     /* free flyer: q = (p, quat xyzw); v = local (lin, ang) */
-    double x = qs[3], y = qs[4], z = qs[5], w = qs[6];
-    double tx = 2 * x, ty = 2 * y, tz = 2 * z;
-    double twx = tx * w, twy = ty * w, twz = tz * w, txx = tx * x, txy = ty * x, txz = tz * x;
-    double tyy = ty * y, tyz = tz * y, tzz = tz * z;
+    T x = qs[3], y = qs[4], z = qs[5], w = qs[6];
+    T tx = 2 * x, ty = 2 * y, tz = 2 * z;
+    T twx = tx * w, twy = ty * w, twz = tz * w, txx = tx * x, txy = ty * x, txz = tz * x;
+    T tyy = ty * y, tyz = tz * y, tzz = tz * z;
     R[0] = 1 - (tyy + tzz); R[1] = txy - twz; R[2] = txz + twy;
     R[3] = txy + twz; R[4] = 1 - (txx + tzz); R[5] = tyz - twx;
     R[6] = txz - twy; R[7] = tyz + twx; R[8] = 1 - (txx + tyy);
     p[0] = qs[0]; p[1] = qs[1]; p[2] = qs[2];
-    double vl[3] = {vs[0], vs[1], vs[2]}, wl[3] = {vs[3], vs[4], vs[5]};
+    T vl[3] = {vs[0], vs[1], vs[2]}, wl[3] = {vs[3], vs[4], vs[5]};
     mv3(R, wl, Va);
     mv3(R, vl, Vl);
-    double c[3];
+    T c[3];
     cross3(p, Va, c);
     Vl[0] += c[0]; Vl[1] += c[1]; Vl[2] += c[2];
   } else {
-    double ang = act ? qs[6 + b] : 0.0;
-    qd = act ? vs[5 + b] : 0.0;
-    double sa, ca;
+    T ang = act ? qs[6 + b] : T(0.0);
+    qd = act ? vs[5 + b] : T(0.0);
+    T sa, ca;
     sincos(ang, &sa, &ca);
     const double* jR = mdl + b * MDL_STRIDE + MDL_oJR;
 #pragma unroll
@@ -275,14 +351,14 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     int anc = par0;
     for (int rd = 0; rd < rounds; rd++) {
       const int src = anc < 0 ? 0 : anc;
-      double Rp[9], pp[3];
+      T Rp[9], pp[3];
 #pragma unroll
       for (int k = 0; k < 9; k++) Rp[k] = shfl(R[k], src);
 #pragma unroll
       for (int k = 0; k < 3; k++) pp[k] = shfl(p[k], src);
       const int anc2 = __shfl_sync(FULL, anc, src);
       if (anc >= 0) {
-        double Rn[9], pn[3];
+        T Rn[9], pn[3];
         mm3(Rp, R, Rn);
         mv3(Rp, p, pn);
 #pragma unroll
@@ -294,9 +370,9 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     }
   }
   /* own twist S qd of the body's joint (the base keeps its twist): V = sum over the path to the root */
-  double Sql[3] = {0, 0, 0}, Sqa[3] = {0, 0, 0};
+  T Sql[3] = {0, 0, 0}, Sqa[3] = {0, 0, 0};
   if (lane > 0) {
-    double a[3] = {R[2], R[5], R[8]}, sl[3];
+    T a[3] = {R[2], R[5], R[8]}, sl[3];
     cross3(p, a, sl);
 #pragma unroll
     for (int k = 0; k < 3; k++) { Sql[k] = sl[k] * qd; Sqa[k] = a[k] * qd; Vl[k] = Sql[k]; Va[k] = Sqa[k]; }
@@ -305,7 +381,7 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     int anc = par0;
     for (int rd = 0; rd < rounds; rd++) {
       const int src = anc < 0 ? 0 : anc;
-      double Vlp[3], Vap[3];
+      T Vlp[3], Vap[3];
 #pragma unroll
       for (int k = 0; k < 3; k++) { Vlp[k] = shfl(Vl[k], src); Vap[k] = shfl(Va[k], src); }
       const int anc2 = __shfl_sync(FULL, anc, src);
@@ -318,7 +394,7 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
   }
   /* own drift term V x (S qd) (motion cross product; zero for the base): A = sum over the path to the root */
   if (lane > 0) {
-    double c1[3], c2[3], c3[3];
+    T c1[3], c2[3], c3[3];
     cross3(Vl, Sqa, c1);
     cross3(Va, Sql, c2);
     cross3(Va, Sqa, c3);
@@ -329,7 +405,7 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     int anc = par0;
     for (int rd = 0; rd < rounds; rd++) {
       const int src = anc < 0 ? 0 : anc;
-      double Alp[3], Aap[3];
+      T Alp[3], Aap[3];
 #pragma unroll
       for (int k = 0; k < 3; k++) { Alp[k] = shfl(Al[k], src); Aap[k] = shfl(Aa[k], src); }
       const int anc2 = __shfl_sync(FULL, anc, src);
@@ -341,37 +417,38 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     }
   }
   /* motion subspace of the body's joint (revolute z): S = (p x a, a) */
-  double Sa_[3] = {R[2], R[5], R[8]}, Sl_[3];
+  T Sa_[3] = {R[2], R[5], R[8]}, Sl_[3];
   cross3(p, Sa_, Sl_);
 
   /* per-body inertial quantities, world coordinates, reference point = world origin */
-  double acc[28];
+  K1Acc<T> acc(sm, lane);
   {
     double m = act ? mdl[b * MDL_STRIDE + MDL_oMASS] : 0.0;
-    double cl[3] = {mdl[b * MDL_STRIDE + MDL_oCOM], mdl[b * MDL_STRIDE + MDL_oCOM + 1], mdl[b * MDL_STRIDE + MDL_oCOM + 2]}, cw[3];
+    double cl[3] = {mdl[b * MDL_STRIDE + MDL_oCOM], mdl[b * MDL_STRIDE + MDL_oCOM + 1], mdl[b * MDL_STRIDE + MDL_oCOM + 2]};
+    T cw[3];
     mv3(R, cl, cw);
     cw[0] += p[0]; cw[1] += p[1]; cw[2] += p[2];
-    double RI[9], Iw[9];
+    T RI[9], Iw[9];
     mm3(R, mdl + b * MDL_STRIDE + MDL_oI, RI);
     /* Iw = RI * R^T */
 #pragma unroll
     for (int i = 0; i < 3; i++)
 #pragma unroll
       for (int j = 0; j < 3; j++) Iw[3 * i + j] = RI[3 * i] * R[3 * j] + RI[3 * i + 1] * R[3 * j + 1] + RI[3 * i + 2] * R[3 * j + 2];
-    double h[3] = {m * cw[0], m * cw[1], m * cw[2]};
-    double c2 = dot3(cw, cw);
+    T h[3] = {m * cw[0], m * cw[1], m * cw[2]};
+    T c2 = dot3(cw, cw);
     /* inertia about the origin: Io = Iw + m (|c|^2 I - c c^T); xx xy xz yy yz zz */
-    double Io[6] = {Iw[0] + m * (c2 - cw[0] * cw[0]), Iw[1] - m * cw[0] * cw[1], Iw[2] - m * cw[0] * cw[2],
+    T Io[6] = {Iw[0] + m * (c2 - cw[0] * cw[0]), Iw[1] - m * cw[0] * cw[1], Iw[2] - m * cw[0] * cw[2],
                     Iw[4] + m * (c2 - cw[1] * cw[1]), Iw[5] - m * cw[1] * cw[2], Iw[8] + m * (c2 - cw[2] * cw[2])};
     /* momentum  P = m (Vl + Va x c),  L_o = Iw Va + c x P */
-    double t[3], P[3], Lo[3];
+    T t[3], P[3], Lo[3];
     cross3(Va, cw, t);
     P[0] = m * (Vl[0] + t[0]); P[1] = m * (Vl[1] + t[1]); P[2] = m * (Vl[2] + t[2]);
     mv3(Iw, Va, Lo);
     cross3(cw, P, t);
     Lo[0] += t[0]; Lo[1] += t[1]; Lo[2] += t[2];
     /* force at zero joint acceleration, no gravity: Y A + V x* (Y V) */
-    double fl[3], fa[3], u[3];
+    T fl[3], fa[3], u[3];
     cross3(Aa, cw, t);
     fl[0] = m * (Al[0] + t[0]); fl[1] = m * (Al[1] + t[1]); fl[2] = m * (Al[2] + t[2]);
     mv3(Iw, Aa, fa);
@@ -397,7 +474,7 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
    * a body's index is larger than its parent's (Pinocchio's depth-first order), so ONE sweep from the last
    * body to the first leaves every subtree sum in place; each lane only ever touches its own component, so
    * the sweep needs no synchronisation. */
-  double* sc = sm + SM_oH;
+  T* sc = sm + SM_oH;
   if (act) {
 #pragma unroll
     for (int k = 0; k < 28; k++) sc[b * 29 + k] = acc[k];
@@ -413,24 +490,21 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
   }
   __syncwarp();
   /* totals and the base placement, broadcast from lane 0 */
-  double mt = shfl(acc[0], 0);
-  double ht[3] = {shfl(acc[1], 0), shfl(acc[2], 0), shfl(acc[3], 0)};
-  double comw[3] = {ht[0] / mt, ht[1] / mt, ht[2] / mt};
-  double R0[9], p0[3];
-#pragma unroll
-  for (int k = 0; k < 9; k++) R0[k] = shfl(R[k], 0);
-#pragma unroll
-  for (int k = 0; k < 3; k++) p0[k] = shfl(p[k], 0);
-  double Y0[10];
+  T mt = shfl(acc[0], 0);
+  T ht[3] = {shfl(acc[1], 0), shfl(acc[2], 0), shfl(acc[3], 0)};
+  T comw[3] = {ht[0] / mt, ht[1] / mt, ht[2] / mt};
+  const K1Root<T, 9> R0(R, sm + K1_DUAL_ROOT, lane);
+  const K1Root<T, 3> p0(p, sm + K1_DUAL_ROOT + 9, lane);
+  T Y0[10];
 #pragma unroll
   for (int k = 0; k < 10; k++) Y0[k] = shfl(acc[k], 0);
 
-  double* Mm = sm + SM_oM;
-  double* nle = sm + SM_oNle;
-  double* Jcom = sm + SM_oJcom;
-  double* Ag = sm + SM_oAg;
-  double* JF = sm + SM_oJF;
-  double* fr = sm + SM_oFr;
+  T* Mm = sm + SM_oM;
+  T* nle = sm + SM_oNle;
+  T* Jcom = sm + SM_oJcom;
+  T* Ag = sm + SM_oAg;
+  T* JF = sm + SM_oJF;
+  T* fr = sm + SM_oFr;
 
   /* zero M and JF (different branches do not couple; non-support columns are zero) */
   for (int k = lane; k < nv * SM_LDM; k += 32) Mm[k] = 0.0;
@@ -446,15 +520,15 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
   const int kb = lane - nb; /* base dof of a base lane */
   if (isbase) {
     const int k = kb % 3;
-    const double rk[3] = {R0[k], R0[3 + k], R0[6 + k]};
+    const T rk[3] = {R0[k], R0[3 + k], R0[6 + k]};
     if (kb < 3) { Sl_[0] = rk[0]; Sl_[1] = rk[1]; Sl_[2] = rk[2]; Sa_[0] = Sa_[1] = Sa_[2] = 0.0; }
-    else { cross3(p0, rk, Sl_); Sa_[0] = rk[0]; Sa_[1] = rk[1]; Sa_[2] = rk[2]; }
+    else { cross3(p0.ptr(), rk, Sl_); Sa_[0] = rk[0]; Sa_[1] = rk[1]; Sa_[2] = rk[2]; }
   }
   /* F = Yc S for the lane's column; nle, Jcom, Ag columns; M entries along the ancestors */
-  double Fl[3], Fa[3];
+  T Fl[3], Fa[3];
   {
-    const double mc = isbase ? Y0[0] : acc[0];
-    double hc[3], Io[6], t[3];
+    const T mc = isbase ? Y0[0] : acc[0];
+    T hc[3], Io[6], t[3];
 #pragma unroll
     for (int k = 0; k < 3; k++) hc[k] = isbase ? Y0[1 + k] : acc[1 + k];
 #pragma unroll
@@ -476,11 +550,11 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
 #pragma unroll
       for (int r = 0; r < 3; r++) Ag[r * TSIDB_NVX + c] = Fa[r] - t[r];
       /* base rows: X0^T F */
-      double u[3], w[3];
-      mtv3(R0, Fl, u);
-      cross3(p0, Fl, t);
-      double d[3] = {Fa[0] - t[0], Fa[1] - t[1], Fa[2] - t[2]};
-      mtv3(R0, d, w);
+      T u[3], w[3];
+      mtv3(R0.ptr(), Fl, u);
+      cross3(p0.ptr(), Fl, t);
+      T d[3] = {Fa[0] - t[0], Fa[1] - t[1], Fa[2] - t[2]};
+      mtv3(R0.ptr(), d, w);
 #pragma unroll
       for (int r = 0; r < 3; r++) {
         Mm[r * SM_LDM + c] = u[r];
@@ -493,12 +567,12 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
   {
     int j = act && lane > 0 ? b : 0;
     for (int st = 0; st < C.maxdepth; st++) {
-      double sjl[3], sja[3];
+      T sjl[3], sja[3];
 #pragma unroll
       for (int k = 0; k < 3; k++) { sjl[k] = shfl(Sl_[k], j); sja[k] = shfl(Sa_[k], j); }
       const int pj = __shfl_sync(FULL, par, j); /* parent of body j: lane j holds it (no lane-indexed constant read) */
       if (j > 0) {
-        double val = dot3(sjl, Fl) + dot3(sja, Fa);
+        T val = dot3(sjl, Fl) + dot3(sja, Fa);
         Mm[(5 + j) * SM_LDM + 5 + b] = val;
         Mm[(5 + b) * SM_LDM + 5 + j] = val;
         j = pj;
@@ -507,7 +581,7 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
   }
   {
     /* base nle = X0^T Fc_root; CoM quantities; centroidal angular momentum and its drift */
-    double F0l[3], F0a[3], Pt[3], Lt[3], fal[3], faa[3];
+    T F0l[3], F0a[3], Pt[3], Lt[3], fal[3], faa[3];
 #pragma unroll
     for (int k = 0; k < 3; k++) {
       F0l[k] = shfl(acc[10 + k], 0); F0a[k] = shfl(acc[13 + k], 0);
@@ -515,17 +589,17 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
       fal[k] = shfl(acc[22 + k], 0); faa[k] = shfl(acc[25 + k], 0);
     }
     if (lane == 0) {
-      double u[3], w[3], t[3];
-      mtv3(R0, F0l, u);
-      cross3(p0, F0l, t);
-      double d[3] = {F0a[0] - t[0], F0a[1] - t[1], F0a[2] - t[2]};
-      mtv3(R0, d, w);
+      T u[3], w[3], t[3];
+      mtv3(R0.ptr(), F0l, u);
+      cross3(p0.ptr(), F0l, t);
+      T d[3] = {F0a[0] - t[0], F0a[1] - t[1], F0a[2] - t[2]};
+      mtv3(R0.ptr(), d, w);
 #pragma unroll
       for (int r = 0; r < 3; r++) { nle[r] = u[r]; nle[3 + r] = w[r]; }
       cross3(comw, Pt, t);
-      double t2[3];
+      T t2[3];
       cross3(comw, fal, t2);
-      const double imt0 = 1.0 / mt; /* one reciprocal for this lane's six divisions by the total mass */
+      const T imt0 = 1.0 / mt; /* one reciprocal for this lane's six divisions by the total mass */
 #pragma unroll
       for (int r = 0; r < 3; r++) {
         fr[FR_COM + r] = comw[r];
@@ -555,14 +629,14 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
       if (k2 < 6) {
         fm = 1; col = k2;
         const int k = k2 % 3;
-        const double rk[3] = {R0[k], R0[3 + k], R0[6 + k]};
+        const T rk[3] = {R0[k], R0[3 + k], R0[6 + k]};
         if (k2 < 3) { Sl_[0] = rk[0]; Sl_[1] = rk[1]; Sl_[2] = rk[2]; Sa_[0] = Sa_[1] = Sa_[2] = 0.0; }
-        else { cross3(p0, rk, Sl_); Sa_[0] = rk[0]; Sa_[1] = rk[1]; Sa_[2] = rk[2]; }
+        else { cross3(p0.ptr(), rk, Sl_); Sa_[0] = rk[0]; Sa_[1] = rk[1]; Sa_[2] = rk[2]; }
       }
     }
     const int fsel = fm < 0 ? 0 : fm;
     const int fb = C.foot_body[fsel];
-    double Rb[9], pb[3];
+    T Rb[9], pb[3];
 #pragma unroll
     for (int k = 0; k < 9; k++) Rb[k] = shfl(R[k], fb);
 #pragma unroll
@@ -572,15 +646,15 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     for (int k = 0; k < 9; k++) fRm[k] = C.fR[fsel][k]; /* lane-indexed constant reads: two addresses per instruction */
 #pragma unroll
     for (int k = 0; k < 3; k++) fpm[k] = C.fp[fsel][k];
-    double Rf[9], pf[3], t[3];
+    T Rf[9], pf[3], t[3];
     mm3(Rb, fRm, Rf);
     mv3(Rb, fpm, pf);
     pf[0] += pb[0]; pf[1] += pb[1]; pf[2] += pb[2];
     if (fm >= 0) {
-      double la[3], ll[3];
+      T la[3], ll[3];
       mtv3(Rf, Sa_, la);
       cross3(pf, Sa_, t);
-      double d[3] = {Sl_[0] - t[0], Sl_[1] - t[1], Sl_[2] - t[2]};
+      T d[3] = {Sl_[0] - t[0], Sl_[1] - t[1], Sl_[2] - t[2]};
       mtv3(Rf, d, ll);
 #pragma unroll
       for (int r = 0; r < 3; r++) {
@@ -590,14 +664,14 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, double* sm, int
     }
     if (isjoint && lane == fb) {
       const int f = fm;
-      double vl[3], va[3], al[3], aa[3];
+      T vl[3], va[3], al[3], aa[3];
       mtv3(Rf, Va, va);
       cross3(pf, Va, t);
-      double d[3] = {Vl[0] - t[0], Vl[1] - t[1], Vl[2] - t[2]};
+      T d[3] = {Vl[0] - t[0], Vl[1] - t[1], Vl[2] - t[2]};
       mtv3(Rf, d, vl);
       mtv3(Rf, Aa, aa);
       cross3(pf, Aa, t);
-      double e[3] = {Al[0] - t[0], Al[1] - t[1], Al[2] - t[2]};
+      T e[3] = {Al[0] - t[0], Al[1] - t[1], Al[2] - t[2]};
       mtv3(Rf, e, al);
       cross3(va, vl, t);
 #pragma unroll
@@ -2661,6 +2735,287 @@ TSIDB_DEV void refs_grad_env(const DevConst& C, const double* mdl, double* sm, c
   refs_adjoint_env<NV>(C, mdl, sm, a, r, env, lane, mask);
 }
 
+/* ================================================================= adjoint of the export in q and v (tsidb_state_grad) */
+/* Stage 1 of one env, after K1 and K2 ran on this env in `sm`: the cotangent of the export (the parts of r, NULL = zero)
+ * pulled back onto K1's outputs.  It lands in `cb` at K1's own offsets (M, JF, Jcom, Ag, nle, frames; zero where the
+ * export does not depend on them), and the terms that depend on q and v directly (posture task, joint-bound rows) land in
+ * cb[SM_oQV + k] (q) and cb[SM_oQV + 32 + k] (v).  Of an env with sizes (n, neq, nin) it reads only what depends on
+ * the state:
+ *   H    rows and columns 0..nv (the dv block; dL/dH_ij + dL/dH_ji multiplies dH_ij); the force block is constant
+ *   g    0..nv
+ *   CE   rows 0..6, columns 0..n ([M_u | -Jc_u^T]); rows 6..neq, columns 0..nv (JF of the feet in contact)
+ *   ce0  0..neq (h_u, -b_mot)
+ *   CI   the actuation rows (torque bounds), columns 0..n; the force and joint-bound rows are constant
+ *   ci0  the actuation rows (h_a) and the joint-bound rows of the joints (v_j); the force rows and base rows are constant
+ *   TA   rows 0..na, columns 0..n;  ta0  0..na
+ * A joint-bound entry of ci0 is clipped to +-1e10 by the export; where the clip binds its derivative is zero. */
+template <int NV>
+TSIDB_DEV void state_adjoint_env(const DevConst& C, const double* mdl, double* sm, double* cb, const StateGradArgs& r,
+                                 int env, int lane, int mask) {
+  constexpr int nv = NV, na = NV - 6;
+  const double BIG = 1e10; /* the export's clip of the joint-bound rows */
+  const int nc = (mask & 1) + ((mask >> 1) & 1);
+  const int neq = 6 + 6 * nc;
+  const int f0 = (mask & 1) ? 0 : 1; /* foot of force slot 0; slot 1 is RF */
+  const int oAct = 34 * nc, oJb = 34 * nc + (C.use_tb ? 2 * na : 0); /* first actuation and joint-bound row of CI */
+  const double* JF = sm + SM_oJF;
+  const double* Jcom = sm + SM_oJcom;
+  const double* Ag = sm + SM_oAg;
+  const double* bv = sm + SM_oBv;
+  const double* fr = sm + SM_oFr;
+  const double* rf = sm + SM_oRef;
+  const double* vs = sm + SM_oQV + 32;
+  const size_t nx = (size_t)r.n_max;
+  const double* H = r.H ? r.H + (size_t)env * nx * nx : nullptr;
+  const double* g = r.g ? r.g + (size_t)env * nx : nullptr;
+  const double* CE = r.CE ? r.CE + (size_t)env * r.neq_max * nx : nullptr;
+  const double* ce0 = r.ce0 ? r.ce0 + (size_t)env * r.neq_max : nullptr;
+  const double* CI = (r.CI && C.use_tb) ? r.CI + (size_t)env * r.nin_max * nx : nullptr;
+  const double* ci0 = r.ci0 ? r.ci0 + (size_t)env * r.nin_max : nullptr;
+  const double* TA = r.TA ? r.TA + (size_t)env * na * nx : nullptr;
+  const double* ta0 = r.ta0 ? r.ta0 + (size_t)env * na : nullptr;
+  for (int k = lane; k < SM_oRef; k += 32) cb[k] = 0.0;
+  double* gb = cb + SM_oGv; /* dL/dg_dv */
+  double* bb = cb + SM_oBv; /* dL/d of the task right-hand sides, at the BV_* offsets */
+  __syncwarp();
+  if (lane < nv) gb[lane] = g ? g[lane] : 0.0;
+  __syncwarp();
+  /* g_dv = -(w_foot JF^T b_foot + w_com Jcom^T b_com + w_am Ag^T b_am + w_post S^T b_post), ce0[6 + 6s + k] = -b_mot[f_s][k] */
+  if (lane < 18) {
+    const double* A = lane < 12 ? JF + lane * TSIDB_NVX : (lane < 15 ? Jcom + (lane - 12) * TSIDB_NVX : Ag + (lane - 15) * TSIDB_NVX);
+    double acc = 0.0;
+#pragma unroll 2
+    for (int j = 0; j < nv; j++) acc += A[j] * gb[j];
+    if (lane < 12) bb[BV_FOOT + lane] = -C.w_foot * acc;
+    else if (lane < 15) bb[BV_COM + lane - 12] = -C.w_com * acc;
+    else bb[BV_AM + lane - 15] = C.use_am ? -C.w_am * acc : 0.0;
+  }
+  if (lane < 12) {
+    const int f = lane / 6;
+    bb[BV_MOT + lane] = (ce0 && ((mask >> f) & 1)) ? -ce0[6 + 6 * (f == f0 ? 0 : 1) + lane % 6] : 0.0;
+  }
+  if (lane < na) {
+    bb[BV_POST + lane] = -C.w_post * gb[6 + lane];
+    /* posture task: b_post = -Kp (q_j - q_ref) - Kd v_j */
+    cb[SM_oQV + 7 + lane] = -mdl[MDL_oPOST + lane] * bb[BV_POST + lane];
+    cb[SM_oQV + 32 + 6 + lane] = -mdl[MDL_oPOST + 23 + lane] * bb[BV_POST + lane];
+  }
+  __syncwarp();
+  /* joint-bound rows: ub = min((v_max - v_j) / dt, 1e10), lb = max((v_min - v_j) / dt, -1e10), ci0 = (-lb, ub) */
+  if (ci0 && C.use_jb && lane >= 6 && lane < nv) {
+    const double vj = vs[lane];
+    const double hi = (C.v_max[lane - 6] - vj) / C.jb_dt, lo = (C.v_min[lane - 6] - vj) / C.jb_dt;
+    double d = 0.0;
+    if (lo > -BIG) d += ci0[oJb + lane] / C.jb_dt;
+    if (hi < BIG) d -= ci0[oJb + nv + lane] / C.jb_dt;
+    cb[SM_oQV + 32 + lane] += d;
+  }
+  /* column j of M, JF, Jcom, Ag and entry j of nle, one lane each */
+  if (lane < nv) {
+    const int j = lane;
+    double jfb[12], jcb[3], agb[3];
+#pragma unroll
+    for (int q = 0; q < 12; q++) jfb[q] = 0.0;
+#pragma unroll
+    for (int q = 0; q < 3; q++) { jcb[q] = 0.0; agb[q] = 0.0; }
+    /* H_dv = w_foot JF^T JF + w_com Jcom^T Jcom (+ w_am Ag^T Ag) + constant diagonal: dL/dA = w A (Hb + Hb^T) */
+    if (H) {
+#pragma unroll 1
+      for (int m = 0; m < nv; m++) {
+        const double s = H[j * nx + m] + H[m * nx + j];
+#pragma unroll
+        for (int q = 0; q < 12; q++) jfb[q] += s * JF[q * TSIDB_NVX + m];
+#pragma unroll
+        for (int q = 0; q < 3; q++) jcb[q] += s * Jcom[q * TSIDB_NVX + m];
+        if (C.use_am) {
+#pragma unroll
+          for (int q = 0; q < 3; q++) agb[q] += s * Ag[q * TSIDB_NVX + m];
+        }
+      }
+    }
+    const double gj = gb[j];
+#pragma unroll
+    for (int q = 0; q < 12; q++) jfb[q] = C.w_foot * (jfb[q] - gj * bv[BV_FOOT + q]);
+#pragma unroll
+    for (int q = 0; q < 3; q++) {
+      jcb[q] = C.w_com * (jcb[q] - gj * bv[BV_COM + q]);
+      agb[q] = C.use_am ? C.w_am * (agb[q] - gj * bv[BV_AM + q]) : 0.0;
+    }
+#pragma unroll
+    for (int q = 0; q < 12; q++) cb[SM_oJF + q * TSIDB_NVX + j] = jfb[q];
+#pragma unroll
+    for (int q = 0; q < 3; q++) { cb[SM_oJcom + q * TSIDB_NVX + j] = jcb[q]; cb[SM_oAg + q * TSIDB_NVX + j] = agb[q]; }
+    /* CE: rows 0..6 are [M_u | -Jc_u^T], rows 6..neq the JF rows of the feet in contact */
+    if (CE) {
+      for (int q = 0; q < 6; q++) cb[SM_oM + q * SM_LDM + j] = CE[q * nx + j];
+      for (int q = 6; q < neq; q++) cb[SM_oJF + (((q < 12) ? f0 : 1) * 6 + (q - 6) % 6) * TSIDB_NVX + j] += CE[q * nx + j];
+    }
+    /* CI actuation rows ([M_a | -Jc_a^T], lower side +, upper side -) and TA ([M_a | -Jc_a^T]) */
+    for (int q = 6; q < nv; q++) {
+      double x = 0.0;
+      if (CI) x += CI[(oAct + q - 6) * nx + j] - CI[(oAct + na + q - 6) * nx + j];
+      if (TA) x += TA[(q - 6) * nx + j];
+      cb[SM_oM + q * SM_LDM + j] = x;
+    }
+    /* Jc = T^T JF_f of force slot s: row j of Jc enters CE row j (j < 6), the actuation rows and TA row j - 6 (j >= 6) */
+    for (int s = 0; s < nc; s++) {
+      const int f = s == 0 ? f0 : 1;
+      double jc[12];
+#pragma unroll
+      for (int k = 0; k < 12; k++) {
+        const int col = nv + 12 * s + k;
+        double x = 0.0;
+        if (j < 6) {
+          if (CE) x -= CE[j * nx + col];
+        } else {
+          if (CI) x += CI[(oAct + na + j - 6) * nx + col] - CI[(oAct + j - 6) * nx + col];
+          if (TA) x -= TA[(j - 6) * nx + col];
+        }
+        jc[k] = x;
+      }
+#pragma unroll
+      for (int m = 0; m < 6; m++) {
+        double acc = 0.0;
+#pragma unroll
+        for (int k = 0; k < 12; k++) acc += C.T[m][k] * jc[k];
+        cb[SM_oJF + (f * 6 + m) * TSIDB_NVX + j] += acc;
+      }
+    }
+    /* ce0 rows 0..6 are h_u; ci0's actuation rows h_a - tau_min and tau_max - h_a; ta0 = h_a */
+    double nb = 0.0;
+    if (j < 6) {
+      if (ce0) nb = ce0[j];
+    } else {
+      if (ci0 && C.use_tb) nb += ci0[oAct + j - 6] - ci0[oAct + na + j - 6];
+      if (ta0) nb += ta0[j - 6];
+    }
+    cb[SM_oNle + j] = nb;
+  }
+  /* the four SE3 laws (contact LF, contact RF, foot LF, foot RF): b = Kp log6(Rf^T R_ref, Rf^T (p_ref - p_f))
+   * + Kd (Rf^T v_ref - v_F) + Rf^T a_ref - a_F, each lane's frame cotangent to its own scratch, summed per foot below */
+  double* wk = sm + SM_oM + 64 * lane; /* K2's Hessian block, dead: E 9, ep 3, dL/dE 9, dL/dep 3, then p 3, R 9, vF 6, aF 6 */
+  if (lane < 4) {
+    const int f = lane & 1;
+    const bool is_contact = lane < 2;
+    double* E = wk;
+    double* ep = wk + 9;
+    double* Eb = wk + 12;
+    double* epb = wk + 21;
+    double* o = wk + 24;
+#pragma unroll
+    for (int k = 0; k < 36; k++) wk[12 + k] = 0.0; /* Eb, epb, o */
+    if (!is_contact || ((mask >> f) & 1)) {
+      double b6[6], kp[6], kd[6], Rr[9], dp[3];
+      const double* gains = C.kp_contact + (is_contact ? 0 : 12);
+#pragma unroll
+      for (int k = 0; k < 6; k++) {
+        b6[k] = bb[(is_contact ? BV_MOT : BV_FOOT) + 6 * f + k];
+        kp[k] = gains[k];
+        kd[k] = gains[6 + k];
+      }
+      const double* ref = is_contact ? rf + RF_CONTACT + 12 * f : rf + RF_FOOT + 24 * f;
+      const double* pf = fr + FR_OMF + f * 12;
+      const double* Rf = pf + 3;
+#pragma unroll
+      for (int c = 0; c < 3; c++)
+#pragma unroll
+        for (int q = 0; q < 3; q++) Rr[3 * q + c] = ref[3 + 3 * c + q];
+      dp[0] = ref[0] - pf[0]; dp[1] = ref[1] - pf[1]; dp[2] = ref[2] - pf[2];
+#pragma unroll
+      for (int i = 0; i < 3; i++)
+#pragma unroll
+        for (int q = 0; q < 3; q++) E[3 * i + q] = Rf[i] * Rr[q] + Rf[3 + i] * Rr[3 + q] + Rf[6 + i] * Rr[6 + q];
+      mtv3(Rf, dp, ep);
+      {
+        double ol[3], oa[3];
+#pragma unroll
+        for (int k = 0; k < 3; k++) { ol[k] = kp[k] * b6[k]; oa[k] = kp[3 + k] * b6[3 + k]; }
+        log6_adj(E, ep, ol, oa, Eb, epb);
+      }
+      /* E = Rf^T R_ref, ep = Rf^T dp, dp = p_ref - p_f; foot task: v = Rf^T v_ref, a = Rf^T a_ref */
+#pragma unroll
+      for (int q = 0; q < 3; q++)
+#pragma unroll
+        for (int i = 0; i < 3; i++) {
+          double x = Rr[3 * q] * Eb[3 * i] + Rr[3 * q + 1] * Eb[3 * i + 1] + Rr[3 * q + 2] * Eb[3 * i + 2] + dp[q] * epb[i];
+          if (!is_contact)
+            x += ref[12 + q] * kd[i] * b6[i] + ref[15 + q] * kd[3 + i] * b6[3 + i] + ref[18 + q] * b6[i] + ref[21 + q] * b6[3 + i];
+          o[3 + 3 * q + i] = x;
+        }
+      double t3[3];
+      mv3(Rf, epb, t3);
+      o[0] = -t3[0]; o[1] = -t3[1]; o[2] = -t3[2];
+#pragma unroll
+      for (int k = 0; k < 6; k++) { o[12 + k] = -kd[k] * b6[k]; o[18 + k] = -b6[k]; }
+    }
+  } else if (lane < 7) {
+    const int q = lane - 4; /* CoM task: b = -Kp (c - c_ref) - Kd (vc - vc_ref) + ac_ref - drift */
+    cb[SM_oFr + FR_COM + q] = -C.kp_com[q] * bb[BV_COM + q];
+    cb[SM_oFr + FR_COM + 3 + q] = -C.kd_com[q] * bb[BV_COM + q];
+    cb[SM_oFr + FR_COM + 6 + q] = -bb[BV_COM + q];
+  } else if (lane < 10) {
+    const int q = lane - 7; /* legacy AM task: b = -Kp L - drift */
+    cb[SM_oFr + FR_L + q] = -C.kp_am[q] * bb[BV_AM + q];
+    cb[SM_oFr + FR_L + 3 + q] = -bb[BV_AM + q];
+  }
+  __syncwarp();
+  const double* w0 = sm + SM_oM + 24;
+  if (lane < 24) { /* placements: foot f = lane / 12, contact lane f and foot-task lane 2 + f */
+    const int f = lane / 12;
+    cb[SM_oFr + FR_OMF + lane] = w0[64 * f + lane % 12] + w0[64 * (2 + f) + lane % 12];
+  }
+  if (lane < 12) { /* velocities and drifts */
+    const int f = lane / 6;
+    cb[SM_oFr + FR_VF + lane] = w0[64 * f + 12 + lane % 6] + w0[64 * (2 + f) + 12 + lane % 6];
+    cb[SM_oFr + FR_AF + lane] = w0[64 * f + 18 + lane % 6] + w0[64 * (2 + f) + 18 + lane % 6];
+  }
+  __syncwarp();
+}
+
+/* one env of tsidb_state_grad.  q, v and the references staged and K1 + K2 run as the dynamics kernel runs them, stage 1
+ * (state_adjoint_env), then stage 2: K1 again in tangent arithmetic once per raw input direction (nq components of q, nv
+ * of v), each pass contracted with stage 1's cotangents.  The tangent passes overwrite `sm` (Dual, 2 SM_oRef doubles);
+ * `cb` (SM_oRef doubles) holds the cotangents and the result. */
+template <int NV>
+TSIDB_DEV void state_grad_env(const DevConst& C, const double* mdl, double* sm, double* cb, const TickArgs& a,
+                              const StateGradArgs& r, int env, int lane) {
+  constexpr int nv = NV, na = NV - 6, nq = NV + 1;
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  const double qv = lane < nq ? ldin(a.q, a, env, lane, nq) : 0.0;
+  const double vv = lane < nv ? ldin(a.v, a, env, lane, nv) : 0.0;
+  if (lane < nq) sm[SM_oQV + lane] = qv;
+  if (lane < nv) sm[SM_oQV + 32 + lane] = vv;
+  stage_refs(C, mdl, sm, a, env, lane, na);
+  __syncwarp();
+  k1_dynamics<NV>(C, mdl, sm, lane);
+  stage_refs_wait();
+  const int mask = a.mask ? (a.mask[env] & 3) : 3;
+  const int nc = (mask & 1) + ((mask >> 1) & 1);
+  k2_assemble<NV>(C, mdl, sm, a, env, lane, mask, 6 + 6 * nc, nv + 12 * nc);
+  state_adjoint_env<NV>(C, mdl, sm, cb, r, env, lane, mask);
+  Dual* ds = reinterpret_cast<Dual*>(sm);
+#pragma unroll 1
+  for (int dir = 0; dir < nq + nv; dir++) {
+    __syncwarp();
+    if (lane < nq) ds[SM_oQV + lane] = Dual(qv, dir == lane ? 1.0 : 0.0);
+    if (lane < nv) ds[SM_oQV + 32 + lane] = Dual(vv, dir == nq + lane ? 1.0 : 0.0);
+    __syncwarp();
+    k1_dynamics<NV>(C, mdl, ds, lane);
+    /* the entries K1 writes: M (nv rows), JF, the nv columns of Jcom and Ag, nle, the frames */
+    double acc = 0.0;
+    for (int k = lane; k < nv * SM_LDM; k += 32) acc += cb[SM_oM + k] * ds[SM_oM + k].d;
+    for (int k = lane; k < 12 * TSIDB_NVX; k += 32) acc += cb[SM_oJF + k] * ds[SM_oJF + k].d;
+    for (int k = lane; k < 6 * TSIDB_NVX + nv; k += 32)
+      if (k >= 6 * TSIDB_NVX || k % TSIDB_NVX < nv) acc += cb[SM_oJcom + k] * ds[SM_oJcom + k].d;
+    for (int k = lane; k < FR_L + 6; k += 32) acc += cb[SM_oFr + k] * ds[SM_oFr + k].d;
+    acc = warp_sum(acc);
+    if (lane == 0) cb[SM_oQV + (dir < nq ? dir : 32 + dir - nq)] += acc;
+  }
+  __syncwarp();
+  if (r.dq && lane < nq) r.dq[eidx(a, env, lane, nq)] = cb[SM_oQV + lane];
+  if (r.dv && lane < nv) r.dv[eidx(a, env, lane, nv)] = cb[SM_oQV + 32 + lane];
+}
+
 /* ================================================================= generic QP solve of one env (tsidb_qp_solve) */
 /* eiquadprog-fast solve_quadprog on a caller-supplied problem, min 1/2 x'Hx + g'x s.t. CE x + ce0 = 0, CI x + ci0 >= 0,
  * step for step as the oracle's eq_solve states it: LLT of H, J = L^-T, x0 = -H^-1 g, the equalities added one by one,
@@ -3620,6 +3975,28 @@ tsidb_refs_grad_kernel(const TickArgs a, const RefsGradArgs r) {
   __syncthreads();
   for (int env = blockIdx.x * TSIDB_R_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_R_CTA_WARPS)
     refs_grad_env<NV>(C, mdl, sm, a, r, env, lane);
+}
+
+/* Adjoint of the export in q and v (tsidb_state_grad): one warp per env on a persistent grid, the CTA's warps sharing the
+ * staged model table.  Per warp: the tangent workspace (K1_DUAL_SIZE Duals), whose start the double K1 and K2 use as
+ * the dynamics kernel's env workspace, and the cotangents (SM_oRef doubles): 48 KB.  4 warps and one CTA per SM leave
+ * 255 registers per thread, which the tangent K1 needs to stay within the dynamics kernel's spills. */
+#define TSIDB_S_CTA_WARPS 4
+#define TSIDB_S_PER_WARP (2 * K1_DUAL_SIZE + SM_oRef)
+#define TSIDB_S_SMEM (((size_t)TSIDB_S_CTA_WARPS * TSIDB_S_PER_WARP + MDL_SIZE) * sizeof(double))
+static_assert(2 * SM_oRef >= SM_PER_ENV && (TSIDB_S_PER_WARP % 2) == 0, "the env workspace fits the Dual view, 16-byte aligned");
+template <int NV>
+__global__ void __launch_bounds__(32 * TSIDB_S_CTA_WARPS, 1)
+tsidb_state_grad_kernel(const TickArgs a, const StateGradArgs r) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  double* sm = smem + wid * TSIDB_S_PER_WARP;
+  const DevConst& C = g_const[a.slot];
+  double* mdl = smem + TSIDB_S_CTA_WARPS * TSIDB_S_PER_WARP;
+  load_table(mdl, a.tables + TBL_oMDL, MDL_SIZE, threadIdx.x, blockDim.x);
+  __syncthreads();
+  for (int env = blockIdx.x * TSIDB_S_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_S_CTA_WARPS)
+    state_grad_env<NV>(C, mdl, sm, sm + 2 * K1_DUAL_SIZE, a, r, env, lane);
 }
 
 /* ---- Small batches: the whole tick of one env in ONE launch ----

@@ -576,16 +576,59 @@ class TsidEngine:
                                        C.byref(ro), self._stream()), "tsidb_refs_grad")
         return out
 
+    def state_grad(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                   refs: Optional[Dict[str, torch.Tensor]] = None, grads: Optional[Dict[str, torch.Tensor]] = None,
+                   parts: Tuple[str, ...] = ("q", "v")) -> Dict[str, torch.Tensor]:
+        """Adjoint of all of :meth:`problem_data` with respect to the state (tsidb_state_grad): from `grads`, dL/d of any
+        of the export's parts H, g, CE, ce0, CI, ci0, TA, ta0 in the layout problem_data returns (strides from the shapes,
+        at least problem_sizes(); an absent part counts as zero; a "status" entry, as :meth:`qp_grad` returns it, is
+        ignored), new CUDA tensors {"q": [N,nq], "v": [N,nv]} for `parts`.  q, v, contact_mask and refs as in
+        :meth:`problem_data`.  The gradient is with respect to the raw doubles of q (the free-flyer quaternion's four
+        components, unnormalised); only the state-dependent entries inside each env's sizes are read, so padding and
+        constant blocks may hold anything.  See INTEGRATION.md, "Differentiating with respect to the state"."""
+        r = self._state_args("state_grad", q, v, contact_mask, refs)
+        n = q.shape[0]
+        parts = tuple(parts)
+        if not parts or set(parts) - {"q", "v"}:
+            raise ValueError(f"state_grad: parts must name q and/or v, got {parts}")
+        floats = self.PROBLEM_PARTS + self.ACTUATION_PARTS
+        grads = {k: t for k, t in (grads or {}).items() if k != "status"}
+        if set(grads) - set(floats):
+            raise ValueError(f"state_grad: unknown parts {sorted(set(grads) - set(floats))}; choose from {floats}")
+        nx0, neq0, nin0 = self.problem_sizes()
+
+        def stride(where, default):  # the first given part that has the axis; the shape check below catches the rest
+            return next((grads[k].shape[d] for k, d in where if k in grads and grads[k].dim() > d), default)
+
+        nx = stride((("H", 2), ("g", 1), ("CE", 2), ("CI", 2), ("TA", 2)), nx0)
+        neq = stride((("ce0", 1), ("CE", 1)), neq0)
+        nin = stride((("ci0", 1), ("CI", 1)), nin0)
+        if nx < nx0 or neq < neq0 or nin < nin0:
+            raise TypeError(f"state_grad: strides ({nx}, {neq}, {nin}) below problem_sizes() ({nx0}, {neq0}, {nin0})")
+        shapes = {"H": (n, nx, nx), "g": (n, nx), "CE": (n, neq, nx), "ce0": (n, neq), "CI": (n, nin, nx), "ci0": (n, nin),
+                  "TA": (n, self.na, nx), "ta0": (n, self.na)}
+        self._qp_tensors("state_grad", grads, shapes)
+        out = {k: torch.empty((n, self.nq if k == "q" else self.nv), dtype=torch.float64, device=self.device) for k in parts}
+        po = _capi.TsidbProblemOut(**{k: t.data_ptr() for k, t in grads.items()})
+        check(self.lib.tsidb_state_grad(self.h, n, 0, q.data_ptr(), v.data_ptr(),
+                                        contact_mask.data_ptr() if contact_mask is not None else None, C.byref(r),
+                                        nx, neq, nin, C.byref(po), out["q"].data_ptr() if "q" in out else None,
+                                        out["v"].data_ptr() if "v" in out else None, self._stream()), "tsidb_state_grad")
+        return out
+
     def tick_layer(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
                    refs: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
-        """A tick as a differentiable function of its references: {tau [N,na], dv [N,nv], f [N,24], status, iters [N]
-        int32}, with tau, dv and f carrying a grad_fn for every tensor of `refs` that requires grad (first order only).
+        """A tick as a differentiable function of its state and references: {tau [N,na], dv [N,nv], f [N,24], status,
+        iters [N] int32}, with tau, dv and f carrying a grad_fn for q, v and every tensor of `refs` that requires grad
+        (first order only).
         f holds the corner forces in the tick's fixed slots, LF 0..11 and RF 12..23, zero for a foot not in contact.
         The forward pass is :meth:`problem_data` (with TA, ta0) followed by :meth:`qp_solve`, not the fast tick: the
         backward pass (:meth:`qp_grad` for g and ce0, then :meth:`refs_grad`) must differentiate the working set its own
         forward pass found, and the two solves can end in different working sets at degenerate contact-corner ties.  That
         costs time: about 74 ms for the forward pass at 65536 walking envs against 3 ms for a tick.  An env whose solve or
-        adjoint status is not 0 contributes zero.  q, v and contact_mask get no gradient."""
+        adjoint status is not 0 contributes zero.  When q or v requires grad, the backward pass asks :meth:`qp_grad` for
+        every part and adds :meth:`state_grad` (q in its raw doubles, the quaternion unnormalised); otherwise it makes
+        the same calls as for references alone.  contact_mask gets no gradient."""
         self._state_args("tick_layer", q, v, contact_mask, refs)
         keys = tuple(k for k in REF_KEYS if refs and refs.get(k) is not None)
         outs = _TickLayer.apply(self, q, v, contact_mask, keys, *(refs[k] for k in keys))
@@ -650,8 +693,8 @@ class _QpLayer(torch.autograd.Function):
 
 
 class _TickLayer(torch.autograd.Function):
-    """forward: TsidEngine.problem_data -> qp_solve; backward: qp_grad (g, ce0) -> refs_grad (the tensors of `keys` are
-    the caller's reference tensors)."""
+    """forward: TsidEngine.problem_data -> qp_solve; backward: qp_grad (g, ce0; every part when q or v needs a gradient)
+    -> refs_grad and state_grad (the tensors of `keys` are the caller's reference tensors)."""
 
     SOL = ("x", "status", "active", "lambda", "lambda_eq")
     PROB = TsidEngine.PROBLEM_PARTS + TsidEngine.ACTUATION_PARTS + ("sizes",)
@@ -688,7 +731,8 @@ class _TickLayer(torch.autograd.Function):
         q, v, mask, *rest = ctx.saved_tensors
         sol, prob, tensors = dict(zip(_TickLayer.SOL, rest[:ns])), dict(zip(_TickLayer.PROB, rest[ns:ns + npb])), rest[ns + npb:]
         parts = tuple(k for i, k in enumerate(ctx.keys) if ctx.needs_input_grad[5 + i])
-        if not parts:
+        sparts = tuple(k for k, i in (("q", 1), ("v", 2)) if ctx.needs_input_grad[i])
+        if not parts and not sparts:
             return (None,) * (5 + len(ctx.keys))
         n, nv = q.shape[0], e.nv
         grads = {}
@@ -706,9 +750,11 @@ class _TickLayer(torch.autograd.Function):
             grads["tau"] = gtau.contiguous()
         if not grads:
             return (None,) * (5 + len(ctx.keys))
-        qg = e.qp_grad(prob, sol, grads, ("g", "ce0"))
-        out = e.refs_grad(q, v, mask, dict(zip(ctx.keys, tensors)), qg["g"], qg["ce0"], parts)
-        return (None,) * 5 + tuple(out.get(k) for k in ctx.keys)
+        refs = dict(zip(ctx.keys, tensors))
+        qg = e.qp_grad(prob, sol, grads, e.PROBLEM_PARTS + e.ACTUATION_PARTS if sparts else ("g", "ce0"))
+        out = e.refs_grad(q, v, mask, refs, qg["g"], qg["ce0"], parts) if parts else {}
+        st = e.state_grad(q, v, mask, refs, qg, sparts) if sparts else {}
+        return (None, st.get("q"), st.get("v"), None, None) + tuple(out.get(k) for k in ctx.keys)
 
 
 def fp64_peak_tflops(device: int = 0) -> float:
