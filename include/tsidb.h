@@ -351,6 +351,46 @@ int tsidb_state_grad(tsidb_handle* h, int n_envs, int layout, const double* q, c
                      const tsidb_refs* refs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* grad, double* dq,
                      double* dv, void* cuda_stream);
 
+/* ---- linearizing the controller: forward-mode derivatives of export + solve ---------------------------------------
+ * tsidb_tick_jvp is the forward-mode derivative (Jacobian-vector product) of "tsidb_problem_data, then tsidb_qp_solve":
+ * for each env and each of n_dirs tangent directions in (q, v, references) it writes the tangent of the solve's x and of
+ * tau = TA x + ta0.  It is the transpose of what tsidb_qp_grad followed by tsidb_state_grad and tsidb_refs_grad compute.
+ *   q, v, contact_mask, refs, `layout`: as in tsidb_problem_data (`layout` applies to them only).
+ *   qp: that call's export (strides n_max, neq_max, nin_max at least tsidb_problem_sizes' and within the caps of
+ *       tsidb_qp_solve); H, CE, CI, sizes and, for a tau tangent, TA are read.  sol: tsidb_qp_solve's result on it; x,
+ *       status, active, lambda and lambda_eq are read.  A caller-enlarged problem is allowed: its appended variables and
+ *       rows are constants.
+ *   dirs: the directions, NULL = zero tangent for that input.  Per env [N][D][k] (shared_dirs == 0) or one set for every
+ *       env [D][k] (shared_dirs != 0: an identity gives a full Jacobian), always row-major: q [nq] in its raw doubles
+ *       (the quaternion unnormalised), v [nv], each reference array in its raw doubles (an SE3 rotation as its 9
+ *       column-major entries; the contact reference of a foot not in contact has no effect).
+ *   out: x [N][D][n_max] (zeros past the env's n) and tau [N][D][na]; NULL = not written, not both.
+ * The derivative is the one of the KKT system of the final working set W, the one that keeps W at a degenerate point
+ * (as tsidb_qp_grad): with G = [CE; CI_W] and nu = [lambda_eq; lambda_W], x' solves
+ *   H x' - G^T nu' = -(H' x + g' - G'^T nu),  G x' = -(G' x + [ce0'; ci0_W']),   tau' = TA' x + TA x' + ta0'.
+ * The export's tangent covers exactly its state- and reference-dependent entries (INTEGRATION.md); a joint-bound entry
+ * of ci0 that the export clips to +-1e10 has zero derivative.  A direction whose q and v parts are zero makes no
+ * tangent pass through the dynamics, so directions in the references alone are cheap.
+ * status[e] = TSIDB_STATUS_ERROR with all-zero tangents where tsidb_qp_grad would refuse the env (a solve status other
+ * than OPTIMAL, sizes that do not fit the strides or fall short of the export's, a corrupt working set, H not positive
+ * definite, dependent working-set rows), TSIDB_STATUS_OPTIMAL otherwise; the rest of the batch is processed and every
+ * byte of every requested output is written.  The host refuses null q, v, qp->H/CE/CI/sizes or sol arrays, both outputs
+ * NULL, n_dirs < 1, n_envs outside [1, max_envs], a bad layout, bad strides and misaligned arrays.  No workspace of the
+ * handle is used (nor its class sort or scheduling hint), so the call may run on any stream.  Asynchronous. */
+typedef struct tsidb_jvp_dirs {
+  const double* q; /* [N][D][nq], or [D][nq] when shared */
+  const double* v; /* [N][D][nv], or [D][nv] */
+  tsidb_refs refs; /* each [N][D][k], or [D][k]; k as in tsidb_refs */
+} tsidb_jvp_dirs;
+typedef struct tsidb_jvp_out {
+  double* x;   /* [N][D][n_max] */
+  double* tau; /* [N][D][na]    */
+} tsidb_jvp_out;
+int tsidb_tick_jvp(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v, const uint8_t* contact_mask,
+                   const tsidb_refs* refs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* qp,
+                   const tsidb_qp_out* sol, int n_dirs, int shared_dirs, const tsidb_jvp_dirs* dirs,
+                   const tsidb_jvp_out* out, int32_t* status, void* cuda_stream);
+
 /* controller.integrate_dv(q, v, dv, dt) (ref:ctrl/WalkController.py:291-295,
  * ref:legacy/biped.py:236-240): v_mean = v + dt/2*dv; v += dt*dv;
  * q = pin.integrate(q, dt*v_mean).  In place on device arrays.                   */

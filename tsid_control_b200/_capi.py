@@ -113,6 +113,14 @@ class TsidbRefsOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("com", "foot_lf", "foot_rf", "contact_lf", "contact_rf", "posture")]
 
 
+class TsidbJvpDirs(C.Structure):
+    _fields_ = [("q", C.c_void_p), ("v", C.c_void_p), ("refs", TsidbRefs)]
+
+
+class TsidbJvpOut(C.Structure):
+    _fields_ = [("x", C.c_void_p), ("tau", C.c_void_p)]
+
+
 def _fill(arr, values) -> None:
     v = np.asarray(values, dtype=np.float64).ravel()
     for i, x in enumerate(v):
@@ -284,6 +292,9 @@ def load_library() -> C.CDLL:
     lib.tsidb_state_grad.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, ip, C.POINTER(TsidbProblemOut), vp,
                                      vp, vp]
     lib.tsidb_state_grad.restype = ip
+    lib.tsidb_tick_jvp.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, ip, C.POINTER(TsidbProblemOut),
+                                   C.POINTER(TsidbQpOut), ip, ip, C.POINTER(TsidbJvpDirs), C.POINTER(TsidbJvpOut), vp, vp]
+    lib.tsidb_tick_jvp.restype = ip
     _LIB = lib
     return lib
 
@@ -301,5 +312,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
     "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve", "tsidb_qp_grad",
-    "tsidb_refs_grad", "tsidb_state_grad",
+    "tsidb_refs_grad", "tsidb_state_grad", "tsidb_tick_jvp",
 ]

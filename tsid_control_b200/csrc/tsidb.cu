@@ -209,6 +209,11 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
   TSIDB_ATTR(tsidb_refs_grad_kernel<24>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_state_grad_kernel<26>, TSIDB_S_SMEM, 1, "state gradient kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_state_grad_kernel<24>, TSIDB_S_SMEM, 1, "state gradient kernel", cudaSharedmemCarveoutMaxShared);
+  /* the forward derivative sizes its shared memory from the call's strides, up to all an SM gives one CTA */
+  CK(cudaFuncSetAttribute(tsidb_tick_jvp_kernel<26>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+  CK(cudaFuncSetAttribute(tsidb_tick_jvp_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+  CK(cudaFuncSetAttribute(tsidb_tick_jvp_kernel<26>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  CK(cudaFuncSetAttribute(tsidb_tick_jvp_kernel<24>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<26, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_SMEM_DOUBLES(26) * sizeof(double)))));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<24, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_SMEM_DOUBLES(24) * sizeof(double)))));
   CK((cudaFuncSetAttribute(tsidb_tick_small_kernel<26, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(TSIDB_SMALL_LOCAL_SMEM_DOUBLES(26) * sizeof(double)))));
@@ -969,6 +974,75 @@ extern "C" int tsidb_state_grad(tsidb_handle* h, int n_envs, int layout, const d
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (h->dc.nv == 26) tsidb_state_grad_kernel<26><<<blocks, 32 * TSIDB_S_CTA_WARPS, TSIDB_S_SMEM, st>>>(a, r);
   else tsidb_state_grad_kernel<24><<<blocks, 32 * TSIDB_S_CTA_WARPS, TSIDB_S_SMEM, st>>>(a, r);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
+/* forward derivative of export + solve: one launch that recomputes K1 and K2 per env, factors the working-set KKT system
+ * and runs K1 in tangent arithmetic per direction, no workspace of the handle */
+extern "C" int tsidb_tick_jvp(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
+                              const uint8_t* contact_mask, const tsidb_refs* refs, int n_max, int neq_max, int nin_max,
+                              const tsidb_problem_out* qp, const tsidb_qp_out* sol, int n_dirs, int shared_dirs,
+                              const tsidb_jvp_dirs* dirs, const tsidb_jvp_out* out, int32_t* status, void* cuda_stream) {
+  if (!h || !q || !v || !qp || !sol || !dirs || !out || !status) { g_err = "tsidb_tick_jvp: null argument"; return -1; }
+  if (!out->x && !out->tau) { g_err = "tsidb_tick_jvp: out->x and out->tau are both NULL"; return -1; }
+  if (n_dirs < 1) { g_err = "tsidb_tick_jvp: n_dirs must be positive"; return -1; }
+  if (n_envs <= 0 || n_envs > h->max_envs) { g_err = "tsidb_tick_jvp: n_envs must be in [1, max_envs]"; return -1; }
+  if (layout != 0 && layout != 1) { g_err = "tsidb_tick_jvp: layout must be 0 ([N][dof]) or 1 ([dof][N])"; return -1; }
+  int nx, neq, nin;
+  problem_maxima(h, &nx, &neq, &nin);
+  if (n_max < nx || neq_max < neq || nin_max < nin || n_max > TSIDB_QP_MAX_N || neq_max > n_max || nin_max > TSIDB_QP_MAX_NIN) {
+    g_err = "tsidb_tick_jvp: strides must be at least tsidb_problem_sizes' maxima, n_max <= TSIDB_QP_MAX_N (64), "
+            "neq_max <= n_max, nin_max <= TSIDB_QP_MAX_NIN (512)";
+    return -1;
+  }
+  if (!qp->H || !qp->CE || !qp->CI || !qp->sizes || !sol->x || !sol->status || !sol->active || !sol->lambda ||
+      !sol->lambda_eq) {
+    g_err = "tsidb_tick_jvp: H, CE, CI, sizes and the solution's x, status, active, lambda and lambda_eq are required";
+    return -1;
+  }
+  if (out->tau && !qp->TA) { g_err = "tsidb_tick_jvp: a tau tangent needs TA"; return -1; }
+  for (const void* p : {(const void*)q, (const void*)v, (const void*)qp->H, (const void*)qp->CE, (const void*)qp->CI,
+                        (const void*)qp->TA, (const void*)sol->x, (const void*)sol->lambda, (const void*)sol->lambda_eq,
+                        (const void*)dirs->q, (const void*)dirs->v, (const void*)dirs->refs.com, (const void*)dirs->refs.foot_lf,
+                        (const void*)dirs->refs.foot_rf, (const void*)dirs->refs.contact_lf, (const void*)dirs->refs.contact_rf,
+                        (const void*)dirs->refs.posture, (const void*)out->x, (const void*)out->tau})
+    if (((uintptr_t)p & 7) != 0) { g_err = "tsidb_tick_jvp: fp64 arrays must be 8-byte aligned"; return -1; }
+  for (const void* p : {(const void*)qp->sizes, (const void*)sol->status, (const void*)sol->active, (const void*)status})
+    if (((uintptr_t)p & 3) != 0) { g_err = "tsidb_tick_jvp: int32 arrays must be 4-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  const size_t per_warp = (size_t)TSIDB_J_PER_WARP(n_max, nin_max) * sizeof(double);
+  int optin = 0;
+  CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+  int warps = (int)(((size_t)optin - MDL_SIZE * sizeof(double)) / per_warp);
+  if (warps > TSIDB_J_MAX_WARPS) warps = TSIDB_J_MAX_WARPS;
+  if (warps < 1) { g_err = "tsidb_tick_jvp: the kernel does not fit an SM at these strides"; return -2; }
+  const size_t smem = (size_t)warps * per_warp + MDL_SIZE * sizeof(double);
+  TickArgs a;
+  memset(&a, 0, sizeof a);
+  a.n_envs = n_envs; a.layout = layout;
+  a.q = q; a.v = v; a.mask = contact_mask;
+  if (refs) {
+    a.r_com = refs->com; a.r_foot[0] = refs->foot_lf; a.r_foot[1] = refs->foot_rf;
+    a.r_contact[0] = refs->contact_lf; a.r_contact[1] = refs->contact_rf; a.r_posture = refs->posture;
+  }
+  a.slot = h->slot;
+  a.tables = h->tables;
+  JvpArgs j;
+  memset(&j, 0, sizeof j);
+  j.n_max = n_max; j.neq_max = neq_max; j.nin_max = nin_max; j.n_dirs = n_dirs; j.shared = shared_dirs != 0;
+  j.H = qp->H; j.CE = qp->CE; j.CI = qp->CI; j.TA = qp->TA; j.sizes = qp->sizes;
+  j.x = sol->x; j.lambda = sol->lambda; j.lambda_eq = sol->lambda_eq; j.sol_status = sol->status; j.active = sol->active;
+  j.dq = dirs->q; j.dv = dirs->v;
+  j.dref[0] = dirs->refs.com; j.dref[1] = dirs->refs.foot_lf; j.dref[2] = dirs->refs.foot_rf;
+  j.dref[3] = dirs->refs.contact_lf; j.dref[4] = dirs->refs.contact_rf; j.dref[5] = dirs->refs.posture;
+  j.ox = out->x; j.otau = out->tau; j.status = status;
+  int blocks = (n_envs + warps - 1) / warps;
+  if (blocks > h->sm_count) blocks = h->sm_count; /* persistent */
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  if (h->dc.nv == 26) tsidb_tick_jvp_kernel<26><<<blocks, 32 * warps, smem, st>>>(a, j);
+  else tsidb_tick_jvp_kernel<24><<<blocks, 32 * warps, smem, st>>>(a, j);
   CK(cudaGetLastError());
   h->launches += 1;
   return 0;

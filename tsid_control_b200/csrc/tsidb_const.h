@@ -166,6 +166,21 @@ struct StateGradArgs {
   double *dq, *dv;
 };
 
+/* arguments of the forward derivative of export + solve (tsidb_tick_jvp): the export qp and its solution sol as
+ * tsidb_qp_grad reads them, n_dirs tangent directions per env ([N][D][k]) or shared by all envs ([D][k]) in q, v and the
+ * tsidb_refs arrays com, foot_lf, foot_rf, contact_lf, contact_rf, posture (NULL = zero), and the tangents of x
+ * [N][D][n_max] and tau [N][D][na] (NULL = not written) */
+struct JvpArgs {
+  int32_t n_max, neq_max, nin_max, n_dirs, shared;
+  const double *H, *CE, *CI, *TA;
+  const int32_t* sizes;
+  const double *x, *lambda, *lambda_eq;
+  const int32_t *sol_status, *active;
+  const double *dq, *dv, *dref[6];
+  double *ox, *otau;
+  int32_t* status;
+};
+
 struct TickArgs {
   int32_t n_envs, layout, pad_;
   const double* q;

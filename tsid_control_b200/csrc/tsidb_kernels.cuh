@@ -3540,6 +3540,140 @@ TSIDB_DEV void qg_reflect(const double* M, int ld, const double* beta, int n, in
 
 TSIDB_DEV double qg_lane(const double (&v)[QP_SLOTS], int i) { return __shfl_sync(FULL, (i >> 5) ? v[QP_SLOTS - 1] : v[0], i & 31); }
 
+/* The factorisation of the working-set KKT system and the solve through it, shared by the adjoint of the QP solve
+ * (qp_grad_env) and the forward derivative of the tick (tick_jvp_env), called in this order:
+ *   qg_working_set, qp_llt, qg_fill_G, qg_lsolve_cols, qg_qr, then per right-hand side qg_lsolve and qg_kkt_solve. */
+/* the working set of an env from the solve's `active` row: W[k] = the CI row of entry k, pos[r] = its entry or -1 for
+ * r < nin; false unless the entries >= 0 are a -1 padded prefix of distinct rows of [0, nin) with neq + |W| <= n.
+ * m = neq + |W| */
+TSIDB_DEV bool qg_working_set(const int32_t* active, int n, int neq, int nin, int* W, int* pos, int& m, int lane) {
+  int act[QP_SLOTS];
+  bool bad = false;
+  for (int r = lane; r < nin; r += 32) pos[r] = -1;
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++) {
+    const int k = lane + 32 * t;
+    act[t] = k < n ? active[k] : -1;
+    bad |= act[t] < -1 || act[t] >= nin;
+  }
+  unsigned long long used = 0;
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++) used |= (unsigned long long)__ballot_sync(FULL, act[t] >= 0) << (32 * t);
+  int w = 0;
+  while (w < 64 && ((used >> w) & 1ull)) w++;
+  bad |= (used & (used + 1)) != 0 || neq + w > n; /* the entries >= 0 are a prefix */
+  __syncwarp();
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++)
+    if (!bad && act[t] >= 0) {
+      pos[act[t]] = lane + 32 * t;
+      W[lane + 32 * t] = act[t];
+    }
+  __syncwarp();
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++) bad |= !bad && act[t] >= 0 && pos[act[t]] != lane + 32 * t; /* duplicate row */
+  m = neq + w;
+  return __ballot_sync(FULL, bad) == 0;
+}
+/* M = G' (row j of G = [CE; CI_W] into column j) */
+TSIDB_DEV void qg_fill_G(const double* CE, const double* CI, const int* W, int nm, int n, int neq, int m, double* M, int ld,
+                         int lane) {
+  for (int j = 0; j < m; j++) {
+    const double* row = j < neq ? CE + (size_t)j * nm : CI + (size_t)W[j - neq] * nm;
+    for (int i = lane; i < n; i += 32) M[i * ld + j] = row[i];
+  }
+}
+/* M = L^-1 M: forward substitution, a lane per column */
+TSIDB_DEV void qg_lsolve_cols(const double* L, double* M, int ld, int n, int m, int lane) {
+  for (int j = lane; j < m; j += 32)
+    for (int i = 0; i < n; i++) {
+      double s = M[i * ld + j];
+      for (int k = 0; k < i; k++) s -= L[i * ld + k] * M[k * ld + j];
+      M[i * ld + j] = s / L[i * ld + i];
+    }
+}
+/* y = L^-1 y, column-oriented; y in the lane-owned registers */
+TSIDB_DEV void qg_lsolve(const double* L, int ld, int n, double (&y)[QP_SLOTS], int lane) {
+  for (int i = 0; i < n; i++) {
+    const double yi = qg_lane(y, i) / L[i * ld + i];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int k = lane + 32 * t;
+      if (k > i && k < n) y[t] -= L[k * ld + i] * yi;
+      else if (k == i) y[t] = yi;
+    }
+  }
+}
+/* Householder QR of M: reflector k in column k (rows k..n-1), R above the diagonal, its diagonal in rdiag.  A diagonal at
+ * or below eps times the largest so far is a dependent row (the solve's own test in add_constraint): false. */
+TSIDB_DEV bool qg_qr(double* M, int ld, double* beta, double* rdiag, int n, int m, int lane) {
+  double R_norm = 1.0;
+  for (int k = 0; k < m; k++) {
+    double s2 = 0.0;
+    for (int i = k + lane; i < n; i += 32) s2 += M[i * ld + k] * M[i * ld + k];
+    s2 = warp_sum(s2);
+    const double x0 = M[k * ld + k], nrm = sqrt(s2);
+    const double alpha = x0 > 0 ? -nrm : nrm;
+    if (!(nrm > TS_EPS * R_norm)) return false;
+    if (nrm > R_norm) R_norm = nrm;
+    const double bk = 1.0 / (nrm * (nrm + fabs(x0))); /* 2 / v'v */
+    __syncwarp();
+    if (lane == 0) { M[k * ld + k] = x0 - alpha; beta[k] = bk; rdiag[k] = alpha; }
+    __syncwarp();
+    for (int j = k + 1 + lane; j < m; j += 32) {
+      double d = 0.0;
+      for (int i = k; i < n; i++) d += M[i * ld + k] * M[i * ld + j];
+      d *= bk;
+      for (int i = k; i < n; i++) M[i * ld + j] -= d * M[i * ld + k];
+    }
+    __syncwarp();
+  }
+  return true;
+}
+/* H p + G' q = xb, G p = -nub through the factors, with y = L^-1 xb and v = nub on entry (lane-owned registers):
+ *   p~ = Q2 Q2' y - Q1 R^-T nub,  q = R^-1 (Q1' y + R^-T nub),  p = L^-T p~;  p is left in y, q in u. */
+TSIDB_DEV void qg_kkt_solve(const double* L, const double* M, int ld, const double* beta, const double* rdiag, int n, int m,
+                            double (&y)[QP_SLOTS], double (&v)[QP_SLOTS], double (&u)[QP_SLOTS], int lane) {
+  qg_reflect(M, ld, beta, n, m, true, y, lane); /* y = Q' L^-1 xb = [z1; z2] */
+  /* v = R^-T nub, column-oriented forward substitution */
+  for (int i = 0; i < m; i++) {
+    const double vi = qg_lane(v, i) / rdiag[i];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int j = lane + 32 * t;
+      if (j > i && j < m) v[t] -= M[i * ld + j] * vi;
+      else if (j == i) v[t] = vi;
+    }
+  }
+  /* q = R^-1 (z1 + v), back substitution; then y = [-v; z2] */
+#pragma unroll
+  for (int t = 0; t < QP_SLOTS; t++) {
+    const int j = lane + 32 * t;
+    u[t] = j < m ? y[t] + v[t] : 0.0;
+    if (j < m) y[t] = -v[t];
+  }
+  for (int i = m - 1; i >= 0; i--) {
+    const double qi = qg_lane(u, i) / rdiag[i];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int j = lane + 32 * t;
+      if (j < i) u[t] -= M[j * ld + i] * qi;
+      else if (j == i) u[t] = qi;
+    }
+  }
+  qg_reflect(M, ld, beta, n, m, false, y, lane); /* p~ */
+  /* p = L^-T p~, column-oriented back substitution */
+  for (int i = n - 1; i >= 0; i--) {
+    const double pi = qg_lane(y, i) / L[i * ld + i];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int k = lane + 32 * t;
+      if (k < i) y[t] -= L[i * ld + k] * pi;
+      else if (k == i) y[t] = pi;
+    }
+  }
+}
+
 /* one env; sm holds qg_layout(a.n_max, a.nin_max).per_env doubles of this warp */
 TSIDB_DEV void qp_grad_env(const QpGradArgs& a, double* sm, int env, int lane) {
   const QgLayout Ly = qg_layout(a.n_max, a.nin_max);
@@ -3553,47 +3687,13 @@ TSIDB_DEV void qp_grad_env(const QpGradArgs& a, double* sm, int env, int lane) {
   bool ok = a.sol_status[env] == ST_OPTIMAL && n >= 1 && n <= nm && neq >= 0 && neq <= n && neq <= a.neq_max && nin >= 0 &&
             nin <= a.nin_max;
   int m = 0;
-  if (ok) {
-    /* the working set: -1 padded entries of [0, nin), no duplicates, neq + |W| <= n */
-    int act[QP_SLOTS];
-    bool bad = false;
-    for (int r = lane; r < nin; r += 32) pos[r] = -1;
-#pragma unroll
-    for (int t = 0; t < QP_SLOTS; t++) {
-      const int k = lane + 32 * t;
-      act[t] = k < n ? a.active[(size_t)env * nm + k] : -1;
-      bad |= act[t] < -1 || act[t] >= nin;
-    }
-    unsigned long long used = 0;
-#pragma unroll
-    for (int t = 0; t < QP_SLOTS; t++) used |= (unsigned long long)__ballot_sync(FULL, act[t] >= 0) << (32 * t);
-    int w = 0;
-    while (w < 64 && ((used >> w) & 1ull)) w++;
-    bad |= (used & (used + 1)) != 0 || neq + w > n; /* the entries >= 0 are a prefix */
-    __syncwarp();
-#pragma unroll
-    for (int t = 0; t < QP_SLOTS; t++)
-      if (!bad && act[t] >= 0) {
-        pos[act[t]] = lane + 32 * t;
-        W[lane + 32 * t] = act[t];
-      }
-    __syncwarp();
-#pragma unroll
-    for (int t = 0; t < QP_SLOTS; t++) bad |= !bad && act[t] >= 0 && pos[act[t]] != lane + 32 * t; /* duplicate row */
-    ok = __ballot_sync(FULL, bad) == 0;
-    m = neq + w;
-  }
+  if (ok) ok = qg_working_set(a.active + (size_t)env * nm, n, neq, nin, W, pos, m, lane);
   const double* H = a.H + (size_t)env * nm * nm;
   if (ok) ok = qp_llt(H, nm, L, ld, n, lane);
   double y[QP_SLOTS], v[QP_SLOTS];
   if (ok) {
-    const double* CE = a.CE + (size_t)env * a.neq_max * nm;
-    const double* CI = a.CI + (size_t)env * a.nin_max * nm;
-    /* M = G' (row j of G into column j), x, nu, y = xb + TA' taub */
-    for (int j = 0; j < m; j++) {
-      const double* row = j < neq ? CE + (size_t)j * nm : CI + (size_t)W[j - neq] * nm;
-      for (int i = lane; i < n; i += 32) M[i * ld + j] = row[i];
-    }
+    /* M = G', x, nu, y = xb + TA' taub */
+    qg_fill_G(a.CE + (size_t)env * a.neq_max * nm, a.CI + (size_t)env * a.nin_max * nm, W, nm, n, neq, m, M, ld, lane);
     for (int i = lane; i < n; i += 32) x[i] = a.x[(size_t)env * nm + i];
     for (int j = lane; j < m; j += 32) nu[j] = j < neq ? a.lambda_eq[(size_t)env * a.neq_max + j] : a.lambda[(size_t)env * nm + j - neq];
 #pragma unroll
@@ -3612,88 +3712,14 @@ TSIDB_DEV void qp_grad_env(const QpGradArgs& a, double* sm, int env, int lane) {
       else if (j >= neq && j < m && a.glambda) v[t] = a.glambda[(size_t)env * nm + j - neq];
     }
     __syncwarp();
-    /* M = L^-1 G': forward substitution, a lane per column */
-    for (int j = lane; j < m; j += 32)
-      for (int i = 0; i < n; i++) {
-        double s = M[i * ld + j];
-        for (int k = 0; k < i; k++) s -= L[i * ld + k] * M[k * ld + j];
-        M[i * ld + j] = s / L[i * ld + i];
-      }
-    /* y = L^-1 y, column-oriented */
-    for (int i = 0; i < n; i++) {
-      const double yi = qg_lane(y, i) / L[i * ld + i];
-#pragma unroll
-      for (int t = 0; t < QP_SLOTS; t++) {
-        const int k = lane + 32 * t;
-        if (k > i && k < n) y[t] -= L[k * ld + i] * yi;
-        else if (k == i) y[t] = yi;
-      }
-    }
+    qg_lsolve_cols(L, M, ld, n, m, lane);
+    qg_lsolve(L, ld, n, y, lane);
     __syncwarp();
-    /* Householder QR of M: reflector k in column k (rows k..n-1), R above the diagonal, its diagonal in rdiag.  A
-     * diagonal at or below eps times the largest so far is a dependent row (the solve's own test in add_constraint). */
-    double R_norm = 1.0;
-    for (int k = 0; k < m; k++) {
-      double s2 = 0.0;
-      for (int i = k + lane; i < n; i += 32) s2 += M[i * ld + k] * M[i * ld + k];
-      s2 = warp_sum(s2);
-      const double x0 = M[k * ld + k], nrm = sqrt(s2);
-      const double alpha = x0 > 0 ? -nrm : nrm;
-      if (!(nrm > TS_EPS * R_norm)) { ok = false; break; }
-      if (nrm > R_norm) R_norm = nrm;
-      const double bk = 1.0 / (nrm * (nrm + fabs(x0))); /* 2 / v'v */
-      __syncwarp();
-      if (lane == 0) { M[k * ld + k] = x0 - alpha; beta[k] = bk; rdiag[k] = alpha; }
-      __syncwarp();
-      for (int j = k + 1 + lane; j < m; j += 32) {
-        double d = 0.0;
-        for (int i = k; i < n; i++) d += M[i * ld + k] * M[i * ld + j];
-        d *= bk;
-        for (int i = k; i < n; i++) M[i * ld + j] -= d * M[i * ld + k];
-      }
-      __syncwarp();
-    }
+    ok = qg_qr(M, ld, beta, rdiag, n, m, lane);
   }
   if (ok) {
-    qg_reflect(M, ld, beta, n, m, true, y, lane); /* y = Q' L^-1 xb = [z1; z2] */
-    /* v = R^-T nub, column-oriented forward substitution */
-    for (int i = 0; i < m; i++) {
-      const double vi = qg_lane(v, i) / rdiag[i];
-#pragma unroll
-      for (int t = 0; t < QP_SLOTS; t++) {
-        const int j = lane + 32 * t;
-        if (j > i && j < m) v[t] -= M[i * ld + j] * vi;
-        else if (j == i) v[t] = vi;
-      }
-    }
-    /* q = R^-1 (z1 + v), back substitution; then y = [-v; z2] */
     double u[QP_SLOTS];
-#pragma unroll
-    for (int t = 0; t < QP_SLOTS; t++) {
-      const int j = lane + 32 * t;
-      u[t] = j < m ? y[t] + v[t] : 0.0;
-      if (j < m) y[t] = -v[t];
-    }
-    for (int i = m - 1; i >= 0; i--) {
-      const double qi = qg_lane(u, i) / rdiag[i];
-#pragma unroll
-      for (int t = 0; t < QP_SLOTS; t++) {
-        const int j = lane + 32 * t;
-        if (j < i) u[t] -= M[j * ld + i] * qi;
-        else if (j == i) u[t] = qi;
-      }
-    }
-    qg_reflect(M, ld, beta, n, m, false, y, lane); /* p~ */
-    /* p = L^-T p~, column-oriented back substitution */
-    for (int i = n - 1; i >= 0; i--) {
-      const double pi = qg_lane(y, i) / L[i * ld + i];
-#pragma unroll
-      for (int t = 0; t < QP_SLOTS; t++) {
-        const int k = lane + 32 * t;
-        if (k < i) y[t] -= L[i * ld + k] * pi;
-        else if (k == i) y[t] = pi;
-      }
-    }
+    qg_kkt_solve(L, M, ld, beta, rdiag, n, m, y, v, u, lane);
 #pragma unroll
     for (int t = 0; t < QP_SLOTS; t++) {
       const int k = lane + 32 * t;
@@ -3729,6 +3755,387 @@ TSIDB_DEV void qp_grad_env(const QpGradArgs& a, double* sm, int env, int lane) {
   if (a.dTA)
     qg_store(a.dTA + (size_t)env * na * nm, na, nm, lane, [&](int r, int j) { return (gt && j < nx) ? gt[r] * x[j] : 0.0; });
   if (a.dta0) qg_store(a.dta0 + (size_t)env * na, 1, na, lane, [&](int, int r) { return gt ? gt[r] : 0.0; });
+}
+
+/* ================================================================= forward derivative of export + solve (tsidb_tick_jvp) */
+/* Per warp: the tangent workspace (K1_DUAL_SIZE Duals), this env's primal workspace (SM_PER_ENV doubles: q, v, the
+ * references, K1 and K2 in double as the tick runs them) followed by the JV_* vectors below, and the KKT factors of
+ * qg_layout(n_max, nin_max). */
+#define JV_oJL SM_PER_ENV          /* the four SE3 laws' log6 Jacobians in (E 9, ep 3), 6 x 12 per lane 0..3        288 */
+#define JV_oA (JV_oJL + 288)       /* a = [JF; Jcom; Ag] x_dv                                                         18 */
+#define JV_oPHI (JV_oA + 18)       /* T f_s of the force slots (6 per slot)                                           12 */
+#define JV_oNUD (JV_oPHI + 12)     /* multiplier of each dynamics row (M | -Jc^T) summed over CE and the actuation rows 32 */
+#define JV_oNUJ (JV_oNUD + 32)     /* multiplier of each contact-motion (JF) row, by foot                              12 */
+#define JV_oDQV (JV_oNUJ + 12)     /* per direction: dq (32), dv (32)                                                 64 */
+#define JV_oDRF (JV_oDQV + 64)     /* per direction: the references' tangents at the RF_* offsets                    106 */
+#define JV_oAD (JV_oDRF + 106)     /* per direction: [JF; Jcom; Ag]' x_dv (18), then JF' nu_dyn (12)                    30 */
+#define JV_oBD (JV_oAD + 30)       /* per direction: the task right-hand sides' tangents at the BV_* offsets           64 */
+#define JV_oDD (JV_oBD + 64)       /* per direction: (M | -Jc^T)' x of the dynamics rows (32), then nle' (32)           64 */
+#define JV_oDK (JV_oDD + 64)       /* the G rows: kind (int, 64), index (int, 64), as 64 doubles; coefficient (64)     128 */
+#define JV_oXD (JV_oDK + 128)      /* per direction: x' (64)                                                          64 */
+#define JV_oM (JV_oXD + 64)        /* m = neq + |W| (int)                                                              2 */
+#define JV_SIZE (JV_oM + 2)
+#define JV_DUALS (2 * K1_DUAL_SIZE)
+#define TSIDB_J_PER_WARP(n_max, nin_max) (JV_DUALS + JV_SIZE + qg_layout(n_max, nin_max).per_env)
+static_assert((JV_DUALS % 2) == 0 && (JV_SIZE % 2) == 0, "every region starts 16-byte aligned");
+
+/* One env of tsidb_tick_jvp.  q, v and the references are staged and K1 + K2 run in double (sm); the working-set KKT
+ * system of sol is factored as tsidb_qp_grad factors it.  Then per direction: K1 in tangent arithmetic seeded with the
+ * direction's q and v parts (skipped when both are zero), the right-hand sides
+ *   r1 = -(H' x + g' - G'^T nu),  r2 = -(G' x + b')    (G = [CE; CI_W], b = [ce0; ci0_W], nu = [lambda_eq; lambda_W])
+ * formed from the tangents of K1's outputs, the task right-hand sides and the references, never from a tangent of the
+ * export, and H x' - G^T nu' = r1, G x' = r2 solved through the factors (qp_grad's system with xb = r1, nub = -r2);
+ * tau' = TA' x + ta0' + TA x'.  The tangent covers the entries state_adjoint_env and refs_adjoint_env read; the rest of
+ * the export (and whatever a caller appended) is constant. */
+/* the per-env part: staging, K1 and K2, the factors and what every direction reuses; false (status 4, zero outputs
+ * written) when the env is not differentiated.  Not inlined, like tick_jvp_dir: the tangent K1 between them then keeps
+ * the registers to itself. */
+template <int NV>
+TSIDB_DEVNI bool tick_jvp_setup(const DevConst& C, const double* mdl, double* sm, double* qs, const TickArgs& a,
+                                const JvpArgs& j, int env, int lane) {
+  constexpr int nv = NV, na = NV - 6, nq = NV + 1;
+  const double BIG = 1e10; /* the export's clip of the joint-bound rows */
+  const QgLayout Ly = qg_layout(j.n_max, j.nin_max);
+  const int nm = j.n_max, ld = Ly.ld, D = j.n_dirs;
+  double *L = qs + Ly.oL, *M = qs + Ly.oM, *x = qs + Ly.ox, *nu = qs + Ly.onu, *beta = qs + Ly.obeta, *rdiag = qs + Ly.ordiag;
+  int* W = reinterpret_cast<int*>(qs + Ly.oI) + Ly.oW;
+  int* pos = reinterpret_cast<int*>(qs + Ly.oI) + Ly.opos;
+  int* dkind = reinterpret_cast<int*>(sm + JV_oDK);
+  int* didx = dkind + 64;
+  double* dcoef = sm + JV_oDK + 64;
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  if (lane < nq) sm[SM_oQV + lane] = ldin(a.q, a, env, lane, nq);
+  if (lane < nv) sm[SM_oQV + 32 + lane] = ldin(a.v, a, env, lane, nv);
+  stage_refs(C, mdl, sm, a, env, lane, na);
+  __syncwarp();
+  k1_dynamics<NV>(C, mdl, sm, lane);
+  stage_refs_wait();
+  const int mask = a.mask ? (a.mask[env] & 3) : 3;
+  const int nc = (mask & 1) + ((mask >> 1) & 1);
+  const int f0 = (mask & 1) ? 0 : 1; /* foot of force slot 0; slot 1 is RF */
+  const int nx_e = nv + 12 * nc, neq_e = 6 + 6 * nc;
+  const int nin_e = 2 * (17 * nc + (C.use_tb ? na : 0) + (C.use_jb ? nv : 0));
+  const int oAct = 34 * nc; /* first actuation row of CI */
+  k2_assemble<NV>(C, mdl, sm, a, env, lane, mask, neq_e, nx_e);
+
+  /* the KKT factors of the final working set; the export's own rows and variables must be there */
+  const int n = j.sizes[(size_t)env * 3], neq = j.sizes[(size_t)env * 3 + 1], nin = j.sizes[(size_t)env * 3 + 2];
+  bool ok = j.sol_status[env] == ST_OPTIMAL && n >= nx_e && n <= nm && neq >= neq_e && neq <= n && neq <= j.neq_max &&
+            nin >= nin_e && nin <= j.nin_max;
+  int m = 0;
+  if (ok) ok = qg_working_set(j.active + (size_t)env * nm, n, neq, nin, W, pos, m, lane);
+  if (ok) ok = qp_llt(j.H + (size_t)env * nm * nm, nm, L, ld, n, lane);
+  if (ok) {
+    qg_fill_G(j.CE + (size_t)env * j.neq_max * nm, j.CI + (size_t)env * j.nin_max * nm, W, nm, n, neq, m, M, ld, lane);
+    for (int i = lane; i < n; i += 32) x[i] = j.x[(size_t)env * nm + i];
+    for (int k = lane; k < m; k += 32) nu[k] = k < neq ? j.lambda_eq[(size_t)env * j.neq_max + k] : j.lambda[(size_t)env * nm + k - neq];
+    __syncwarp();
+    qg_lsolve_cols(L, M, ld, n, m, lane);
+    __syncwarp();
+    ok = qg_qr(M, ld, beta, rdiag, n, m, lane);
+  }
+  if (lane == 0) j.status[env] = ok ? ST_OPTIMAL : ST_ERROR;
+  if (!ok) { /* every byte of every requested output */
+    for (int d = 0; d < D; d++) {
+      if (j.ox) for (int k = lane; k < nm; k += 32) j.ox[((size_t)env * D + d) * nm + k] = 0.0;
+      if (j.otau && lane < na) j.otau[((size_t)env * D + d) * na + lane] = 0.0;
+    }
+    return false;
+  }
+
+  /* once per env: the log6 Jacobians, a, T f, the multipliers of the dynamics and contact-motion rows, the G rows */
+  const double* JF = sm + SM_oJF; /* [JF; Jcom; Ag]: 18 rows of stride TSIDB_NVX */
+  const double* fr = sm + SM_oFr;
+  const double* rf = sm + SM_oRef;
+  if (lane < 4) {
+    const int f = lane & 1;
+    const bool is_contact = lane < 2;
+    const double* ref = is_contact ? rf + RF_CONTACT + 12 * f : rf + RF_FOOT + 24 * f;
+    const double* pf = fr + FR_OMF + f * 12;
+    const double* Rf = pf + 3;
+    double Rr[9], dp[3], E[9], ep[3];
+#pragma unroll
+    for (int c = 0; c < 3; c++)
+#pragma unroll
+      for (int q = 0; q < 3; q++) Rr[3 * q + c] = ref[3 + 3 * c + q];
+    dp[0] = ref[0] - pf[0]; dp[1] = ref[1] - pf[1]; dp[2] = ref[2] - pf[2];
+#pragma unroll
+    for (int i = 0; i < 3; i++)
+#pragma unroll
+      for (int q = 0; q < 3; q++) E[3 * i + q] = Rf[i] * Rr[q] + Rf[3 + i] * Rr[3 + q] + Rf[6 + i] * Rr[6 + q];
+    mtv3(Rf, dp, ep);
+    double* JL = sm + JV_oJL + 72 * lane;
+    for (int k = 0; k < 6; k++) { /* row k of d log6 / d(E, ep): the adjoint with a unit cotangent */
+      double ol[3] = {0, 0, 0}, oa[3] = {0, 0, 0};
+      if (k < 3) ol[k] = 1.0; else oa[k - 3] = 1.0;
+      double* row = JL + 12 * k;
+      for (int i = 0; i < 12; i++) row[i] = 0.0;
+      log6_adj(E, ep, ol, oa, row, row + 9);
+    }
+  }
+  if (lane < 18) {
+    double s = 0.0;
+    for (int k = 0; k < nv; k++) s += JF[lane * TSIDB_NVX + k] * x[k];
+    sm[JV_oA + lane] = s;
+  }
+  if (lane < 12) {
+    const int s = lane / 6, mm = lane % 6;
+    double t = 0.0;
+    if (s < nc)
+      for (int k = 0; k < 12; k++) t += C.T[mm][k] * x[nv + 12 * s + k];
+    sm[JV_oPHI + lane] = t;
+    const int f = lane / 6; /* contact-motion row of foot f: 6 + 6 s + k with s its force slot */
+    sm[JV_oNUJ + lane] = ((mask >> f) & 1) ? nu[6 + 6 * (f == f0 ? 0 : 1) + lane % 6] : 0.0;
+  }
+  if (lane < nv) {
+    double t = 0.0;
+    if (lane < 6) t = nu[lane];
+    else if (C.use_tb) {
+      const int lo = pos[oAct + lane - 6], up = pos[oAct + na + lane - 6];
+      if (lo >= 0) t += nu[neq + lo];
+      if (up >= 0) t -= nu[neq + up];
+    }
+    sm[JV_oNUD + lane] = t;
+  }
+  /* G rows: kind 1 = dynamics row idx with sign coef, 2 = contact-motion row (JF row idx), 3 = joint-bound row of
+   * joint idx (coef = d ci0 / d v_idx), 0 = constant */
+  for (int r = lane; r < m; r += 32) {
+    int kind = 0, idx = 0;
+    double coef = 0.0;
+    if (r < neq) {
+      if (r < 6) { kind = 1; idx = r; coef = 1.0; }
+      else if (r < neq_e) { kind = 2; idx = (((r < 12) ? f0 : 1) * 6) + (r - 6) % 6; }
+    } else if (W[r - neq] < nin_e) {
+      int side = 0, i = 0, slot = 0;
+      const int blk = ci_block(C, W[r - neq], nc, na, nv, side, i, slot);
+      if (blk == 2) { kind = 1; idx = 6 + i; coef = side ? -1.0 : 1.0; }
+      else if (blk == 3 && i >= 6) {
+        const double vj = sm[SM_oQV + 32 + i];
+        const double hi = (C.v_max[i - 6] - vj) / C.jb_dt, lo = (C.v_min[i - 6] - vj) / C.jb_dt;
+        kind = 3; idx = i;
+        coef = side ? (hi < BIG ? -1.0 / C.jb_dt : 0.0) : (lo > -BIG ? 1.0 / C.jb_dt : 0.0);
+      }
+    }
+    dkind[r] = kind; didx[r] = idx; dcoef[r] = coef;
+  }
+  if (lane == 0) *reinterpret_cast<int*>(sm + JV_oM) = m;
+  __syncwarp();
+  return true;
+}
+
+/* one direction d after its tangents are staged in sm (and, when kin, the tangent K1 ran in ds): the right-hand sides,
+ * the solve through the factors and the stores of x' and tau' */
+template <int NV>
+TSIDB_DEVNI void tick_jvp_dir(const DevConst& C, const double* mdl, const Dual* ds, double* sm, const double* qs,
+                              const TickArgs& a, const JvpArgs& j, int env, int d, bool kin, int lane) {
+  constexpr int nv = NV, na = NV - 6;
+  const QgLayout Ly = qg_layout(j.n_max, j.nin_max);
+  const int nm = j.n_max, ld = Ly.ld, D = j.n_dirs;
+  const double *L = qs + Ly.oL, *M = qs + Ly.oM, *x = qs + Ly.ox, *beta = qs + Ly.obeta, *rdiag = qs + Ly.ordiag;
+  const int* dkind = reinterpret_cast<const int*>(sm + JV_oDK);
+  const int* didx = dkind + 64;
+  const double* dcoef = sm + JV_oDK + 64;
+  const int n = j.sizes[(size_t)env * 3], m = *reinterpret_cast<const int*>(sm + JV_oM);
+  const int mask = a.mask ? (a.mask[env] & 3) : 3;
+  const int nc = (mask & 1) + ((mask >> 1) & 1);
+  const int f0 = (mask & 1) ? 0 : 1;
+  const int nx_e = nv + 12 * nc;
+  const double* JF = sm + SM_oJF;
+  const double* fr = sm + SM_oFr;
+  const double* rf = sm + SM_oRef;
+  const double* TA = j.TA + (size_t)env * na * nm;
+  const size_t row = j.shared ? (size_t)d : (size_t)env * D + d;
+  for (int k = lane; k < RF_POST + na; k += 32) { /* the references' tangents */
+    const double* p;
+    int nd, i;
+    if (k < RF_FOOT) { p = j.dref[0]; nd = 9; i = k; }
+    else if (k < RF_CONTACT) { p = j.dref[1 + (k - RF_FOOT) / 24]; nd = 24; i = (k - RF_FOOT) % 24; }
+    else if (k < RF_POST) { p = j.dref[3 + (k - RF_CONTACT) / 12]; nd = 12; i = (k - RF_CONTACT) % 12; }
+    else { p = j.dref[5]; nd = na; i = k - RF_POST; }
+    sm[JV_oDRF + k] = (p && i < nd) ? p[row * nd + i] : 0.0;
+  }
+  __syncwarp();
+  {
+    auto T = [&](int k) -> double { return kin ? ds[k].d : 0.0; }; /* tangent of K1's output at sm offset k */
+    const double* dq = sm + JV_oDQV;
+    const double* dvv = sm + JV_oDQV + 32;
+    const double* drf = sm + JV_oDRF;
+    /* the task right-hand sides' tangents (k2_assemble / se3_rhs) */
+    double* bd = sm + JV_oBD;
+    if (lane < 4) {
+      const int f = lane & 1;
+      const bool is_contact = lane < 2;
+      double b6[6] = {0, 0, 0, 0, 0, 0};
+      if (!is_contact || ((mask >> f) & 1)) {
+        const int oref = is_contact ? RF_CONTACT + 12 * f : RF_FOOT + 24 * f;
+        const double* ref = rf + oref;
+        const double* rd = drf + oref;
+        const double* gains = C.kp_contact + (is_contact ? 0 : 12);
+        Dual Rf[9], pf[3], Rr[9], dp[3], E[9], ep[3];
+#pragma unroll
+        for (int k = 0; k < 3; k++) pf[k] = Dual(fr[FR_OMF + 12 * f + k], T(SM_oFr + FR_OMF + 12 * f + k));
+#pragma unroll
+        for (int k = 0; k < 9; k++) Rf[k] = Dual(fr[FR_OMF + 12 * f + 3 + k], T(SM_oFr + FR_OMF + 12 * f + 3 + k));
+#pragma unroll
+        for (int c = 0; c < 3; c++)
+#pragma unroll
+          for (int q = 0; q < 3; q++) Rr[3 * q + c] = Dual(ref[3 + 3 * c + q], rd[3 + 3 * c + q]);
+#pragma unroll
+        for (int k = 0; k < 3; k++) dp[k] = Dual(ref[k], rd[k]) - pf[k];
+#pragma unroll
+        for (int i = 0; i < 3; i++)
+#pragma unroll
+          for (int q = 0; q < 3; q++) E[3 * i + q] = Rf[i] * Rr[q] + Rf[3 + i] * Rr[3 + q] + Rf[6 + i] * Rr[6 + q];
+        mtv3(Rf, dp, ep);
+        const double* JL = sm + JV_oJL + 72 * lane;
+        Dual vl[6], al[6];
+        if (!is_contact) {
+          Dual vr[6], ar[6];
+#pragma unroll
+          for (int k = 0; k < 6; k++) { vr[k] = Dual(ref[12 + k], rd[12 + k]); ar[k] = Dual(ref[18 + k], rd[18 + k]); }
+          mtv3(Rf, vr, vl); mtv3(Rf, vr + 3, vl + 3);
+          mtv3(Rf, ar, al); mtv3(Rf, ar + 3, al + 3);
+        }
+#pragma unroll
+        for (int k = 0; k < 6; k++) {
+          double pe = 0.0;
+#pragma unroll
+          for (int i = 0; i < 9; i++) pe += JL[12 * k + i] * E[i].d;
+#pragma unroll
+          for (int i = 0; i < 3; i++) pe += JL[12 * k + 9 + i] * ep[i].d;
+          const double vF = T(SM_oFr + FR_VF + 6 * f + k), aF = T(SM_oFr + FR_AF + 6 * f + k);
+          b6[k] = gains[k] * pe + gains[6 + k] * ((is_contact ? 0.0 : vl[k].d) - vF) + (is_contact ? 0.0 : al[k].d) - aF;
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < 6; k++) bd[(is_contact ? BV_MOT : BV_FOOT) + 6 * f + k] = b6[k];
+    } else if (lane < 7) {
+      const int r = lane - 4;
+      bd[BV_COM + r] = -C.kp_com[r] * (T(SM_oFr + FR_COM + r) - drf[RF_COM + r]) -
+                       C.kd_com[r] * (T(SM_oFr + FR_COM + 3 + r) - drf[RF_COM + 3 + r]) + drf[RF_COM + 6 + r] -
+                       T(SM_oFr + FR_COM + 6 + r);
+    } else if (lane < 10) {
+      const int r = lane - 7;
+      bd[BV_AM + r] = -C.kp_am[r] * T(SM_oFr + FR_L + r) - T(SM_oFr + FR_L + 3 + r);
+    }
+    if (lane < na)
+      bd[BV_POST + lane] = -mdl[MDL_oPOST + lane] * (dq[7 + lane] - drf[RF_POST + lane]) - mdl[MDL_oPOST + 23 + lane] * dvv[6 + lane];
+    /* [JF; Jcom; Ag]' x_dv, JF' nu_dyn, (M | -Jc^T)' x and nle' of the dynamics rows */
+    const double* nud = sm + JV_oNUD;
+    if (lane < 18) {
+      double s = 0.0;
+      if (kin)
+        for (int k = 0; k < nv; k++) s += ds[SM_oJF + lane * TSIDB_NVX + k].d * x[k];
+      sm[JV_oAD + lane] = s;
+    } else if (lane < 30) {
+      double s = 0.0;
+      if (kin)
+        for (int k = 0; k < nv; k++) s += ds[SM_oJF + (lane - 18) * TSIDB_NVX + k].d * nud[k];
+      sm[JV_oAD + lane] = s;
+    }
+    if (lane < nv) {
+      double s = 0.0;
+      if (kin) {
+        for (int k = 0; k < nv; k++) s += ds[SM_oM + lane * SM_LDM + k].d * x[k];
+        for (int sl = 0; sl < nc; sl++) {
+          const int f = sl == 0 ? f0 : 1;
+          for (int mm = 0; mm < 6; mm++) s -= ds[SM_oJF + (f * 6 + mm) * TSIDB_NVX + lane].d * sm[JV_oPHI + 6 * sl + mm];
+        }
+      }
+      sm[JV_oDD + lane] = s;
+      sm[JV_oDD + 32 + lane] = T(SM_oNle + lane);
+    }
+    __syncwarp();
+    /* r1 into y (xb), -r2 into v (nub) */
+    const double* ad = sm + JV_oAD;
+    const double* bv = sm + SM_oBv;
+    const double* dd = sm + JV_oDD;
+    const double* nuj = sm + JV_oNUJ;
+    double y[QP_SLOTS], v[QP_SLOTS], u[QP_SLOTS];
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int c = lane + 32 * t;
+      double r1 = 0.0;
+      if (c < nv) {
+        double hx = 0.0, gd = 0.0, gt = 0.0;
+        for (int q = 0; q < 18; q++) {
+          const double w = q < 12 ? C.w_foot : (q < 15 ? C.w_com : (C.use_am ? C.w_am : 0.0));
+          const double Jq = JF[q * TSIDB_NVX + c], Jd = T(SM_oJF + q * TSIDB_NVX + c);
+          hx += w * (Jd * sm[JV_oA + q] + Jq * ad[q]);
+          gd += w * (Jd * bv[BV_FOOT + q] + Jq * bd[BV_FOOT + q]);
+        }
+        gd = -gd - (c >= 6 ? C.w_post * bd[BV_POST + c - 6] : 0.0);
+        if (kin) {
+          for (int i = 0; i < nv; i++) gt += nud[i] * ds[SM_oM + i * SM_LDM + c].d;
+          for (int q = 0; q < 12; q++) gt += nuj[q] * ds[SM_oJF + q * TSIDB_NVX + c].d;
+        }
+        r1 = -(hx + gd - gt);
+      } else if (c < nx_e) {
+        const int sl = (c - nv) / 12, k = (c - nv) % 12, f = sl == 0 ? f0 : 1;
+        double s = 0.0;
+        for (int mm = 0; mm < 6; mm++) s += C.T[mm][k] * ad[18 + f * 6 + mm];
+        r1 = -s;
+      }
+      y[t] = r1;
+      double r2 = 0.0;
+      if (c < m) {
+        const int kind = dkind[c], i = didx[c];
+        if (kind == 1) r2 = -dcoef[c] * (dd[i] + dd[32 + i]);
+        else if (kind == 2) r2 = -(ad[i] - bd[BV_MOT + i]);
+        else if (kind == 3) r2 = -dcoef[c] * dvv[i];
+      }
+      v[t] = -r2;
+    }
+    qg_lsolve(L, ld, n, y, lane);
+    qg_kkt_solve(L, M, ld, beta, rdiag, n, m, y, v, u, lane);
+    double* xd = sm + JV_oXD;
+#pragma unroll
+    for (int t = 0; t < QP_SLOTS; t++) {
+      const int c = lane + 32 * t;
+      if (c < nm) {
+        const double val = c < n ? y[t] : 0.0;
+        xd[c] = val;
+        if (j.ox) j.ox[((size_t)env * D + d) * nm + c] = val;
+      }
+    }
+    __syncwarp();
+    if (j.otau && lane < na) {
+      double s = dd[6 + lane] + dd[32 + 6 + lane];
+      for (int k = 0; k < n; k++) s += TA[(size_t)lane * nm + k] * xd[k];
+      j.otau[((size_t)env * D + d) * na + lane] = s;
+    }
+  }
+}
+
+/* K1 in tangent arithmetic seeded with one direction's q and v parts (tq, tv: this lane's component) */
+template <int NV>
+TSIDB_DEVNI void tick_jvp_k1(const DevConst& C, const double* mdl, Dual* ds, const double* sm, double tq, double tv, int lane) {
+  if (lane < NV + 1) ds[SM_oQV + lane] = Dual(sm[SM_oQV + lane], tq);
+  if (lane < NV) ds[SM_oQV + 32 + lane] = Dual(sm[SM_oQV + 32 + lane], tv);
+  __syncwarp();
+  k1_dynamics<NV>(C, mdl, ds, lane);
+}
+
+/* One env of tsidb_tick_jvp: tick_jvp_setup, then per direction its tangents staged, the tangent K1 when the direction
+ * has a q or v part, and tick_jvp_dir. */
+template <int NV>
+TSIDB_DEV void tick_jvp_env(const DevConst& C, const double* mdl, Dual* ds, double* sm, double* qs, const TickArgs& a,
+                            const JvpArgs& j, int env, int lane) {
+  constexpr int nv = NV, na = NV - 6, nq = NV + 1;
+  if (!tick_jvp_setup<NV>(C, mdl, sm, qs, a, j, env, lane)) return;
+  const int D = j.n_dirs;
+#pragma unroll 1
+  for (int d = 0; d < D; d++) {
+    const size_t row = j.shared ? (size_t)d : (size_t)env * D + d;
+    const double tq = (j.dq && lane < nq) ? j.dq[row * nq + lane] : 0.0;
+    const double tv = (j.dv && lane < nv) ? j.dv[row * nv + lane] : 0.0;
+    sm[JV_oDQV + lane] = tq;
+    sm[JV_oDQV + 32 + lane] = tv;
+    const bool kin = __ballot_sync(FULL, tq != 0.0 || tv != 0.0) != 0;
+    if (kin) tick_jvp_k1<NV>(C, mdl, ds, sm, tq, tv, lane);
+    __syncwarp();
+    tick_jvp_dir<NV>(C, mdl, ds, sm, qs, a, j, env, d, kin, lane);
+  }
 }
 
 #ifndef TSIDB_EMU
@@ -3997,6 +4404,26 @@ tsidb_state_grad_kernel(const TickArgs a, const StateGradArgs r) {
   __syncthreads();
   for (int env = blockIdx.x * TSIDB_S_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_S_CTA_WARPS)
     state_grad_env<NV>(C, mdl, sm, sm + 2 * K1_DUAL_SIZE, a, r, env, lane);
+}
+
+/* Forward derivative of export + solve (tsidb_tick_jvp): one warp per env on a persistent grid, the CTA's warps sharing the
+ * staged model table.  Per warp TSIDB_J_PER_WARP(n_max, nin_max) doubles of dynamic shared memory (tick_jvp_env): 101 KB
+ * at the export's strides for robot/v1, so a CTA holds two warps and one CTA runs per SM; the host picks the warps per CTA
+ * (up to TSIDB_J_MAX_WARPS) that fit the call's strides. */
+#define TSIDB_J_MAX_WARPS 2
+template <int NV>
+__global__ void __launch_bounds__(32 * TSIDB_J_MAX_WARPS, 1)
+tsidb_tick_jvp_kernel(const TickArgs a, const JvpArgs j) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, warps = blockDim.x >> 5;
+  const int per_warp = TSIDB_J_PER_WARP(j.n_max, j.nin_max);
+  double* w = smem + (size_t)wid * per_warp;
+  const DevConst& C = g_const[a.slot];
+  double* mdl = smem + (size_t)warps * per_warp;
+  load_table(mdl, a.tables + TBL_oMDL, MDL_SIZE, threadIdx.x, blockDim.x);
+  __syncthreads();
+  for (int env = blockIdx.x * warps + wid; env < a.n_envs; env += gridDim.x * warps)
+    tick_jvp_env<NV>(C, mdl, reinterpret_cast<Dual*>(w), w + JV_DUALS, w + JV_DUALS + JV_SIZE, a, j, env, lane);
 }
 
 /* ---- Small batches: the whole tick of one env in ONE launch ----

@@ -634,6 +634,89 @@ class TsidEngine:
         outs = _TickLayer.apply(self, q, v, contact_mask, keys, *(refs[k] for k in keys))
         return dict(zip(("tau", "dv", "f", "status", "iters"), outs))
 
+    def tick_jvp(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                 refs: Optional[Dict[str, torch.Tensor]] = None, tangents: Optional[Dict[str, torch.Tensor]] = None,
+                 prob: Optional[Dict[str, torch.Tensor]] = None, sol: Optional[Dict[str, torch.Tensor]] = None
+                 ) -> Dict[str, torch.Tensor]:
+        """Forward-mode derivative of :meth:`tick_layer`'s forward pass (tsidb_tick_jvp): for D tangent directions,
+        `tangents` maps "q", "v" and reference names to [N,D,k] (per env) or [D,k] (shared by every env) float64 tensors,
+        all of one kind (an absent name: zero tangent).  Returns new CUDA tensors x [N,D,n_max] (the tangent of the solve's
+        x), tau [N,D,na], dv [N,D,nv] and f [N,D,24] (in the tick's fixed LF/RF slots, as tick_layer maps x) and status
+        [N] int32 (4 with zero tangents where qp_grad would refuse the env).  `prob` (problem_data with TA, ta0) and `sol`
+        (qp_solve on it) are the forward pass; without them the call runs it.  q is differentiated in its raw doubles
+        (the quaternion unnormalised), SE3 references in their raw 12 or 24 doubles.  See INTEGRATION.md, "Linearizing
+        the controller"."""
+        r = self._state_args("tick_jvp", q, v, contact_mask, refs)
+        n = q.shape[0]
+        tangents = dict(tangents or {})
+        dims = dict(self._ref_dims, q=self.nq, v=self.nv)
+        if not tangents or set(tangents) - set(dims):
+            raise ValueError(f"tick_jvp: tangents must name some of {tuple(dims)}, got {sorted(tangents)}")
+        ranks = {t.dim() if isinstance(t, torch.Tensor) else -1 for t in tangents.values()}
+        if ranks - {2, 3} or len(ranks) != 1:
+            raise TypeError("tick_jvp: tangents must all be [N,D,k] (per env) or all [D,k] (shared)")
+        shared = ranks == {2}
+        d = next(iter(tangents.values())).shape[0 if shared else 1]
+        for k, t in tangents.items():
+            want = (d, dims[k]) if shared else (n, d, dims[k])
+            if t.dtype is not torch.float64 or not t.is_cuda or t.get_device() != self._dev_index or not t.is_contiguous() \
+                    or tuple(t.shape) != want or d < 1:
+                raise TypeError(f"tick_jvp: tangents[{k!r}]: expected a contiguous torch.float64 tensor of shape {want} "
+                                f"on the engine's device")
+        if (prob is None) != (sol is None):
+            raise ValueError("tick_jvp: prob and sol go together")
+        if prob is None:
+            prob = self.problem_data(q, v, contact_mask, refs, parts=self.PROBLEM_PARTS + self.ACTUATION_PARTS)
+            sol = self.qp_solve(prob)
+        for k in ("CE", "CI", "TA"):
+            if k not in prob:
+                raise ValueError(f"tick_jvp: prob needs {k}")
+        n_, nx, neq, nin = self._qp_problem("tick_jvp", prob)
+        if n_ != n:
+            raise TypeError(f"tick_jvp: prob has {n_} envs, q has {n}")
+        need = ("x", "status", "active", "lambda", "lambda_eq")
+        if set(need) - set(sol):
+            raise ValueError(f"tick_jvp: sol needs {need}")
+        sol = {k: sol[k] for k in need}
+        self._qp_tensors("tick_jvp", sol, {"x": (n, nx), "status": (n,), "active": (n, nx), "lambda": (n, nx),
+                                           "lambda_eq": (n, neq)})
+        f64 = dict(dtype=torch.float64, device=self.device)
+        out = {"x": torch.empty((n, d, nx), **f64), "tau": torch.empty((n, d, self.na), **f64),
+               "status": torch.empty(n, dtype=torch.int32, device=self.device)}
+        dr = _capi.TsidbRefs(**{k: t.data_ptr() for k, t in tangents.items() if k in REF_KEYS})
+        jd = _capi.TsidbJvpDirs(q=tangents["q"].data_ptr() if "q" in tangents else None,
+                                v=tangents["v"].data_ptr() if "v" in tangents else None, refs=dr)
+        jo = _capi.TsidbJvpOut(x=out["x"].data_ptr(), tau=out["tau"].data_ptr())
+        po = _capi.TsidbProblemOut(**{k: t.data_ptr() for k, t in prob.items()})
+        so = _capi.TsidbQpOut(**{k: t.data_ptr() for k, t in sol.items()})
+        check(self.lib.tsidb_tick_jvp(self.h, n, 0, q.data_ptr(), v.data_ptr(),
+                                      contact_mask.data_ptr() if contact_mask is not None else None, C.byref(r), nx, neq, nin,
+                                      C.byref(po), C.byref(so), d, int(shared), C.byref(jd), C.byref(jo),
+                                      out["status"].data_ptr(), self._stream()), "tsidb_tick_jvp")
+        out["dv"], out["f"] = _TickLayer.split_x(out["x"], contact_mask, self.nv)
+        return out
+
+    def tick_jacobian(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                      refs: Optional[Dict[str, torch.Tensor]] = None, wrt: Tuple[str, ...] = ("q", "v")
+                      ) -> Dict[str, torch.Tensor]:
+        """The Jacobian of :meth:`tick_layer`'s forward pass (not of the fast tick: at degenerate contact-corner ties the
+        two solves can end in different working sets) with respect to the raw doubles of the inputs named in `wrt`, in
+        that order: {"tau": [N,na,K], "dv": [N,nv,K], "f": [N,24,K], "status": [N]}, K the total size of those inputs.
+        One :meth:`tick_jvp` call with shared identity directions."""
+        dims = dict(self._ref_dims, q=self.nq, v=self.nv)
+        wrt = tuple(wrt)
+        if not wrt or set(wrt) - set(dims) or len(set(wrt)) != len(wrt):
+            raise ValueError(f"tick_jacobian: wrt must name distinct inputs among {tuple(dims)}, got {wrt}")
+        K = sum(dims[k] for k in wrt)
+        eye = torch.eye(K, dtype=torch.float64, device=self.device)
+        tangents, c = {}, 0
+        for k in wrt:
+            tangents[k] = eye[:, c:c + dims[k]].contiguous()
+            c += dims[k]
+        o = self.tick_jvp(q, v, contact_mask, refs, tangents)
+        return {"tau": o["tau"].transpose(1, 2).contiguous(), "dv": o["dv"].transpose(1, 2).contiguous(),
+                "f": o["f"].transpose(1, 2).contiguous(), "status": o["status"]}
+
     def ci_row(self, block: int, side: int, i: int) -> int:
         return int(self.lib.tsidb_ci_row(self.h, block, side, i))
 
@@ -722,7 +805,32 @@ class _TickLayer(torch.autograd.Function):
         ctx.engine, ctx.keys = engine, keys
         ctx.mark_non_differentiable(sol["status"], sol["iters"])
         ctx.save_for_backward(q, v, mask, *(sol[k] for k in _TickLayer.SOL), *(prob[k] for k in _TickLayer.PROB), *tensors)
+        ctx.save_for_forward(q, v, mask, *(sol[k] for k in _TickLayer.SOL), *(prob[k] for k in _TickLayer.PROB), *tensors)
         return sol["tau"], x[:, :nv].contiguous(), f, sol["status"], sol["iters"]
+
+    @staticmethod
+    def split_x(x: torch.Tensor, mask: Optional[torch.Tensor], nv: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """x [N,D,n_max] -> dv [N,D,nv], f [N,D,24] in the tick's fixed slots (LF 0..11, RF 12..23), as forward maps x."""
+        n = x.shape[0]
+        lf, rf = (t.unsqueeze(2) for t in _TickLayer._feet(mask, n, x.device))
+        zero = torch.zeros((), dtype=x.dtype, device=x.device)
+        s0, s1 = x[:, :, nv:nv + 12], x[:, :, nv + 12:nv + 24]
+        f = torch.cat([torch.where(lf, s0, zero), torch.where(rf, torch.where(lf, s1, s0), zero)], dim=2)
+        return x[:, :, :nv].contiguous(), f
+
+    @staticmethod
+    def jvp(ctx, _gengine, tq, tv, _gmask, _gkeys, *trefs):
+        """forward mode: tsidb_tick_jvp with one per-env direction, the inputs' tangents (None = zero)."""
+        e, ns, npb = ctx.engine, len(_TickLayer.SOL), len(_TickLayer.PROB)
+        q, v, mask, *rest = ctx.saved_tensors
+        sol, prob, tensors = dict(zip(_TickLayer.SOL, rest[:ns])), dict(zip(_TickLayer.PROB, rest[ns:ns + npb])), rest[ns + npb:]
+        tangents = {k: t for k, t in (("q", tq), ("v", tv)) if t is not None}
+        tangents.update({k: t for k, t in zip(ctx.keys, trefs) if t is not None})
+        if not tangents:
+            return None, None, None, None, None
+        tangents = {k: t.contiguous().unsqueeze(1) for k, t in tangents.items()}
+        o = e.tick_jvp(q, v, mask, dict(zip(ctx.keys, tensors)), tangents, prob, sol)
+        return o["tau"][:, 0], o["dv"][:, 0], o["f"][:, 0], None, None
 
     @staticmethod
     @once_differentiable
