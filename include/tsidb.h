@@ -351,6 +351,40 @@ int tsidb_state_grad(tsidb_handle* h, int n_envs, int layout, const double* q, c
                      const tsidb_refs* refs, int n_max, int neq_max, int nin_max, const tsidb_problem_out* grad, double* dq,
                      double* dv, void* cuda_stream);
 
+/* ---- the controller's gains and weights -------------------------------------------------------------------------------
+ * tsidb_gains holds the task gains and weights of tsidb_conf (same names and meaning), the parameters a caller may change
+ * after tsidb_create (tsid's setKp / setKd / updateTaskWeight) and differentiate.  Every env of a handle uses the same
+ * values.  The field order is the column order of tsidb_gains_grad's output (TSIDB_GAINS_LEN doubles); posture entries
+ * past na are unused. */
+#define TSIDB_GAINS_LEN 84
+typedef struct tsidb_gains {
+  double kp_contact[6], kd_contact[6], kp_foot[6], kd_foot[6], kp_com[3], kd_com[3];
+  double kp_posture[TSIDB_MAX_NA], kd_posture[TSIDB_MAX_NA], kp_am[3];
+  double w_foot, w_com, w_posture, w_am, w_force_reg;
+} tsidb_gains;
+/* the handle's current values (host pointer) */
+int tsidb_get_gains(const tsidb_handle* h, tsidb_gains* out);
+/* replaces them for every later call of the handle (tick, host calls, rollout, problem data and every gradient call).
+ * Synchronises the device.  Refused (< 0, the handle left exactly as it was): a null argument, a non-finite entry,
+ * w_foot, w_com or w_posture <= 0, a w_force_reg that leaves the force block of the Hessian not positive definite, and a
+ * w_am whose sign differs from the handle's (the AM task is on exactly when it was created with w_am > 0).  Gains may
+ * take any finite value.  A CUDA error while the new values are uploaded returns -2 and puts the previous values back. */
+int tsidb_set_gains(tsidb_handle* h, const tsidb_gains* g);
+/* tsidb_gains_grad is the adjoint of tsidb_problem_data with respect to the handle's current gains and weights, per env:
+ * given dH = dL/dH [N][n_max][n_max], dg = dL/dg [N][n_max] and dce0 = dL/dce0 [N][neq_max] (DEVICE arrays in the layout
+ * tsidb_qp_grad writes, with the caller's strides n_max >= and neq_max >= those of tsidb_problem_sizes; NULL counts as
+ * zero), it writes out [N][TSIDB_GAINS_LEN] (in the call's `layout`, columns in tsidb_gains order).  dH is the gradient
+ * with respect to every entry of the full H, so tsidb_qp_grad's lower-triangular gradient composes unchanged.  Gains and
+ * weights enter only H (its dv block and the force blocks of the feet in contact), g (entries 0..nv) and the
+ * contact-motion rows 6..6+6nc of ce0; nothing else is read, so padding, appended variables or rows and every other entry
+ * may hold anything.  Exact zeros: posture columns past na, kp_am and w_am when the AM task is off, the contact gains of a
+ * foot not in contact.  A gain shared by the envs (all of them, as the handle uses them) has as gradient the sum of the
+ * rows.  q, v, contact_mask, refs and `layout` as in tsidb_refs_grad.  No workspace of the handle is used, so the call may
+ * run on any stream.  Asynchronous on cuda_stream. */
+int tsidb_gains_grad(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v, const uint8_t* contact_mask,
+                     const tsidb_refs* refs, int n_max, int neq_max, const double* dH, const double* dg, const double* dce0,
+                     double* out, void* cuda_stream);
+
 /* ---- linearizing the controller: forward-mode derivatives of export + solve ---------------------------------------
  * tsidb_tick_jvp is the forward-mode derivative (Jacobian-vector product) of "tsidb_problem_data, then tsidb_qp_solve":
  * for each env and each of n_dirs tangent directions in (q, v, references) it writes the tangent of the solve's x and of

@@ -109,6 +109,17 @@ class TsidbQpOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("x", "status", "iters", "active", "lambda", "lambda_eq", "tau")]
 
 
+# tsidb_gains (include/tsidb.h): the task gains and weights, field order = column order of tsidb_gains_grad
+GAIN_FIELDS = (("kp_contact", 6), ("kd_contact", 6), ("kp_foot", 6), ("kd_foot", 6), ("kp_com", 3), ("kd_com", 3),
+               ("kp_posture", 23), ("kd_posture", 23), ("kp_am", 3), ("w_foot", 1), ("w_com", 1), ("w_posture", 1),
+               ("w_am", 1), ("w_force_reg", 1))
+GAINS_LEN = sum(k for _, k in GAIN_FIELDS)  # TSIDB_GAINS_LEN
+
+
+class TsidbGains(C.Structure):
+    _fields_ = [(k, C.c_double * n) if n > 1 else (k, C.c_double) for k, n in GAIN_FIELDS]
+
+
 class TsidbRefsOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("com", "foot_lf", "foot_rf", "contact_lf", "contact_rf", "posture")]
 
@@ -295,6 +306,12 @@ def load_library() -> C.CDLL:
     lib.tsidb_tick_jvp.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, ip, C.POINTER(TsidbProblemOut),
                                    C.POINTER(TsidbQpOut), ip, ip, C.POINTER(TsidbJvpDirs), C.POINTER(TsidbJvpOut), vp, vp]
     lib.tsidb_tick_jvp.restype = ip
+    lib.tsidb_get_gains.argtypes = [vp, C.POINTER(TsidbGains)]
+    lib.tsidb_get_gains.restype = ip
+    lib.tsidb_set_gains.argtypes = [vp, C.POINTER(TsidbGains)]
+    lib.tsidb_set_gains.restype = ip
+    lib.tsidb_gains_grad.argtypes = [vp, ip, ip, vp, vp, vp, C.POINTER(TsidbRefs), ip, ip, vp, vp, vp, vp, vp]
+    lib.tsidb_gains_grad.restype = ip
     _LIB = lib
     return lib
 
@@ -312,5 +329,5 @@ EXPORTED_SYMBOLS = [
     "tsidb_gait_reset", "tsidb_gait_state", "tsidb_gait_step", "tsidb_rollout", "tsidb_diagnostics",
     "tsidb_foot_trajectory", "tsidb_footstep_plan", "tsidb_gait_set_plan", "tsidb_debug_terms",
     "tsidb_problem_sizes", "tsidb_problem_data", "tsidb_qp_solve", "tsidb_qp_grad",
-    "tsidb_refs_grad", "tsidb_state_grad", "tsidb_tick_jvp",
+    "tsidb_refs_grad", "tsidb_state_grad", "tsidb_tick_jvp", "tsidb_get_gains", "tsidb_set_gains", "tsidb_gains_grad",
 ]

@@ -36,6 +36,7 @@ static bool g_slot_used[8][TSIDB_MAX_SLOTS]; /* per device */
 struct tsidb_handle {
   int device, slot, max_envs, sm_count;
   DevConst dc;
+  tsidb_conf conf;       /* the conf the handle was created with, its gains and weights as tsidb_set_gains left them */
   int32_t* counter;      /* device, TSIDB_NCOUNTER per chunk ([16..16+TSIDB_NKEY): sizes of the (class, bucket) bins of the class sort): work counters of the active-set ([0],[4],[5]), elimination ([8..10]) and basis ([12..14]) kernels, [1..3] class sizes */
   double* ws;            /* device: solver images, SA_IMAGE doubles per slot */
   double* ws3;           /* device: assembly images, SE_IMAGE doubles per slot */
@@ -176,6 +177,14 @@ static int upload_const(tsidb_handle* h) {
   return 0;
 }
 
+/* the QP export's section of the global table, from h->conf and h->dc */
+static int upload_problem_table(tsidb_handle* h) {
+  double pt[PT_SIZE];
+  tsidb_fill_problem_table(&h->conf, &h->dc, pt);
+  CK(cudaMemcpy(h->tables + TBL_oPROB, pt, sizeof pt, cudaMemcpyHostToDevice));
+  return 0;
+}
+
 /* everything of tsidb_create that can fail after the handle exists; on any failure the caller destroys the handle
  * (tsidb_destroy tolerates members that were never created), which also returns the constant-memory slot */
 static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDeviceProp& prop, int max_envs, int device) {
@@ -207,6 +216,8 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
   TSIDB_ATTR(tsidb_dynamics_kernel<24>, smem, TSIDB_D_CTAS_PER_SM, "dynamics kernel", d_carve);
   TSIDB_ATTR(tsidb_refs_grad_kernel<26>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_refs_grad_kernel<24>, TSIDB_R_SMEM, 1, "references gradient kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_gains_grad_kernel<26>, TSIDB_G_SMEM, 1, "gains gradient kernel", cudaSharedmemCarveoutMaxShared);
+  TSIDB_ATTR(tsidb_gains_grad_kernel<24>, TSIDB_G_SMEM, 1, "gains gradient kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_state_grad_kernel<26>, TSIDB_S_SMEM, 1, "state gradient kernel", cudaSharedmemCarveoutMaxShared);
   TSIDB_ATTR(tsidb_state_grad_kernel<24>, TSIDB_S_SMEM, 1, "state gradient kernel", cudaSharedmemCarveoutMaxShared);
   /* the forward derivative sizes its shared memory from the call's strides, up to all an SM gives one CTA */
@@ -247,10 +258,11 @@ static int create_impl(tsidb_handle* h, const tsidb_conf* conf, const cudaDevice
   CK(cudaMalloc(&h->cls_pos, (size_t)max_envs * sizeof(int32_t)));
   CK(cudaMalloc(&h->tables, TBL_SIZE * sizeof(double)));
   if (upload_const(h) != 0) return -2;
+  if (upload_problem_table(h) != 0) return -2;
   {
-    double pt[PT_SIZE];
-    tsidb_fill_problem_table(conf, &h->dc, pt);
-    CK(cudaMemcpy(h->tables + TBL_oPROB, pt, sizeof pt, cudaMemcpyHostToDevice));
+    double G[12][12];
+    tsidb_force_gram(conf, h->dc.T, G);
+    CK(cudaMemcpy(h->tables + TBL_oFRG, G, sizeof G, cudaMemcpyHostToDevice));
   }
   /* host-call staging: inputs q(nq) v(nv) refs(9+24+24+12+12+na); outputs tau(na) ddq(nv) f(24) */
   const int na = h->dc.na, nv = h->dc.nv, nq = h->dc.nq;
@@ -306,6 +318,7 @@ extern "C" int tsidb_create(const tsidb_model* model, const tsidb_conf* conf, in
   tsidb_handle* h = new tsidb_handle();
   memset((void*)h, 0, sizeof *h);
   h->dc = dc;
+  h->conf = *conf;
   h->device = device;
   h->max_envs = max_envs;
   h->slot = -1;
@@ -380,6 +393,53 @@ extern "C" int tsidb_set_default_refs(tsidb_handle* h, const double* com9, const
   CK(cudaSetDevice(h->device));
   CK(cudaDeviceSynchronize()); /* constants may be in use by a running tick */
   return upload_const(h);
+}
+
+extern "C" int tsidb_get_gains(const tsidb_handle* h, tsidb_gains* out) {
+  if (!h || !out) { g_err = "tsidb_get_gains: null argument"; return -1; }
+  tsidb_gains_of_conf(&h->conf, out);
+  return 0;
+}
+
+/* everything is checked on copies first: a refused call returns -1 and leaves the handle as it was */
+extern "C" int tsidb_set_gains(tsidb_handle* h, const tsidb_gains* g) {
+  if (!h || !g) { g_err = "tsidb_set_gains: null argument"; return -1; }
+  static_assert(sizeof(tsidb_gains) == TSIDB_GAINS_LEN * sizeof(double), "tsidb_gains is TSIDB_GAINS_LEN doubles");
+  const double* p = reinterpret_cast<const double*>(g);
+  for (int k = 0; k < TSIDB_GAINS_LEN; k++)
+    if (!isfinite(p[k])) { g_err = "tsidb_set_gains: entry " + std::to_string(k) + " is not finite"; return -1; }
+  if (!(g->w_foot > 0.0) || !(g->w_com > 0.0) || !(g->w_posture > 0.0)) {
+    g_err = "tsidb_set_gains: w_foot, w_com and w_posture must be > 0";
+    return -1;
+  }
+  if ((g->w_am > 0.0) != (h->dc.use_am != 0)) {
+    g_err = h->dc.use_am ? "tsidb_set_gains: the handle was created with the AM task on: w_am must stay > 0"
+                         : "tsidb_set_gains: the handle was created with the AM task off: w_am must stay <= 0";
+    return -1;
+  }
+  tsidb_conf conf = h->conf;
+  tsidb_gains_to_conf(g, &conf);
+  DevConst dc = h->dc;
+  tsidb_gains_to_devconst(g, &dc);
+  std::string err;
+  if (!tsidb_factor_force_block(&conf, &dc, &err)) { g_err = "tsidb_set_gains: w_force_reg: " + err; return -1; }
+  CK(cudaSetDevice(h->device));
+  CK(cudaDeviceSynchronize()); /* constants may be in use by a running tick */
+  /* a CUDA error during the upload puts the previous values back on the host and uploads them again, so that host and
+   * device agree on them as far as the device still accepts copies */
+  const tsidb_conf old_conf = h->conf;
+  const DevConst old_dc = h->dc;
+  h->conf = conf;
+  h->dc = dc;
+  if (upload_const(h) != 0 || upload_problem_table(h) != 0) {
+    const std::string keep = g_err;
+    h->conf = old_conf;
+    h->dc = old_dc;
+    if (upload_const(h) == 0) upload_problem_table(h);
+    g_err = keep;
+    return -2;
+  }
+  return 0;
 }
 
 /* the dynamics kernel over a.n_envs envs on a persistent grid (kernel D of the tick; also the first stage of the QP export) */
@@ -974,6 +1034,48 @@ extern "C" int tsidb_state_grad(tsidb_handle* h, int n_envs, int layout, const d
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (h->dc.nv == 26) tsidb_state_grad_kernel<26><<<blocks, 32 * TSIDB_S_CTA_WARPS, TSIDB_S_SMEM, st>>>(a, r);
   else tsidb_state_grad_kernel<24><<<blocks, 32 * TSIDB_S_CTA_WARPS, TSIDB_S_SMEM, st>>>(a, r);
+  CK(cudaGetLastError());
+  h->launches += 1;
+  return 0;
+}
+
+/* adjoint of the export in the gains and weights: one launch that recomputes K1 per env, no workspace of the handle */
+extern "C" int tsidb_gains_grad(tsidb_handle* h, int n_envs, int layout, const double* q, const double* v,
+                                const uint8_t* contact_mask, const tsidb_refs* refs, int n_max, int neq_max, const double* dH,
+                                const double* dg, const double* dce0, double* out, void* cuda_stream) {
+  if (!h || !q || !v || !out) { g_err = "tsidb_gains_grad: null argument"; return -1; }
+  if (n_envs <= 0 || n_envs > h->max_envs) { g_err = "tsidb_gains_grad: n_envs must be in [1, max_envs]"; return -1; }
+  if (layout != 0 && layout != 1) { g_err = "tsidb_gains_grad: layout must be 0 ([N][dof]) or 1 ([dof][N])"; return -1; }
+  int nx, neq, nin;
+  problem_maxima(h, &nx, &neq, &nin);
+  if (n_max < nx || neq_max < neq) {
+    g_err = "tsidb_gains_grad: n_max and neq_max must be at least tsidb_problem_sizes' n_max and neq_max";
+    return -1;
+  }
+  for (const void* p : {(const void*)q, (const void*)v, (const void*)dH, (const void*)dg, (const void*)dce0, (const void*)out})
+    if (((uintptr_t)p & 7) != 0) { g_err = "tsidb_gains_grad: fp64 arrays must be 8-byte aligned"; return -1; }
+  CK(cudaSetDevice(h->device));
+  TickArgs a;
+  memset(&a, 0, sizeof a);
+  a.n_envs = n_envs; a.layout = layout;
+  a.q = q; a.v = v; a.mask = contact_mask;
+  if (refs) {
+    a.r_com = refs->com; a.r_foot[0] = refs->foot_lf; a.r_foot[1] = refs->foot_rf;
+    a.r_contact[0] = refs->contact_lf; a.r_contact[1] = refs->contact_rf; a.r_posture = refs->posture;
+  }
+  a.slot = h->slot;
+  a.tables = h->tables;
+  GainsGradArgs r;
+  memset(&r, 0, sizeof r);
+  r.n_max = n_max; r.neq_max = neq_max;
+  r.dH = dH; r.dg = dg; r.dce0 = dce0;
+  r.frg = h->tables + TBL_oFRG;
+  r.out = out;
+  int blocks = (n_envs + TSIDB_G_CTA_WARPS - 1) / TSIDB_G_CTA_WARPS;
+  if (blocks > h->sm_count) blocks = h->sm_count; /* persistent */
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  if (h->dc.nv == 26) tsidb_gains_grad_kernel<26><<<blocks, 32 * TSIDB_G_CTA_WARPS, TSIDB_G_SMEM, st>>>(a, r);
+  else tsidb_gains_grad_kernel<24><<<blocks, 32 * TSIDB_G_CTA_WARPS, TSIDB_G_SMEM, st>>>(a, r);
   CK(cudaGetLastError());
   h->launches += 1;
   return 0;

@@ -166,6 +166,16 @@ struct StateGradArgs {
   double *dq, *dv;
 };
 
+/* arguments of the adjoint of the export in the gains and weights (tsidb_gains_grad): dL/dH [N][n_max][n_max], dL/dg
+ * [N][n_max], dL/dce0 [N][neq_max] with the caller's strides (NULL = zero), the force block's Gram matrix (W T)^T (W T)
+ * (12 x 12, device) and dL/d(gains) [N][TSIDB_GAINS_LEN] in the call's layout */
+struct GainsGradArgs {
+  int32_t n_max, neq_max;
+  const double *dH, *dg, *dce0;
+  const double* frg;
+  double* out;
+};
+
 /* arguments of the forward derivative of export + solve (tsidb_tick_jvp): the export qp and its solution sol as
  * tsidb_qp_grad reads them, n_dirs tangent directions per env ([N][D][k]) or shared by all envs ([D][k]) in q, v and the
  * tsidb_refs arrays com, foot_lf, foot_rf, contact_lf, contact_rf, posture (NULL = zero), and the tangents of x

@@ -11,8 +11,8 @@
 #include "../../include/tsidb.h"
 #include "tsidb_const.h"
 
-/* force block of the Hessian, identical for every env and foot: w_freg (W T)^T (W T) + hreg I */
-static inline void tsidb_force_hessian(const tsidb_conf* c, const double (*T)[12], double (*Hf)[12]) {
+/* Gram matrix of the force regularisation, (W T)^T (W T): the derivative of the force block in w_force_reg */
+static inline void tsidb_force_gram(const tsidb_conf* c, const double (*T)[12], double (*G)[12]) {
   for (int i = 0; i < 12; i++)
     for (int j = 0; j < 12; j++) {
       double s = 0.0;
@@ -20,8 +20,93 @@ static inline void tsidb_force_hessian(const tsidb_conf* c, const double (*T)[12
         const double wr = c->force_reg_weights[r];
         s += (wr * T[r][i]) * (wr * T[r][j]);
       }
-      Hf[i][j] = c->w_force_reg * s + (i == j ? c->hessian_reg : 0.0);
+      G[i][j] = s;
     }
+}
+
+/* force block of the Hessian, identical for every env and foot: w_freg (W T)^T (W T) + hreg I */
+static inline void tsidb_force_hessian(const tsidb_conf* c, const double (*T)[12], double (*Hf)[12]) {
+  double G[12][12];
+  tsidb_force_gram(c, T, G);
+  for (int i = 0; i < 12; i++)
+    for (int j = 0; j < 12; j++) Hf[i][j] = c->w_force_reg * G[i][j] + (i == j ? c->hessian_reg : 0.0);
+}
+
+/* the force block's factor Lf, its inverse and the traces of DevConst from c and D->T (tsidb_create and tsidb_set_gains
+ * both come here, so the two produce the same bits); false, D untouched: the block is not positive definite */
+static inline bool tsidb_factor_force_block(const tsidb_conf* c, DevConst* D, std::string* err) {
+  double Hf[12][12], Lf[12][12], Lfinv[12][12];
+  memset(Lf, 0, sizeof Lf);
+  memset(Lfinv, 0, sizeof Lfinv);
+  tsidb_force_hessian(c, D->T, Hf);
+  double Hf_trace = 0.0;
+  for (int i = 0; i < 12; i++) Hf_trace += Hf[i][i];
+  for (int j = 0; j < 12; j++) {
+    double s = Hf[j][j];
+    for (int k = 0; k < j; k++) s -= Lf[j][k] * Lf[j][k];
+    if (!(s > 0.0)) { *err = "conf: force block of the Hessian is not positive definite"; return false; }
+    Lf[j][j] = sqrt(s);
+    for (int i = j + 1; i < 12; i++) {
+      double t = Hf[i][j];
+      for (int k = 0; k < j; k++) t -= Lf[i][k] * Lf[j][k];
+      Lf[i][j] = t / Lf[j][j];
+    }
+  }
+  /* inverse of the lower factor, column by column */
+  for (int cidx = 0; cidx < 12; cidx++)
+    for (int i = 0; i < 12; i++) {
+      double s = (i == cidx) ? 1.0 : 0.0;
+      for (int k = 0; k < i; k++) s -= Lf[i][k] * Lfinv[k][cidx];
+      Lfinv[i][cidx] = s / Lf[i][i];
+    }
+  double Lfinv_trace = 0.0;
+  for (int i = 0; i < 12; i++) Lfinv_trace += Lfinv[i][i];
+  memcpy(D->Lf, Lf, sizeof Lf);
+  memcpy(D->Lfinv, Lfinv, sizeof Lfinv);
+  D->Hf_trace = Hf_trace;
+  D->Lfinv_trace = Lfinv_trace;
+  return true;
+}
+
+/* tsidb_gains <-> the gain and weight fields of tsidb_conf and DevConst */
+static inline void tsidb_gains_of_conf(const tsidb_conf* c, tsidb_gains* g) {
+  memcpy(g->kp_contact, c->kp_contact, sizeof g->kp_contact);
+  memcpy(g->kd_contact, c->kd_contact, sizeof g->kd_contact);
+  memcpy(g->kp_foot, c->kp_foot, sizeof g->kp_foot);
+  memcpy(g->kd_foot, c->kd_foot, sizeof g->kd_foot);
+  memcpy(g->kp_com, c->kp_com, sizeof g->kp_com);
+  memcpy(g->kd_com, c->kd_com, sizeof g->kd_com);
+  memcpy(g->kp_posture, c->kp_posture, sizeof g->kp_posture);
+  memcpy(g->kd_posture, c->kd_posture, sizeof g->kd_posture);
+  memcpy(g->kp_am, c->kp_am, sizeof g->kp_am);
+  g->w_foot = c->w_foot; g->w_com = c->w_com; g->w_posture = c->w_posture; g->w_am = c->w_am;
+  g->w_force_reg = c->w_force_reg;
+}
+static inline void tsidb_gains_to_conf(const tsidb_gains* g, tsidb_conf* c) {
+  memcpy(c->kp_contact, g->kp_contact, sizeof g->kp_contact);
+  memcpy(c->kd_contact, g->kd_contact, sizeof g->kd_contact);
+  memcpy(c->kp_foot, g->kp_foot, sizeof g->kp_foot);
+  memcpy(c->kd_foot, g->kd_foot, sizeof g->kd_foot);
+  memcpy(c->kp_com, g->kp_com, sizeof g->kp_com);
+  memcpy(c->kd_com, g->kd_com, sizeof g->kd_com);
+  memcpy(c->kp_posture, g->kp_posture, sizeof g->kp_posture);
+  memcpy(c->kd_posture, g->kd_posture, sizeof g->kd_posture);
+  memcpy(c->kp_am, g->kp_am, sizeof g->kp_am);
+  c->w_foot = g->w_foot; c->w_com = g->w_com; c->w_posture = g->w_posture; c->w_am = g->w_am;
+  c->w_force_reg = g->w_force_reg;
+}
+static inline void tsidb_gains_to_devconst(const tsidb_gains* g, DevConst* D) {
+  memcpy(D->kp_contact, g->kp_contact, sizeof D->kp_contact);
+  memcpy(D->kd_contact, g->kd_contact, sizeof D->kd_contact);
+  memcpy(D->kp_foot, g->kp_foot, sizeof D->kp_foot);
+  memcpy(D->kd_foot, g->kd_foot, sizeof D->kd_foot);
+  memcpy(D->kp_com, g->kp_com, sizeof D->kp_com);
+  memcpy(D->kd_com, g->kd_com, sizeof D->kd_com);
+  memcpy(D->kp_post, g->kp_posture, sizeof D->kp_post);
+  memcpy(D->kd_post, g->kd_posture, sizeof D->kd_post);
+  memcpy(D->kp_am, g->kp_am, sizeof D->kp_am);
+  D->w_foot = g->w_foot; D->w_com = g->w_com; D->w_post = g->w_posture; D->w_am = g->w_am;
+  D->w_freg = g->w_force_reg;
 }
 
 static inline bool tsidb_fill_devconst(const tsidb_model* m, const tsidb_conf* c, DevConst* D, std::string* err) {
@@ -118,30 +203,7 @@ static inline bool tsidb_fill_devconst(const tsidb_model* m, const tsidb_conf* c
   D->nin_ref_fixed = 2 * ((D->use_tb ? D->na : 0) + (D->use_jb ? D->nv : 0));
 
   /* force block of the Hessian and its factor (identical for all envs and feet) */
-  double Hf[12][12];
-  tsidb_force_hessian(c, D->T, Hf);
-  D->Hf_trace = 0.0;
-  for (int i = 0; i < 12; i++) D->Hf_trace += Hf[i][i];
-  for (int j = 0; j < 12; j++) {
-    double s = Hf[j][j];
-    for (int k = 0; k < j; k++) s -= D->Lf[j][k] * D->Lf[j][k];
-    if (!(s > 0.0)) { *err = "conf: force block of the Hessian is not positive definite"; return false; }
-    D->Lf[j][j] = sqrt(s);
-    for (int i = j + 1; i < 12; i++) {
-      double t = Hf[i][j];
-      for (int k = 0; k < j; k++) t -= D->Lf[i][k] * D->Lf[j][k];
-      D->Lf[i][j] = t / D->Lf[j][j];
-    }
-  }
-  /* inverse of the lower factor, column by column */
-  for (int cidx = 0; cidx < 12; cidx++)
-    for (int i = 0; i < 12; i++) {
-      double s = (i == cidx) ? 1.0 : 0.0;
-      for (int k = 0; k < i; k++) s -= D->Lf[i][k] * D->Lfinv[k][cidx];
-      D->Lfinv[i][cidx] = s / D->Lf[i][i];
-    }
-  D->Lfinv_trace = 0.0;
-  for (int i = 0; i < 12; i++) D->Lfinv_trace += D->Lfinv[i][i];
+  if (!tsidb_factor_force_block(c, D, err)) return false;
   /* neutral default references */
   for (int f = 0; f < 2; f++) {
     D->ref_foot[f][3] = D->ref_foot[f][7] = D->ref_foot[f][11] = 1.0;

@@ -240,7 +240,8 @@ TSIDB_DEV void stage_model(const DevConst& C, double* mdl, int tid, int nthreads
 #define TBL_oLF ((MDL_SIZE + 1) & ~1)
 #define TBL_oLANE (TBL_oLF + 144)   /* LaneConst of the 32 lanes, value j of lane l at [j][l]: 19 x 32 */
 #define TBL_oPROB (TBL_oLANE + 19 * 32)   /* constants of the QP export (PT_*, tsidb_const.h), filled on the host */
-#define TBL_SIZE (TBL_oPROB + PT_SIZE)
+#define TBL_oFRG (TBL_oPROB + PT_SIZE)   /* Gram matrix of the force regularisation (W T)^T (W T), 12 x 12 (tsidb_gains_grad) */
+#define TBL_SIZE (TBL_oFRG + 144)
 TSIDB_DEV void load_table(double* dst, const double* src, int count /* even */, int tid, int nthreads) {
   const double2* s2 = reinterpret_cast<const double2*>(src);
   double2* d2 = reinterpret_cast<double2*>(dst);
@@ -688,7 +689,9 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, T* sm, int lane
 }
 
 /* ================================================================= K2: assembly */
-/* tsid::TaskSE3Equality::compute in the local frame: b = Kp log6(oMf^-1 Mref) + Kd (R^T vref - v) + R^T aref - drift */
+/* tsid::TaskSE3Equality::compute in the local frame: b = Kp log6(oMf^-1 Mref) + Kd (R^T vref - v) + R^T aref - drift.
+ * The adjoints restate its error E = Rf^T R_ref, ep = Rf^T (p_ref - p_f) (refs_adjoint_env, state_adjoint_env) and
+ * gains_adjoint_env the whole law, so that the tick's kernels stay untouched: a change here goes there too. */
 TSIDB_DEV void se3_rhs(const double* fr, int f, const double* kp, const double* kd, const double* ref12,
                        const double* vref, const double* aref, double* b6) {
   const double* pf = fr + FR_OMF + f * 12;
@@ -2735,6 +2738,198 @@ TSIDB_DEV void refs_grad_env(const DevConst& C, const double* mdl, double* sm, c
   refs_adjoint_env<NV>(C, mdl, sm, a, r, env, lane, mask);
 }
 
+/* ================================================================= adjoint of the export in the gains (tsidb_gains_grad) */
+/* dL/d(gains and weights) of one env after K1 (frames, JF, Jcom, Ag in shared memory; references staged), in tsidb_gains
+ * order (TSIDB_GAINS_LEN).  The gains and weights enter
+ *   H_dv  = w_foot JF^T JF + w_com Jcom^T Jcom + w_post S^T S (+ w_am Ag^T Ag) + hreg I,
+ *   H_ff  = w_freg G + hreg I per foot in contact (G = (W T)^T (W T), r.frg),
+ *   g_dv  = -(w_foot JF^T b_foot + w_com Jcom^T b_com + w_post S^T b_post + w_am Ag^T b_am),  ce0[6 + 6s + k] = -b_mot,
+ * so with y_r = J_r gb:  wb = <Hb, J^T J> - sum_r b_r y_r,  bb = -w y (bb_post = -w_post gb[6:], bb_mot = -ce0b), and the
+ * gradient of each gain is bb times the term it multiplies in the task law.  <Hb, J_r^T J_r> = J_r Hb J_r^T: lane j forms
+ * column j of J Hb from the rows of Hb (coalesced) and the warp reduces.  Lanes 0..3: the SE3 laws (contact LF, contact
+ * RF, foot LF, foot RF), 4..6: CoM, 7..9: AM, lanes < na: posture. */
+template <int NV>
+TSIDB_DEV void gains_adjoint_env(const DevConst& C, const double* mdl, double* sm, const TickArgs& a, const GainsGradArgs& r,
+                                 int env, int lane, int mask) {
+  constexpr int nv = NV, na = NV - 6;
+  const int nc = (mask & 1) + ((mask >> 1) & 1);
+  const int f0 = (mask & 1) ? 0 : 1; /* foot of contact slot 0; slot 1 is RF */
+  const size_t nx = (size_t)r.n_max;
+  const double* Hb = r.dH ? r.dH + (size_t)env * nx * nx : nullptr;
+  const double* JF = sm + SM_oJF;
+  const double* Jcom = sm + SM_oJcom;
+  const double* Ag = sm + SM_oAg;
+  const double* fr = sm + SM_oFr;
+  const double* rf = sm + SM_oRef;
+  const double* qs = sm + SM_oQV;
+  const double* vs = sm + SM_oQV + 32;
+  double* gb = sm + SM_oBv;      /* dL/dg_dv at [0, nv), y = J gb at [32, 50): foot 12, CoM 3, AM 3 */
+  double* res = sm + SM_oM;      /* the gradient in tsidb_gains order; K1's scratch region is dead after K1 */
+  double* part = sm + SM_oM + 96; /* lane l < 4 of the SE3 laws: its kp and kd terms at [12 l, 12 l + 12) */
+  if (lane < nv) gb[lane] = r.dg ? r.dg[(size_t)env * nx + lane] : 0.0;
+  __syncwarp();
+  if (lane < 18) {
+    const double* A = lane < 12 ? JF + lane * TSIDB_NVX : (lane < 15 ? Jcom + (lane - 12) * TSIDB_NVX : Ag + (lane - 15) * TSIDB_NVX);
+    double acc = 0.0;
+    if (lane < 15 || C.use_am) {
+#pragma unroll 2
+      for (int j = 0; j < nv; j++) acc += A[j] * gb[j];
+    }
+    gb[32 + lane] = acc;
+  }
+  /* <Hb, J^T J> of the foot, CoM and AM tasks, the posture's sum of Hb_jj (j >= 6) and <Hb_ff, G> of the feet in contact */
+  double hf = 0.0, hc = 0.0, ha = 0.0, hp = 0.0, hr = 0.0;
+  if (Hb && lane < nv) {
+    const int j = lane;
+    double uf[12], uc[3], ua[3];
+#pragma unroll
+    for (int q = 0; q < 12; q++) uf[q] = 0.0;
+#pragma unroll
+    for (int q = 0; q < 3; q++) { uc[q] = 0.0; ua[q] = 0.0; }
+#pragma unroll 1
+    for (int i = 0; i < nv; i++) {
+      const double h = Hb[i * nx + j];
+#pragma unroll
+      for (int q = 0; q < 12; q++) uf[q] += JF[q * TSIDB_NVX + i] * h;
+#pragma unroll
+      for (int q = 0; q < 3; q++) uc[q] += Jcom[q * TSIDB_NVX + i] * h;
+      if (C.use_am) {
+#pragma unroll
+        for (int q = 0; q < 3; q++) ua[q] += Ag[q * TSIDB_NVX + i] * h;
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < 12; q++) hf += uf[q] * JF[q * TSIDB_NVX + j];
+#pragma unroll
+    for (int q = 0; q < 3; q++) hc += uc[q] * Jcom[q * TSIDB_NVX + j];
+    if (C.use_am) {
+#pragma unroll
+      for (int q = 0; q < 3; q++) ha += ua[q] * Ag[q * TSIDB_NVX + j];
+    }
+    if (j >= 6) hp = Hb[j * nx + j];
+    if (j < 12)
+      for (int s = 0; s < nc; s++) {
+        const double* blk = Hb + (nv + 12 * s) * (nx + 1);
+#pragma unroll 4
+        for (int i = 0; i < 12; i++) hr += blk[i * nx + j] * r.frg[i * 12 + j];
+      }
+  }
+  __syncwarp();
+  const double* y = gb + 32;
+  double wf = 0.0, wc = 0.0, wa = 0.0, wp = 0.0; /* - b_r y_r of the foot, CoM, AM and posture tasks */
+  if (lane < 4) {
+    const int f = lane & 1;
+    const bool is_contact = lane < 2;
+    double kpb[6], kdb[6];
+#pragma unroll
+    for (int k = 0; k < 6; k++) { kpb[k] = 0.0; kdb[k] = 0.0; }
+    if (!is_contact || ((mask >> f) & 1)) { /* a contact not in contact: exact zeros */
+      /* se3_rhs's law, restated with its intermediate terms kept (log6 pe, velocity error ve), which the gains'
+       * gradients multiply; se3_rhs itself stays as the tick's kernels compile it.  The two must stay in step. */
+      const double* gains = C.kp_contact + (is_contact ? 0 : 12);
+      const double* ref = is_contact ? rf + RF_CONTACT + 12 * f : rf + RF_FOOT + 24 * f;
+      const double* pf = fr + FR_OMF + f * 12;
+      const double* Rf = pf + 3;
+      const double* vF = fr + FR_VF + f * 6;
+      const double* aF = fr + FR_AF + f * 6;
+      double Rr[9], dp[3], E[9], ep[3], pe[6];
+#pragma unroll
+      for (int c = 0; c < 3; c++)
+#pragma unroll
+        for (int q = 0; q < 3; q++) Rr[3 * q + c] = ref[3 + 3 * c + q];
+      dp[0] = ref[0] - pf[0]; dp[1] = ref[1] - pf[1]; dp[2] = ref[2] - pf[2];
+#pragma unroll
+      for (int i = 0; i < 3; i++)
+#pragma unroll
+        for (int q = 0; q < 3; q++) E[3 * i + q] = Rf[i] * Rr[q] + Rf[3 + i] * Rr[3 + q] + Rf[6 + i] * Rr[6 + q];
+      mtv3(Rf, dp, ep);
+      log6_dev(E, ep, pe);
+      double ve[6], bb[6]; /* velocity error Rf^T v_ref - v_F (v_ref = 0 for a contact), bb = dL/db */
+      if (is_contact) {
+        const int row = 6 + 6 * ((f == f0) ? 0 : 1);
+#pragma unroll
+        for (int k = 0; k < 6; k++) {
+          ve[k] = -vF[k];
+          bb[k] = r.dce0 ? -r.dce0[(size_t)env * r.neq_max + row + k] : 0.0;
+        }
+      } else {
+        double vl[3], va[3], al[3], aa[3];
+        mtv3(Rf, ref + 12, vl); mtv3(Rf, ref + 15, va);
+        mtv3(Rf, ref + 18, al); mtv3(Rf, ref + 21, aa);
+#pragma unroll
+        for (int k = 0; k < 3; k++) { ve[k] = vl[k] - vF[k]; ve[3 + k] = va[k] - vF[3 + k]; }
+#pragma unroll
+        for (int k = 0; k < 6; k++) {
+          bb[k] = -C.w_foot * y[6 * f + k];
+          const double b = (gains[k] * pe[k] + gains[6 + k] * ve[k] + (k < 3 ? al[k] : aa[k - 3])) - aF[k]; /* se3_rhs */
+          wf -= b * y[6 * f + k];
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < 6; k++) { kpb[k] = bb[k] * pe[k]; kdb[k] = bb[k] * ve[k]; }
+    }
+#pragma unroll
+    for (int k = 0; k < 6; k++) { part[12 * lane + k] = kpb[k]; part[12 * lane + 6 + k] = kdb[k]; }
+  } else if (lane < 7) { /* CoM: b = -Kp (c - c_ref) - Kd (vc - vc_ref) + ac_ref - drift */
+    const int q = lane - 4;
+    const double e = fr[FR_COM + q] - rf[RF_COM + q], ed = fr[FR_COM + 3 + q] - rf[RF_COM + 3 + q];
+    const double bb = -C.w_com * y[12 + q];
+    res[24 + q] = -bb * e;
+    res[27 + q] = -bb * ed;
+    const double b = (-C.kp_com[q] * e - C.kd_com[q] * ed + rf[RF_COM + 6 + q]) - fr[FR_COM + 6 + q];
+    wc = -b * y[12 + q];
+  } else if (lane < 10) { /* legacy AM: b = -Kp L - drift */
+    const int q = lane - 7;
+    double g = 0.0;
+    if (C.use_am) {
+      const double bb = -C.w_am * y[15 + q];
+      g = -bb * fr[FR_L + q];
+      wa = (C.kp_am[q] * fr[FR_L + q] + fr[FR_L + 3 + q]) * y[15 + q];
+    }
+    res[76 + q] = g;
+  }
+  if (lane < 23) { /* posture: b = -Kp (q_j - q_ref) - Kd v_j; columns past na are exact zeros */
+    double gp = 0.0, gd = 0.0;
+    if (lane < na) {
+      const double e = qs[7 + lane] - rf[RF_POST + lane], gj = gb[6 + lane];
+      const double bb = -C.w_post * gj;
+      gp = -bb * e;
+      gd = -bb * vs[6 + lane];
+      wp = (mdl[MDL_oPOST + lane] * e + mdl[MDL_oPOST + 23 + lane] * vs[6 + lane]) * gj;
+    }
+    res[30 + lane] = gp;
+    res[53 + lane] = gd;
+  }
+  const double sf = warp_sum(hf + wf), sc = warp_sum(hc + wc), sa = warp_sum(ha + wa), sp = warp_sum(hp + wp);
+  const double sr = warp_sum(hr);
+  __syncwarp();
+  if (lane < 24) { /* both contacts share kp_contact / kd_contact, both feet kp_foot / kd_foot */
+    const int o = lane + (lane >= 12 ? 12 : 0);
+    res[lane] = part[o] + part[o + 12];
+  } else if (lane == 24) {
+    res[79] = sf; res[80] = sc; res[81] = sp; res[82] = C.use_am ? sa : 0.0; res[83] = sr;
+  }
+  __syncwarp();
+  for (int k = lane; k < TSIDB_GAINS_LEN; k += 32) r.out[eidx(a, env, k, TSIDB_GAINS_LEN)] = res[k];
+}
+
+/* one env of tsidb_gains_grad: q, v and the references staged as the dynamics kernel stages them, K1, then the adjoint.
+ * Nothing is written to the handle's images. */
+template <int NV>
+TSIDB_DEV void gains_grad_env(const DevConst& C, const double* mdl, double* sm, const TickArgs& a, const GainsGradArgs& r,
+                              int env, int lane) {
+  constexpr int nv = NV, na = NV - 6, nq = NV + 1;
+  __syncwarp(); /* every lane is done with the previous env's shared memory */
+  if (lane < nq) sm[SM_oQV + lane] = ldin(a.q, a, env, lane, nq);
+  if (lane < nv) sm[SM_oQV + 32 + lane] = ldin(a.v, a, env, lane, nv);
+  stage_refs(C, mdl, sm, a, env, lane, na);
+  __syncwarp();
+  k1_dynamics<NV>(C, mdl, sm, lane);
+  stage_refs_wait();
+  const int mask = a.mask ? (a.mask[env] & 3) : 3;
+  gains_adjoint_env<NV>(C, mdl, sm, a, r, env, lane, mask);
+}
+
 /* ================================================================= adjoint of the export in q and v (tsidb_state_grad) */
 /* Stage 1 of one env, after K1 and K2 ran on this env in `sm`: the cotangent of the export (the parts of r, NULL = zero)
  * pulled back onto K1's outputs.  It lands in `cb` at K1's own offsets (M, JF, Jcom, Ag, nle, frames; zero where the
@@ -4382,6 +4577,24 @@ tsidb_refs_grad_kernel(const TickArgs a, const RefsGradArgs r) {
   __syncthreads();
   for (int env = blockIdx.x * TSIDB_R_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_R_CTA_WARPS)
     refs_grad_env<NV>(C, mdl, sm, a, r, env, lane);
+}
+
+/* Adjoint of the export in the gains and weights (tsidb_gains_grad): shaped like the references' adjoint, one warp per
+ * env on a persistent grid, 12-warp CTAs sharing the staged model table, one CTA per SM. */
+#define TSIDB_G_CTA_WARPS 12
+#define TSIDB_G_SMEM (((size_t)TSIDB_G_CTA_WARPS * SM_PER_ENV + MDL_SIZE) * sizeof(double))
+template <int NV>
+__global__ void __launch_bounds__(32 * TSIDB_G_CTA_WARPS, 1)
+tsidb_gains_grad_kernel(const TickArgs a, const GainsGradArgs r) {
+  extern __shared__ double smem[];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  double* sm = smem + wid * SM_PER_ENV;
+  const DevConst& C = g_const[a.slot];
+  double* mdl = smem + TSIDB_G_CTA_WARPS * SM_PER_ENV;
+  load_table(mdl, a.tables + TBL_oMDL, MDL_SIZE, threadIdx.x, blockDim.x);
+  __syncthreads();
+  for (int env = blockIdx.x * TSIDB_G_CTA_WARPS + wid; env < a.n_envs; env += gridDim.x * TSIDB_G_CTA_WARPS)
+    gains_grad_env<NV>(C, mdl, sm, a, r, env, lane);
 }
 
 /* Adjoint of the export in q and v (tsidb_state_grad): one warp per env on a persistent grid, the CTA's warps sharing the

@@ -51,6 +51,8 @@ class TsidEngine:
         check(self.lib.tsidb_create(C.byref(self.cm), C.byref(self.cc), self.max_envs, device, C.byref(h)), "tsidb_create")
         self.h = h
         self._out_cache: Dict[int, dict] = {}
+        self._gains_version = 0  # bumped by every set_gains(); tick_layer's backward checks it
+        self._gain_dims = tuple((k, model.na if k in ("kp_posture", "kd_posture") else n) for k, n in _capi.GAIN_FIELDS)
 
     def close(self) -> None:
         if getattr(self, "h", None):
@@ -616,8 +618,88 @@ class TsidEngine:
                                         out["v"].data_ptr() if "v" in out else None, self._stream()), "tsidb_state_grad")
         return out
 
+    GAIN_NAMES = tuple(k for k, _ in _capi.GAIN_FIELDS)
+
+    def gains(self) -> Dict[str, torch.Tensor]:
+        """The handle's task gains and weights (tsidb_get_gains): {name: float64 tensor [k]} on the engine's device, k = 6,
+        3 or na for the gains and 1 for each weight; names as in tsidb_conf (GAIN_NAMES)."""
+        g = _capi.TsidbGains()
+        check(self.lib.tsidb_get_gains(self.h, C.byref(g)), "tsidb_get_gains")
+        flat = np.frombuffer(bytes(g), dtype=np.float64)
+        out, c = {}, 0
+        for (k, n), (_, kk) in zip(_capi.GAIN_FIELDS, self._gain_dims):
+            out[k] = torch.tensor(flat[c:c + kk], dtype=torch.float64, device=self.device)
+            c += n
+        return out
+
+    def set_gains(self, gains: Dict[str, object]) -> None:
+        """Replaces some of the task gains and weights for every later call (tsidb_set_gains, tsid's setKp / setKd /
+        updateTaskWeight): `gains` maps names of :meth:`gains` to values of its shapes (tensors or array-likes); an absent
+        name keeps its value.  Synchronises the device.  Raises TsidbError, the handle unchanged, on a non-finite value,
+        w_foot, w_com or w_posture <= 0, a w_force_reg that leaves the force block not positive definite, or a w_am that
+        would switch the AM task on or off.  Values equal bit for bit to the current ones are a no-op: no library call, no
+        device synchronisation, and the gains version that tick_layer's backward pass checks stays as it is."""
+        unknown = set(gains) - set(self.GAIN_NAMES)
+        if unknown:
+            raise ValueError(f"set_gains: unknown names {sorted(unknown)}; choose from {self.GAIN_NAMES}")
+        g = _capi.TsidbGains()
+        check(self.lib.tsidb_get_gains(self.h, C.byref(g)), "tsidb_get_gains")
+        current = bytes(g)
+        dims = dict(self._gain_dims)
+        for k, val in gains.items():
+            if isinstance(val, torch.Tensor):
+                val = val.detach().to("cpu", torch.float64).numpy()
+            a = np.asarray(val, dtype=np.float64).reshape(-1)
+            if a.shape != (dims[k],):
+                raise ValueError(f"set_gains: {k}: expected {dims[k]} values, got {a.size}")
+            if dims[k] == 1 and k.startswith("w_"):
+                setattr(g, k, float(a[0]))
+            else:
+                field = getattr(g, k)
+                for i, x in enumerate(a):
+                    field[i] = float(x)
+        if bytes(g) == current:
+            return
+        check(self.lib.tsidb_set_gains(self.h, C.byref(g)), "tsidb_set_gains")
+        self._gains_version += 1
+
+    def gains_grad(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
+                   refs: Optional[Dict[str, torch.Tensor]] = None, grads: Optional[Dict[str, torch.Tensor]] = None,
+                   parts: Optional[Tuple[str, ...]] = None) -> Dict[str, torch.Tensor]:
+        """Adjoint of :meth:`problem_data` with respect to the handle's current gains and weights (tsidb_gains_grad), per
+        env: from `grads`, the dict :meth:`qp_grad` returns (H, g and ce0 are read, absent = zero; every other entry is
+        ignored), new CUDA tensors {name: [N,k]} for the names in `parts` (default: all of GAIN_NAMES), shapes as
+        :meth:`gains` with a leading env axis.  A gain every env shares has as gradient the sum over envs.  q, v,
+        contact_mask and refs as in :meth:`problem_data`.  See INTEGRATION.md, "Differentiating with respect to the gains
+        and weights"."""
+        r = self._state_args("gains_grad", q, v, contact_mask, refs)
+        n = q.shape[0]
+        parts = self.GAIN_NAMES if parts is None else tuple(parts)
+        if set(parts) - set(self.GAIN_NAMES):
+            raise ValueError(f"gains_grad: unknown names {sorted(set(parts) - set(self.GAIN_NAMES))}")
+        grads = {k: t for k, t in (grads or {}).items() if k in ("H", "g", "ce0")}
+        nx0, neq0, _ = self.problem_sizes()
+        nx = grads["g"].shape[-1] if "g" in grads else (grads["H"].shape[-1] if "H" in grads else nx0)
+        neq = grads["ce0"].shape[-1] if "ce0" in grads else neq0
+        if nx < nx0 or neq < neq0:
+            raise TypeError(f"gains_grad: strides ({nx}, {neq}) below problem_sizes() ({nx0}, {neq0})")
+        self._qp_tensors("gains_grad", grads, {"H": (n, nx, nx), "g": (n, nx), "ce0": (n, neq)})
+        out = torch.empty((n, _capi.GAINS_LEN), dtype=torch.float64, device=self.device)
+        ptr = {k: (t.data_ptr() if k in grads else None) for k, t in (("H", grads.get("H")), ("g", grads.get("g")),
+                                                                      ("ce0", grads.get("ce0")))}
+        check(self.lib.tsidb_gains_grad(self.h, n, 0, q.data_ptr(), v.data_ptr(),
+                                        contact_mask.data_ptr() if contact_mask is not None else None, C.byref(r), nx, neq,
+                                        ptr["H"], ptr["g"], ptr["ce0"], out.data_ptr(), self._stream()), "tsidb_gains_grad")
+        res, c = {}, 0
+        for (k, nfield), (_, kk) in zip(_capi.GAIN_FIELDS, self._gain_dims):
+            if k in parts:
+                res[k] = out[:, c:c + kk].contiguous()
+            c += nfield
+        return res
+
     def tick_layer(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
-                   refs: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
+                   refs: Optional[Dict[str, torch.Tensor]] = None,
+                   gains: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
         """A tick as a differentiable function of its state and references: {tau [N,na], dv [N,nv], f [N,24], status,
         iters [N] int32}, with tau, dv and f carrying a grad_fn for q, v and every tensor of `refs` that requires grad
         (first order only).
@@ -628,10 +710,23 @@ class TsidEngine:
         costs time: about 74 ms for the forward pass at 65536 walking envs against 3 ms for a tick.  An env whose solve or
         adjoint status is not 0 contributes zero.  When q or v requires grad, the backward pass asks :meth:`qp_grad` for
         every part and adds :meth:`state_grad` (q in its raw doubles, the quaternion unnormalised); otherwise it makes
-        the same calls as for references alone.  contact_mask gets no gradient."""
+        the same calls as for references alone.  contact_mask gets no gradient.
+        `gains` maps names of :meth:`gains` to tensors of its shapes: the forward pass first applies them as
+        :meth:`set_gains` does (which synchronises), and when any of them requires grad the backward pass also asks
+        qp_grad for H and adds :meth:`gains_grad`, summed over the envs.  The backward pass raises if set_gains changed
+        the gains after the forward pass (its gradients would be those of other gains); calls that pass the same values,
+        such as the ticks of one closed loop, leave each other's backward passes valid."""
         self._state_args("tick_layer", q, v, contact_mask, refs)
         keys = tuple(k for k in REF_KEYS if refs and refs.get(k) is not None)
-        outs = _TickLayer.apply(self, q, v, contact_mask, keys, *(refs[k] for k in keys))
+        gains = dict(gains or {})
+        dims = dict(self._gain_dims)
+        for k, t in gains.items():
+            if k not in dims:
+                raise ValueError(f"tick_layer: unknown gain {k!r}; choose from {self.GAIN_NAMES}")
+            if not isinstance(t, torch.Tensor) or t.dtype is not torch.float64 or tuple(t.shape) != (dims[k],):
+                raise TypeError(f"tick_layer: gains[{k!r}]: expected a torch.float64 tensor of shape ({dims[k]},)")
+        gkeys = tuple(k for k in self.GAIN_NAMES if k in gains)
+        outs = _TickLayer.apply(self, q, v, contact_mask, keys, gkeys, *(refs[k] for k in keys), *(gains[k] for k in gkeys))
         return dict(zip(("tau", "dv", "f", "status", "iters"), outs))
 
     def tick_jvp(self, q: torch.Tensor, v: torch.Tensor, contact_mask: Optional[torch.Tensor] = None,
@@ -792,7 +887,11 @@ class _TickLayer(torch.autograd.Function):
         return (m & 1) != 0, (m & 2) != 0
 
     @staticmethod
-    def forward(ctx, engine, q, v, mask, keys, *tensors):
+    def forward(ctx, engine, q, v, mask, keys, gkeys, *tensors):
+        tensors, gtensors = tensors[:len(keys)], tensors[len(keys):]
+        if gkeys:
+            engine.set_gains(dict(zip(gkeys, gtensors)))
+        ctx.gains_version, ctx.gkeys = engine._gains_version, gkeys
         refs = dict(zip(keys, tensors))
         prob = engine.problem_data(q, v, mask, refs, parts=engine.PROBLEM_PARTS + engine.ACTUATION_PARTS)
         sol = engine.qp_solve(prob)
@@ -819,8 +918,12 @@ class _TickLayer(torch.autograd.Function):
         return x[:, :, :nv].contiguous(), f
 
     @staticmethod
-    def jvp(ctx, _gengine, tq, tv, _gmask, _gkeys, *trefs):
+    def jvp(ctx, _gengine, tq, tv, _gmask, _gkeys, _ggkeys, *trefs):
         """forward mode: tsidb_tick_jvp with one per-env direction, the inputs' tangents (None = zero)."""
+        if any(t is not None for t in trefs[len(ctx.keys):]):
+            raise NotImplementedError("tick_layer: forward mode in the gains and weights is not implemented "
+                                      "(reverse mode is: tick_layer's backward pass, gains_grad)")
+        trefs = trefs[:len(ctx.keys)]
         e, ns, npb = ctx.engine, len(_TickLayer.SOL), len(_TickLayer.PROB)
         q, v, mask, *rest = ctx.saved_tensors
         sol, prob, tensors = dict(zip(_TickLayer.SOL, rest[:ns])), dict(zip(_TickLayer.PROB, rest[ns:ns + npb])), rest[ns + npb:]
@@ -836,12 +939,17 @@ class _TickLayer(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, gtau, gdv, gf, _gstatus, _giters):
         e, ns, npb = ctx.engine, len(_TickLayer.SOL), len(_TickLayer.PROB)
+        if e._gains_version != ctx.gains_version:
+            raise RuntimeError("tick_layer: set_gains ran after the forward pass; its gradients would be those of other "
+                               "gains and weights")
         q, v, mask, *rest = ctx.saved_tensors
         sol, prob, tensors = dict(zip(_TickLayer.SOL, rest[:ns])), dict(zip(_TickLayer.PROB, rest[ns:ns + npb])), rest[ns + npb:]
-        parts = tuple(k for i, k in enumerate(ctx.keys) if ctx.needs_input_grad[5 + i])
+        nk, none = len(ctx.keys), (None,) * (6 + len(ctx.keys) + len(ctx.gkeys))
+        parts = tuple(k for i, k in enumerate(ctx.keys) if ctx.needs_input_grad[6 + i])
+        gparts = tuple(k for i, k in enumerate(ctx.gkeys) if ctx.needs_input_grad[6 + nk + i])
         sparts = tuple(k for k, i in (("q", 1), ("v", 2)) if ctx.needs_input_grad[i])
-        if not parts and not sparts:
-            return (None,) * (5 + len(ctx.keys))
+        if not parts and not sparts and not gparts:
+            return none
         n, nv = q.shape[0], e.nv
         grads = {}
         if gdv is not None or gf is not None:
@@ -857,12 +965,15 @@ class _TickLayer(torch.autograd.Function):
         if gtau is not None:
             grads["tau"] = gtau.contiguous()
         if not grads:
-            return (None,) * (5 + len(ctx.keys))
-        refs = dict(zip(ctx.keys, tensors))
-        qg = e.qp_grad(prob, sol, grads, e.PROBLEM_PARTS + e.ACTUATION_PARTS if sparts else ("g", "ce0"))
+            return none
+        refs = dict(zip(ctx.keys, tensors[:nk]))
+        qparts = e.PROBLEM_PARTS + e.ACTUATION_PARTS if sparts else (("H", "g", "ce0") if gparts else ("g", "ce0"))
+        qg = e.qp_grad(prob, sol, grads, qparts)
         out = e.refs_grad(q, v, mask, refs, qg["g"], qg["ce0"], parts) if parts else {}
         st = e.state_grad(q, v, mask, refs, qg, sparts) if sparts else {}
-        return (None, st.get("q"), st.get("v"), None, None) + tuple(out.get(k) for k in ctx.keys)
+        gg = {k: t.sum(0) for k, t in e.gains_grad(q, v, mask, refs, qg, gparts).items()} if gparts else {}
+        return (None, st.get("q"), st.get("v"), None, None, None) + tuple(out.get(k) for k in ctx.keys) + \
+            tuple(gg.get(k) for k in ctx.gkeys)
 
 
 def fp64_peak_tflops(device: int = 0) -> float:
