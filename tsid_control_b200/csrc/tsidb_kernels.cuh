@@ -91,6 +91,12 @@ TSIDB_DEV Dual operator*(double a, const Dual& b) { return Dual(a * b.v, a * b.d
 TSIDB_DEV Dual operator/(const Dual& a, const Dual& b) { const double r = a.v / b.v; return Dual(r, (a.d - r * b.d) / b.v); }
 TSIDB_DEV Dual operator/(double a, const Dual& b) { const double r = a / b.v; return Dual(r, -r * b.d / b.v); }
 TSIDB_DEV Dual& operator+=(Dual& a, const Dual& b) { a.v += b.v; a.d += b.d; return a; }
+/* K1's reference point, one coordinate: the base position as read, rounded toward zero to whole metres; a plain double
+ * also in the tangent passes.  q - c is exact and (a reference position) - c rounds at the size of the difference, never
+ * at the size of c; |q - c| < 1 m bounds the lever arms at any distance, and for a base within a metre of the origin
+ * (c = 0) the arithmetic is that of world-origin algebra. */
+TSIDB_DEV double ref_point(double x) { return trunc(x); }
+TSIDB_DEV double ref_point(const Dual& x) { return trunc(x.v); }
 TSIDB_DEV void sincos(const Dual& x, Dual* s, Dual* c) {
   double sv, cv;
   sincos(x.v, &sv, &cv);
@@ -200,9 +206,13 @@ TSIDB_DEV void log6_dev(const double* R, const double* p, double* out) {
 }
 
 /* ================================================================= K1: dynamics */
-/* lane <-> body.  Everything is expressed in WORLD coordinates (Plücker vectors taken at the
- * world origin), which makes the per-body work independent once the placements are known;
- * only the placement/velocity chain (top-down) and the subtree sums (bottom-up) walk the tree. */
+/* lane <-> body.  Everything is expressed in world AXES with Plücker vectors taken at the env's own reference point c
+ * (ref_point: the base position in whole metres, a plain double also in the tangent passes), which makes the per-body work
+ * independent once the placements are known; only the placement/velocity chain (top-down) and the subtree sums
+ * (bottom-up) walk the tree.  Taken at the world origin instead, the inertias moved there (m |c|^2) and the momenta
+ * (c x P) of a robot at distance d are O(m d^2) terms whose differences are M, h and J: their rounding grew with d^2.
+ * The frames and the CoM in the Fr block stay relative to c; stage_refs_wait moves the reference positions there too,
+ * and dynamics_env adds c back where a world position leaves the kernel (DESIGN.md, reference point). */
 /* per-body model constants staged in shared memory, one copy per CTA: a lane reads the constants of ITS body, and
  * lane-dependent addresses into __constant__ memory are served one address at a time */
 #define MDL_STRIDE 27   /* jR 9, jp 3, mass 1, com 3, inertia 9, parent, depth; odd: conflict-free lane <-> body reads */
@@ -315,7 +325,8 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, T* sm, int lane
     R[0] = 1 - (tyy + tzz); R[1] = txy - twz; R[2] = txz + twy;
     R[3] = txy + twz; R[4] = 1 - (txx + tzz); R[5] = tyz - twx;
     R[6] = txz - twy; R[7] = tyz + twx; R[8] = 1 - (txx + tyy);
-    p[0] = qs[0]; p[1] = qs[1]; p[2] = qs[2];
+    /* relative to the reference point c (ref_point) */
+    p[0] = qs[0] - ref_point(qs[0]); p[1] = qs[1] - ref_point(qs[1]); p[2] = qs[2] - ref_point(qs[2]);
     T vl[3] = {vs[0], vs[1], vs[2]}, wl[3] = {vs[3], vs[4], vs[5]};
     mv3(R, wl, Va);
     mv3(R, vl, Vl);
@@ -421,7 +432,7 @@ TSIDB_DEV void k1_dynamics(const DevConst& C, const double* mdl, T* sm, int lane
   T Sa_[3] = {R[2], R[5], R[8]}, Sl_[3];
   cross3(p, Sa_, Sl_);
 
-  /* per-body inertial quantities, world coordinates, reference point = world origin */
+  /* per-body inertial quantities, world axes, reference point = c (ref_point) */
   K1Acc<T> acc(sm, lane);
   {
     double m = act ? mdl[b * MDL_STRIDE + MDL_oMASS] : 0.0;
@@ -2005,10 +2016,19 @@ TSIDB_DEV void stage_refs(const DevConst& C, const double* mdl, double* sm, cons
   asm volatile("cp.async.commit_group;" ::: "memory");
 #endif
 }
-TSIDB_DEV void stage_refs_wait() {
+/* ... and waited for; the five reference positions (CoM, the two foot tasks, the two contacts) are then taken relative
+ * to the env's reference point c (ref_point of q[0:3] staged at SM_oQV), as K1's frames and CoM are: nothing rounds at
+ * the size of the distance from the origin.  Lane k staged coordinate k of q and of each of the five (stage_refs, the q
+ * staging of every caller), so it shifts them after its own wait, with no extra barrier. */
+TSIDB_DEV void stage_refs_wait(double* sm, int lane) {
 #ifndef TSIDB_EMU
   asm volatile("cp.async.wait_group 0;" ::: "memory");
 #endif
+  if (lane < 3) {
+    const double c = ref_point(sm[SM_oQV + lane]);
+    double* rf = sm + SM_oRef + lane;
+    rf[RF_COM] -= c; rf[RF_FOOT] -= c; rf[RF_FOOT + 24] -= c; rf[RF_CONTACT] -= c; rf[RF_CONTACT + 12] -= c;
+  }
   __syncwarp();
 }
 
@@ -2048,12 +2068,14 @@ TSIDB_DEV void dynamics_env(const DevConst& C, const double* mdl, double* sm, co
   __syncwarp();
   k1_dynamics<NV>(C, mdl, sm, lane);
   const double* fr = sm + SM_oFr;
-  if (a.o_com && lane < 9) a.o_com[eidx(a, env, lane, 9)] = fr[FR_COM + lane];
+  /* world positions again: K1's CoM and soles are relative to the reference point c */
+  const double cw = lane < 3 ? ref_point(sm[SM_oQV + lane]) : 0.0;
+  if (a.o_com && lane < 9) a.o_com[eidx(a, env, lane, 9)] = fr[FR_COM + lane] + cw;
 #pragma unroll
   for (int f = 0; f < 2; f++)
     if (a.o_foot[f] && lane < 12) {
       /* (p, R column-major) */
-      double val = (lane < 3) ? fr[FR_OMF + f * 12 + lane] : fr[FR_OMF + f * 12 + 3 + 3 * ((lane - 3) % 3) + (lane - 3) / 3];
+      double val = (lane < 3) ? fr[FR_OMF + f * 12 + lane] + cw : fr[FR_OMF + f * 12 + 3 + 3 * ((lane - 3) % 3) + (lane - 3) / 3];
       a.o_foot[f][eidx(a, env, lane, 12)] = val;
     }
   if (a.kin_only) return;
@@ -2080,7 +2102,7 @@ TSIDB_DEV void dynamics_env(const DevConst& C, const double* mdl, double* sm, co
   for (int k = lane; k < 162; k += 32) eimg[SE_oMu + k] = sm[SM_oM + k];
   __syncwarp();
   PHASE_SYNC_D();
-  stage_refs_wait();
+  stage_refs_wait(sm, lane);
   k2_assemble<NV>(C, mdl, sm, a, env, lane, mask, neq, n);
   /* solver image (layout a_layout(nv, nc)): the parts that do not depend on the elimination */
   /* rows of the feet in contact, in force-block order (block 0 = LF if it is in contact, else RF), row by row */
@@ -2733,7 +2755,7 @@ TSIDB_DEV void refs_grad_env(const DevConst& C, const double* mdl, double* sm, c
   stage_refs(C, mdl, sm, a, env, lane, na);
   __syncwarp();
   k1_dynamics<NV>(C, mdl, sm, lane);
-  stage_refs_wait();
+  stage_refs_wait(sm, lane);
   const int mask = a.mask ? (a.mask[env] & 3) : 3;
   refs_adjoint_env<NV>(C, mdl, sm, a, r, env, lane, mask);
 }
@@ -2925,7 +2947,7 @@ TSIDB_DEV void gains_grad_env(const DevConst& C, const double* mdl, double* sm, 
   stage_refs(C, mdl, sm, a, env, lane, na);
   __syncwarp();
   k1_dynamics<NV>(C, mdl, sm, lane);
-  stage_refs_wait();
+  stage_refs_wait(sm, lane);
   const int mask = a.mask ? (a.mask[env] & 3) : 3;
   gains_adjoint_env<NV>(C, mdl, sm, a, r, env, lane, mask);
 }
@@ -3183,7 +3205,7 @@ TSIDB_DEV void state_grad_env(const DevConst& C, const double* mdl, double* sm, 
   stage_refs(C, mdl, sm, a, env, lane, na);
   __syncwarp();
   k1_dynamics<NV>(C, mdl, sm, lane);
-  stage_refs_wait();
+  stage_refs_wait(sm, lane);
   const int mask = a.mask ? (a.mask[env] & 3) : 3;
   const int nc = (mask & 1) + ((mask >> 1) & 1);
   k2_assemble<NV>(C, mdl, sm, a, env, lane, mask, 6 + 6 * nc, nv + 12 * nc);
@@ -4004,7 +4026,7 @@ TSIDB_DEVNI bool tick_jvp_setup(const DevConst& C, const double* mdl, double* sm
   stage_refs(C, mdl, sm, a, env, lane, na);
   __syncwarp();
   k1_dynamics<NV>(C, mdl, sm, lane);
-  stage_refs_wait();
+  stage_refs_wait(sm, lane);
   const int mask = a.mask ? (a.mask[env] & 3) : 3;
   const int nc = (mask & 1) + ((mask >> 1) & 1);
   const int f0 = (mask & 1) ? 0 : 1; /* foot of force slot 0; slot 1 is RF */
@@ -4420,11 +4442,11 @@ tsidb_dynamics_kernel(const TickArgs a) {
   int env = a.perm ? a.perm[slot] : slot;
   for (int r = 0; r < rounds; r++) {
     /* the warp's next env: its q, v are prefetched while this one is computed (not in kinematics-only calls, which
-     * stage no references and so have no copy group to ride on) */
-    const bool more = r + 1 < rounds && !a.kin_only;
+     * stage no references and so have no copy group to ride on; they still move on to the next slot) */
+    const bool more = r + 1 < rounds;
     const int slot_n = more ? slot_of(r + 1) : slot;
     const int env_n = more ? (a.perm ? a.perm[slot_n] : slot_n) : -1;
-    dynamics_env<NV>(C, mdl, sm, a, env, slot, lane, r > 0 && !a.kin_only, env_n);
+    dynamics_env<NV>(C, mdl, sm, a, env, slot, lane, r > 0 && !a.kin_only, a.kin_only ? -1 : env_n);
     slot = slot_n;
     env = env_n;
   }
